@@ -14,9 +14,16 @@ clip + AdamW, decoder renorm, counters, metrics).  The YAML batch (128) is launc
 construction, so the headline batch is `--batch` (default 75776 = 4 waves of 148 x 128-row tiles;
 config-legal: TrainingConfig.batch_size >= 1); the YAML-batch number is reported as `yaml_batch`.
 
-Timing: the K-step block is timed `--repeats` times (CUDA events on the launching stream, barrier +
-synchronize on both sides of every block, max over ranks per block) and the MEDIAN block is
-reported, min / max next to it - one straggler in a 16 ms window cannot set the number.
+Timing: `--steps` K is the number of timed steps of the headline value (and of the e2e leg).  They
+run back to back after `--warmup` untimed ones and CUDA events on the launching stream cut them into
+`--repeats` blocks (at most K; barrier + synchronize before and after, max over ranks per block);
+the MEDIAN block's time per step is reported, min / max next to it - one straggler block cannot set
+the number.  The defaults, 1250 steps in 25 blocks of 50 (about 1 s at 0.76 ms per step), keep the
+timed window long against clock and scheduler noise.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (the step's metrics
+and the model state it left, bench.dump_outputs) as DIR/<name>.npy; the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 
 N > 1: one process per GPU, each training an independent layer's SAE (4 encoder + 4 decoder layers
 of whisper-tiny; no data-path collective), value = sum of rows/s, weak scaling.  The same JSON line
@@ -29,6 +36,7 @@ from __future__ import annotations
 
 import argparse
 import contextlib
+import dataclasses
 import gc
 import json
 import os
@@ -260,41 +268,77 @@ def _max_over_ranks(vals: list[float], dist_on: bool) -> list[float]:
 
 
 def time_blocks(run_steps, steps: int, warmup: int, repeats: int, dist_on: bool) -> tuple[dict, int]:
-    """`repeats` timed blocks of exactly `steps` steps each: CUDA events on the launching stream,
-    barrier + synchronize on both sides of every block, max over ranks per block.  Returns the block
-    statistics (seconds) and this rank's kernel launches inside ONE block."""
+    """Exactly `steps` timed steps after `warmup` untimed ones, run back to back and cut into
+    min(`repeats`, `steps`) consecutive blocks of near-equal length by CUDA events on the launching
+    stream; barrier + synchronize before the first block and after the last, max over ranks per block.
+    Returns seconds PER STEP (median / min / max over the blocks) and this rank's kernel launches
+    over the `steps` steps."""
     from whisper_sae_b200 import ops
 
     run_steps(0, warmup)
     torch.cuda.synchronize()
-    secs, launches, pos = [], 0, warmup
-    for _ in range(repeats):
-        if dist_on:
-            torch.distributed.barrier()
-        torch.cuda.synchronize()
-        start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        l0 = ops.GPU_LAUNCHES
-        start.record()
-        run_steps(pos, steps)
-        end.record()
-        torch.cuda.synchronize()
-        launches = ops.GPU_LAUNCHES - l0
-        if dist_on:
-            torch.distributed.barrier()
-        secs.append(start.elapsed_time(end) / 1e3)
-        pos += steps
+    nblk = max(1, min(repeats, steps))
+    sizes = [steps // nblk + (i < steps % nblk) for i in range(nblk)]
+    events = [torch.cuda.Event(enable_timing=True) for _ in range(nblk + 1)]
+    if dist_on:
+        torch.distributed.barrier()
+    torch.cuda.synchronize()
+    l0 = ops.GPU_LAUNCHES
+    events[0].record()
+    pos = warmup
+    for i, n in enumerate(sizes):
+        run_steps(pos, n)
+        events[i + 1].record()
+        pos += n
+    torch.cuda.synchronize()
+    launches = ops.GPU_LAUNCHES - l0
+    if dist_on:
+        torch.distributed.barrier()
+    secs = [events[i].elapsed_time(events[i + 1]) / 1e3 / n for i, n in enumerate(sizes)]
     secs = _max_over_ranks(secs, dist_on)
     srt = sorted(secs)
-    return {"median": statistics.median(secs), "min": srt[0], "max": srt[-1], "repeats": repeats}, launches
+    return {"median": statistics.median(secs), "min": srt[0], "max": srt[-1], "blocks": nblk}, launches
 
 
 def step_runner(tr, batches):
+    """run(pos, count): `count` train steps on `batches` from index `pos`; run.last is the
+    TrainingMetrics of the latest step."""
     n = len(batches)
 
     def run(pos: int, count: int) -> None:
         for i in range(count):
-            tr.train_step(batches[(pos + i) % n])
+            run.last = tr.train_step(batches[(pos + i) % n])
+    run.last = None
     return run
+
+
+DUMP_LIMIT_BYTES = 60 << 20          # with the .npy headers, under 64 MB however counted
+
+
+def dump_outputs(out_dir: Path, metrics, model) -> None:
+    """What a caller of the timed path holds after its last step, one `out_dir/<name>.npy` each: the
+    returned TrainingMetrics fields (float64) and the model's state_dict (float32; integer counters as
+    float64).  Above DUMP_LIMIT_BYTES in all, every array over 1 MiB keeps the same fraction of its
+    elements, at sorted flat indices drawn from a generator seeded with 0: the same elements on every
+    run with the same shapes."""
+    import numpy as np
+
+    arrays = {k: np.array(v, dtype=np.float64) for k, v in dataclasses.asdict(metrics).items()}
+    for name, t in model.state_dict().items():
+        t = t.detach().cpu().contiguous()
+        arrays[name] = (t.float() if t.is_floating_point() else t.double()).numpy()
+    big = sorted(k for k, a in arrays.items() if a.nbytes > 1 << 20)
+    big_bytes = sum(arrays[k].nbytes for k in big)
+    small_bytes = sum(a.nbytes for a in arrays.values()) - big_bytes
+    if small_bytes + big_bytes > DUMP_LIMIT_BYTES:
+        frac = (DUMP_LIMIT_BYTES - small_bytes) / big_bytes
+        for k in big:
+            flat = arrays[k].reshape(-1)
+            idx = torch.randperm(flat.size, generator=torch.Generator().manual_seed(0))[:int(flat.size * frac)]
+            arrays[k] = flat[idx.sort().values.numpy()]
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", a)
 
 
 def epoch_runner(tr, host_batches):
@@ -675,7 +719,8 @@ def workload_config(args, wl: dict, n_gpus: int) -> dict:
     }
 
 
-def side_workload(name: str, batch: int, dev: str, rank: int, world: int, steps: int, warmup: int, repeats: int,
+def side_workload(name: str, batch: int, dev: str, rank: int, world: int, steps_per_block: int, warmup: int,
+                  repeats: int,
                   peaks: dict, peak_src: str, dp: bool, global_rows: int | None, profile: bool) -> dict:
     """One entry of the `workloads` block: the same step at another BASELINE config."""
     wl = WORKLOADS[name]
@@ -685,14 +730,14 @@ def side_workload(name: str, batch: int, dev: str, rank: int, world: int, steps:
     rows = synth(nb * batch, wl["d"], seed=777 + rank)
     batches = [rows[i * batch:(i + 1) * batch].to(dev) for i in range(nb)]
     with ClockSampler(int(dev.split(":")[1])) as clocks:
-        blk, launches = time_blocks(step_runner(tr, batches), steps, warmup, repeats, dist_on)
+        blk, launches = time_blocks(step_runner(tr, batches), steps_per_block * repeats, warmup, repeats, dist_on)
     n_ranks = world if dp else 1
     out = {"config": f"{wl['label']} TopKSAE {wl['d']}->{wl['d'] * wl['expansion']} k={wl['k']} "
                      f"(BASELINE.json {wl['cfg']}), {batch} rows per GPU x {n_ranks} GPU(s), bf16",
-           "value": batch * steps * n_ranks / blk["median"], "unit": UNIT,
-           "ms_per_step": 1e3 * blk["median"] / steps,
-           "ms_per_step_min_max": [1e3 * blk["min"] / steps, 1e3 * blk["max"] / steps],
-           "gpu_launches": launches, "clocks": clocks.summary()}
+           "value": batch * n_ranks / blk["median"], "unit": UNIT,
+           "ms_per_step": 1e3 * blk["median"],
+           "ms_per_step_min_max": [1e3 * blk["min"], 1e3 * blk["max"]],
+           "gpu_launches": launches // repeats, "clocks": clocks.summary()}
     tr.release_graphs()      # (captured graphs that hold NCCL kernels must not outlive the communicator)
     del tr
     if profile:
@@ -713,10 +758,11 @@ def side_workload(name: str, batch: int, dev: str, rank: int, world: int, steps:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=1250, help="timed steps of the headline value and the e2e leg")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--repeats", type=int, default=25,
-                    help="timed blocks of --steps steps; the median block is reported")
+                    help="blocks the --steps timed steps are cut into; the median block's time per step "
+                         "is reported")
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--workload", choices=sorted(WORKLOADS), default="tiny")
     ap.add_argument("--batch", type=int, default=None,
@@ -729,7 +775,13 @@ def main() -> None:
     ap.add_argument("--value-only", action="store_true",
                     help="only the HBM-resident timed leg (used under ncu; prints a reduced line)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", type=Path, default=None, metavar="DIR",
+                    help="write the metrics and model state of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs is not None:
+        ap.error("--dump-outputs writes the outputs of the B200 path: not with --impl reference")
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload]
     world_env = int(os.environ.get("WORLD_SIZE", "1"))
@@ -767,15 +819,20 @@ def main() -> None:
 
     # ---- value: inputs resident in HBM ----
     with ClockSampler(local_rank) as clocks:
-        blk, launches = time_blocks(step_runner(tr, dev_batches), args.steps, args.warmup, repeats, dist_on)
-    sec = blk["median"]
-    value = args.batch * args.steps * world / sec
+        runner = step_runner(tr, dev_batches)
+        blk, launches = time_blocks(runner, args.steps, args.warmup, repeats, dist_on)
+    sec = blk["median"]                      # per step
+    value = args.batch * world / sec
+    if args.dump_outputs is not None:
+        tr.consolidate_weights()             # data parallel: gathers every rank's weight rows (collective)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, runner.last, tr.model)
 
     if args.value_only:
         if rank == 0:
             print(json.dumps({"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world,
                               "steps": args.steps, "warmup": args.warmup,
-                              "ms_per_step": 1e3 * sec / args.steps, "gpu_launches": launches,
+                              "ms_per_step": 1e3 * sec, "gpu_launches": launches,
                               "note": "value-only leg (not a bench line)"}))
         if dist_on:
             tr.release_graphs()
@@ -786,8 +843,9 @@ def main() -> None:
 
     # ---- e2e: pinned host batches through SAETrainer.train_epoch (H2D + metrics D2H inside) ----
     host_batches = [rows[i * args.batch:(i + 1) * args.batch].pin_memory() for i in range(nb)]
+    # each block is one train_epoch call (its first H2D copy is not overlapped, as in any epoch)
     blk_e, _ = time_blocks(epoch_runner(tr, host_batches), args.steps, args.warmup, repeats, dist_on)
-    e2e = args.batch * args.steps * world / blk_e["median"]
+    e2e = args.batch * world / blk_e["median"]
     h2d_bytes = args.batch * d * 4 + 64          # batch + control block
     resident = resident_loader_rate(tr, rows, args.batch, dev) if (rank == 0 and not dp) else None
 
@@ -808,31 +866,32 @@ def main() -> None:
         tr_small, _ = make_trainer(wl, cfg_batch, dev, layer_seed=rank, use_amp=bf16)
         small_rows = synth(16 * cfg_batch, d, seed=4321 + rank).to(dev)
         small = [small_rows[i * cfg_batch:(i + 1) * cfg_batch].contiguous() for i in range(16)]
-        blk_s, _ = time_blocks(step_runner(tr_small, small), 100, 10, 5, False)
+        blk_s, _ = time_blocks(step_runner(tr_small, small), 500, 10, 5, False)
         del tr_small
         det_info = None
         if bf16:      # the bit-reproducible accumulation mode, for the record (SAETrainer(deterministic=True))
             tr_det, _ = make_trainer(wl, args.batch, dev, layer_seed=rank, deterministic=True)
-            blk_d, _ = time_blocks(step_runner(tr_det, dev_batches), args.steps, 3, 5, False)
-            det_info = {"ms_per_step": 1e3 * blk_d["median"] / args.steps,
-                        "value": args.batch * args.steps / blk_d["median"], "unit": UNIT,
+            # 5 blocks as long as one headline block
+            blk_d, _ = time_blocks(step_runner(tr_det, dev_batches), 5 * max(1, args.steps // repeats), 3, 5, False)
+            det_info = {"ms_per_step": 1e3 * blk_d["median"],
+                        "value": args.batch / blk_d["median"], "unit": UNIT,
                         "note": "ordered split-K / fixed-point cross-row sums instead of float atomics; "
                                 "bit-identical from run to run (tests/test_gpu_fullsize.py)"}
             del tr_det
         line = {
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": 1e3 * sec / args.steps, "higher_is_better": True,
+            "warmup": args.warmup, "ms_per_step": 1e3 * sec, "higher_is_better": True,
             "scaling": "strong" if wl["dp"] else "weak", "vs_baseline": None,
             "dtype": "bf16" if bf16 else "f32", "data": "synthetic",
             "config": workload_config(args, wl, world),
-            "timing": {"repeats": repeats, "block_ms_median": 1e3 * sec, "block_ms_min": 1e3 * blk["min"],
-                       "block_ms_max": 1e3 * blk["max"],
-                       "method": "median over `repeats` blocks of `steps` steps; each block bracketed by "
-                                 "barrier + synchronize, CUDA events, max over ranks"},
+            "timing": {"blocks": blk["blocks"], "step_ms_median": 1e3 * sec, "step_ms_min": 1e3 * blk["min"],
+                       "step_ms_max": 1e3 * blk["max"],
+                       "method": "`steps` steps back to back cut into `blocks` blocks by CUDA events, median "
+                                 "block time per step; barrier + synchronize around the run, max over ranks"},
             "e2e": {"value": e2e, "unit": UNIT, "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 32,
-                    "ms_per_step": 1e3 * blk_e["median"] / args.steps,
-                    "ms_per_step_min_max": [1e3 * blk_e["min"] / args.steps, 1e3 * blk_e["max"] / args.steps],
-                    "h2d_gbs_per_gpu": h2d_bytes * args.steps / blk_e["median"] / 1e9,
+                    "ms_per_step": 1e3 * blk_e["median"],
+                    "ms_per_step_min_max": [1e3 * blk_e["min"], 1e3 * blk_e["max"]],
+                    "h2d_gbs_per_gpu": h2d_bytes / blk_e["median"] / 1e9,
                     "host_numa": numa},
             "gpu_launches": launches,
             "clocks": clocks.summary(),
@@ -840,8 +899,8 @@ def main() -> None:
             "rooflines": {n: {kk: vv for kk, vv in e.items() if kk != "per_step"} for n, e in table.items()},
             "kernel_shares": {n: e["share_of_step"] for n, e in table.items()},
             "kernel_avg_ms": {n: e["avg_ms"] for n, e in table.items()},
-            "yaml_batch": {"batch_rows": cfg_batch, "value": cfg_batch * 100 / blk_s["median"], "unit": UNIT,
-                           "ms_per_step": 1e3 * blk_s["median"] / 100},
+            "yaml_batch": {"batch_rows": cfg_batch, "value": cfg_batch / blk_s["median"], "unit": UNIT,
+                           "ms_per_step": 1e3 * blk_s["median"]},
             "deterministic_mode": det_info,
             "resident_loader": resident,
         }
@@ -852,18 +911,18 @@ def main() -> None:
 
     # ---- `workloads` block: BASELINE configs[2] / [3] ----
     if args.workload == "tiny" and not args.no_side_workloads:
-        s_steps = max(3, min(args.steps, 10))
+        s_block = max(3, min(args.steps, 10))
         s_rep = max(3, min(repeats, 7))
         if not dist_on:
             for name, key in (("small-dp", "small"), ("large-dp", "large-v3")):
-                side[key] = side_workload(name, WORKLOADS[name]["batch"], dev, rank, world, s_steps, 3, s_rep,
+                side[key] = side_workload(name, WORKLOADS[name]["batch"], dev, rank, world, s_block, 3, s_rep,
                                           peaks, peak_src, dp=False, global_rows=None, profile=True)
         else:
             for name, key in (("small-dp", "small"), ("large-dp", "large-v3")):
                 full = WORKLOADS[name]["batch"]
-                weak = side_workload(name, full, dev, rank, world, s_steps, 3, s_rep, peaks, peak_src,
+                weak = side_workload(name, full, dev, rank, world, s_block, 3, s_rep, peaks, peak_src,
                                      dp=True, global_rows=full * world, profile=False)
-                strong = side_workload(name, full // world, dev, rank, world, s_steps, 3, s_rep, peaks,
+                strong = side_workload(name, full // world, dev, rank, world, s_block, 3, s_rep, peaks,
                                        peak_src, dp=True, global_rows=(full // world) * world, profile=False)
                 side[key + "_dp_weak"] = dict(weak, scaling="weak (fixed rows per GPU), batch-sharded, NCCL gradient exchange")
                 side[key + "_dp_strong"] = dict(strong, scaling="strong (fixed global batch), batch-sharded, NCCL gradient exchange")

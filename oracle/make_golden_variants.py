@@ -1,5 +1,6 @@
 """Golden vectors for the transcoder / crosscoder variants from the LIVE reference (build container
-only; same rules as make_golden.py).  Writes tests/golden/variants.pt.
+only; same rules as make_golden.py).  Writes tests/golden/variants.pt (transcoders) and
+tests/golden/variants_crosscoder.pt (crosscoders), two files so that each stays under 1 MB.
 
     PYTHONDONTWRITEBYTECODE=1 python oracle/make_golden_variants.py
 """
@@ -87,6 +88,7 @@ if __name__ == "__main__":
     big["grads"] = {n: {"sum": g.double().sum().item(), "abs_sum": g.double().abs().sum().item(),
                         "sample": g.reshape(-1)[::997].clone()} for n, g in big["grads"].items()}
     GOLDEN.mkdir(parents=True, exist_ok=True)
-    torch.save(cases, GOLDEN / "variants.pt")
+    torch.save({n: c for n, c in cases.items() if not n.startswith("crosscoder")}, GOLDEN / "variants.pt")
+    torch.save({n: c for n, c in cases.items() if n.startswith("crosscoder")}, GOLDEN / "variants_crosscoder.pt")
     for n, c in cases.items():
         print(n, "loss", round(c["loss"], 6), "l0", c["l0"])

@@ -7,7 +7,7 @@ Plain-tensor restatements (dense torch ops + autograd for the gradients) of
     /root/reference/src/whisper_sae/sae/crosscoder.py   TopKCrossLayerCrosscoder (:326-379), decode (:171-188)
 
 operating on ``state_dict``-shaped dicts.  Pinned by ``oracle/make_golden_variants.py`` (live
-reference, build container only) -> ``tests/golden/variants.pt`` -> ``tests/test_oracle_golden.py``.
+reference) -> ``tests/golden/variants{,_crosscoder}.pt`` -> ``tests/test_oracle_golden.py``.
 """
 
 from __future__ import annotations

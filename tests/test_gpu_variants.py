@@ -1,5 +1,6 @@
 """Transcoder / crosscoder variants of the hot path (BASELINE config 5) on the fused CUDA path,
-against golden vectors produced by the live reference (oracle/make_golden_variants.py)."""
+against golden vectors produced by the live reference (oracle/make_golden_variants.py:
+tests/golden/variants.pt and variants_crosscoder.pt)."""
 
 import pytest
 import torch
@@ -115,7 +116,7 @@ def _build_crosscoder(r, precision, state=None):
 
 @pytest.mark.parametrize("name", ["crosscoder_64x4_128_k8", "crosscoder_subset_64x2_128_k8"])
 def test_crosscoder_fp32_matches_reference(name):
-    fx = load_golden("variants")[name]
+    fx = load_golden("variants_crosscoder")[name]
     r = fx["recipe"]
     m = _build_crosscoder(r, "fp32", fx["state"])
     acts = {li: _inputs(r["seed"] + 20 + i, r["B"], r["d"]).cuda() for i, li in enumerate(r["layer_indices"])}
@@ -137,7 +138,7 @@ def test_crosscoder_fp32_matches_reference(name):
 @pytest.mark.parametrize("precision,tol", [("fp32", 1e-5), ("bf16", 2e-2)])
 def test_crosscoder_whisper_tiny_shape(precision, tol):
     """tests/test_crosscoder.py:421-436 shape (BASELINE config 5): d=384, 4 layers, 3072 features, k=32."""
-    fx = load_golden("variants")["crosscoder_tiny_384x4_3072_k32"]
+    fx = load_golden("variants_crosscoder")["crosscoder_tiny_384x4_3072_k32"]
     r = fx["recipe"]
     m = _build_crosscoder(r, precision)
     acts = {li: _inputs(r["seed"] + 20 + i, r["B"], r["d"]).cuda() for i, li in enumerate(r["layer_indices"])}

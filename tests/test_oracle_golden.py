@@ -183,7 +183,7 @@ def _variant_inputs(seed, *shape):
 def test_variants_oracle_matches_reference(name):
     from oracle import variants_oracle as V
 
-    fx = load_golden("variants")[name]
+    fx = load_golden("variants_crosscoder" if name.startswith("crosscoder") else "variants")[name]
     r = fx["recipe"]
     if name.startswith("crosscoder"):
         acts = {li: _variant_inputs(r["seed"] + 20 + i, r["B"], r["d"]) for i, li in enumerate(r["layer_indices"])}

@@ -195,7 +195,7 @@ def test_nccl_two_rank_step_matches_golden_and_single_device(tmp_path):
     from pathlib import Path
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with `gpurun --gpus 2`)")
+        pytest.skip("needs 2 GPUs")
     root = Path(__file__).resolve().parents[1]
     port = 29500 + os.getpid() % 400
     out = subprocess.run(
