@@ -33,7 +33,9 @@ extern "C" {
 
 typedef void* wsae_stream_t; /* cudaStream_t */
 
-/* Library / build identification: returns 100 * major + minor of the ABI (currently 111: + wsae_encode_topk_dense, wsae_encode_dense, wsae_row_step with the fused counters, wsae_graph_launch, wsae_memcpy_async). */
+/* Library / build identification: returns 100 * major + minor of the ABI (currently 111: + wsae_encode_topk_dense, wsae_encode_dense, wsae_row_step with the fused counters, wsae_graph_launch, wsae_memcpy_async; later
+ * additions that change no existing behaviour keep the number: wsae_encode_topk_chunked, and k up to 256 in
+ * wsae_decode_backward / _at / _rows_at). */
 int wsae_abi_version(void);
 
 /* cudaGraphLaunch(graph_exec, stream) for an instantiated CUDA graph of the calls below (the host mirror
@@ -75,7 +77,8 @@ int wsae_pack_encoder(const float* w_enc /*[F,d]*/, const float* b_enc /*[F] nul
  * are never written.  Emits, per row, the k largest pre-activations (signed, pre-ReLU) and their
  * feature indices, unordered.  Ties at the k-th value resolve to the lowest feature index.
  * nsplit > 1 splits F across CTAs (latency at small B); part_* are [B, nsplit_eff*k] scratch
- * (nsplit_eff from wsae_encode_effective_splits) and may be NULL when nsplit == 1.  k <= 64. */
+ * (nsplit_eff from wsae_encode_effective_splits) and may be NULL when nsplit == 1.  k <= 64
+ * (larger k: wsae_encode_topk_dense or wsae_encode_topk_chunked). */
 int wsae_encode_effective_splits(int F, int nsplit);
 int wsae_encode_topk(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
                      int Kp, int k_used_cols, int k, int nsplit, float* part_val,
@@ -89,6 +92,15 @@ int wsae_encode_topk(const void* a_packed, const void* w_packed, int B, int Bp, 
 int wsae_encode_topk_dense(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
                            int Kp, int k_used_cols, int k, float* pre_ws, float* out_val /*[B,k]*/,
                            int32_t* out_idx /*[B,k]*/, wsae_stream_t stream);
+
+/* K1 for k > 64 (the fused epilogue of wsae_encode_topk stops at k = 64): wsae_encode_topk_dense
+ * over consecutive chunks of chunk_rows packed rows (a multiple of 128), one library call.  pre_ws is
+ * chunk_rows * F floats of scratch, reused by every chunk (size it to stay in L2: ~32-48 MB).
+ * Results bit-identical to one wsae_encode_topk_dense call over all B rows.  F <= 49152, F % 4 == 0,
+ * k <= 65535. */
+int wsae_encode_topk_chunked(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
+                             int Kp, int k_used_cols, int k, int chunk_rows, float* pre_ws,
+                             float* out_val /*[B,k]*/, int32_t* out_idx /*[B,k]*/, wsae_stream_t stream);
 
 /* The GEMM half alone: pre_ws[B, F] = A' x W'^T with the bias (sae/model.py:111), no selection. */
 int wsae_encode_dense(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp, int Kp,
@@ -150,8 +162,11 @@ int wsae_backward_sparse(const float* resid, const float* x /*nullable if !d_w_e
  * reconstruction and the k dot products (bf16 x bf16 -> fp32 FHFMA against the bf16-rounded
  * residual, the same rounding K4 consumes).  Outputs as in wsae_decode_mse / wsae_backward_sparse
  * (weight gradients are left to K4); resid / resid_bf16 / stats / last_activated / d_b_enc /
- * d_b_dec / dpre_val may each be NULL.  d_b_enc and d_b_dec are accumulated (+=).  Returns
- * WSAE_E_UNSUPPORTED for an fp32 decoder, k > 32 or d % 8 != 0: use K2 + K3 then. */
+ * d_b_dec / dpre_val may each be NULL.  d_b_enc and d_b_dec are accumulated (+=).
+ * k ranges: k <= 32 one warp per row; 32 < k <= 256 (d % 128 == 0 only) a team of ceil(k / 32)
+ * warps per row, each holding 32 of the k gathered rows, meeting once per 64 columns to form the
+ * residual.  Returns WSAE_E_UNSUPPORTED for an fp32 decoder, d % 8 != 0, k > 256, or k > 32 with
+ * d % 128 != 0 or with wsae_decode_backward_det's workspace: use K2 + K3 then. */
 int wsae_decode_backward(const float* target, const void* w_decT, int w_is_bf16,
                          const float* b_dec, const float* b_pre /*nullable*/, const int32_t* idx,
                          const float* val, const float* grad_out /*nullable*/, float coef, int B,

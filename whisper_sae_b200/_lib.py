@@ -75,6 +75,11 @@ _SIGNATURES = {
          c_void_p, c_void_p, c_void_p, c_void_p],
         c_int,
     ),
+    "wsae_encode_topk_chunked": (
+        [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+         c_void_p, c_void_p, c_void_p, c_void_p],
+        c_int,
+    ),
     "wsae_graph_launch": ([c_void_p, c_void_p], c_int),
     "wsae_encode_dense": (
         [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p],

@@ -1058,6 +1058,307 @@ decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16*
   }
 }
 
+// ================================================================================================
+// K23, wide form (32 < k <= 256, d % 128 == 0): a TEAM of ceil(k / 32) warps per activation row.
+//
+// The tensor form above needs every 64-column half slice of all k gathered rows in one warp's
+// registers; that is what caps it at k = 32.  Here warp w of a team owns the selected entries
+// [32 w, 32 w + 32) of the row and runs the tensor form's slice code on them unchanged (fragment-order
+// LDG.128 gather, FHFMA.BF16 partial reconstruction, mma.sync dot products against the bf16
+// residual).  Per half slice the warps meet once:
+//   1. each warp parks its partial reconstruction of the 64 columns in shared memory (ping-pong by
+//      half-slice parity) and the team meets at a named barrier (bar.sync 1 + team, 32 * team size);
+//   2. every warp sums the team's partials in warp order - the same fp32 additions in every warp, so
+//      every warp holds the same residual - and forms the residual; warp 0 of the team alone writes
+//      resid / resid_bf16 and accumulates the SSE and the decoder-bias gradient;
+//   3. every warp runs its dot products against the bf16 residual with the decoder registers it holds.
+// A warp reads a partial buffer again only two half slices later, after the next barrier, so one
+// barrier per half slice is enough.  Each decoder row is still gathered once; the cost over the
+// tensor form is one shared-memory exchange and one barrier per half slice.  Entries past k (the tail
+// of the last warp) get activation 0 and gather a spread-out row, like the tensor form's invalid
+// entries: they add nothing and get no dv.
+// ================================================================================================
+constexpr int kWideMaxK = 256;
+constexpr int kWideMaxWarps = 8;
+
+__device__ __forceinline__ void team_sync(int id, int nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+
+__global__ void __maxnreg__(160)   // 156 registers, no spills: the tensor form's budget
+decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
+                            const float* __restrict__ b_dec, const float* __restrict__ b_pre,
+                            const int32_t* __restrict__ idx, const float* __restrict__ val,
+                            const float* __restrict__ grad_out, float coef, int B, int d, int F, int k,
+                            float* __restrict__ resid, __nv_bfloat16* __restrict__ resid_bf16,
+                            FusedStats* __restrict__ stats, long long* __restrict__ last_activated,
+                            const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
+                            float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
+                            const float* const* __restrict__ target_at,
+                            const long long* const* __restrict__ rows_at, int stamp_words, int l2hint) {
+  const uint64_t pol_x = l2_policy((l2hint & 1) ? 1 : 0);
+  const uint64_t pol_w = l2_policy((l2hint & 2) ? 2 : 0);
+  // [d] bias | [teams][d] db_dec partials | [2][warps][64] partial reconstructions |
+  // [warps] bf16 residual ping-pong + 16 zero bytes | fired bitmap
+  extern __shared__ __align__(16) float fsm[];
+  pdl_prologue();
+  if (target_at != nullptr) target = *target_at;
+  const long long* perm = rows_at != nullptr ? *rows_at : nullptr;
+  const int lane = threadIdx.x & 31;
+  const int warp = threadIdx.x >> 5;
+  const int nwarps = blockDim.x >> 5;
+  const int tsize = (k + 31) >> 5;           // warps per team
+  const int teams = nwarps / tsize;
+  const int team = warp / tsize;
+  const int tw = warp - team * tsize;        // rank in the team: owns entries [32 tw, 32 tw + 32)
+  const int entry = 32 * tw + lane;
+  const int bar_id = 1 + team;
+  const int bar_n = 32 * tsize;
+  const int rho = lane >> 3;
+  const int chi = lane & 7;
+  float* s_bias = fsm;
+  float* s_g = fsm + d + team * d;
+  float* s_part = fsm + (1 + teams) * d;
+  char* dyn = reinterpret_cast<char*>(s_part + 2 * nwarps * 64);
+  const uint32_t gbuf = smem_u32(dyn) + warp * kTcGBytes;
+  const uint32_t zbuf = smem_u32(dyn) + nwarps * kTcGBytes;
+  uint32_t* s_fired = reinterpret_cast<uint32_t*>(dyn + nwarps * kTcGBytes + 16);
+  if (threadIdx.x < 4) reinterpret_cast<uint32_t*>(dyn + nwarps * kTcGBytes)[threadIdx.x] = 0u;
+  for (int i = threadIdx.x; i < stamp_words; i += blockDim.x) s_fired[i] = 0u;
+  for (int i = threadIdx.x; i < d; i += blockDim.x) {
+    s_bias[i] = b_dec[i] + (b_pre != nullptr ? b_pre[i] : 0.f);
+    for (int t = 0; t < teams; ++t) fsm[d + t * d + i] = 0.f;
+  }
+  __syncthreads();
+
+  const float s = coef * (grad_out != nullptr ? *grad_out : 1.f);
+  const long long stamp = (last_activated != nullptr && step_count != nullptr) ? (*step_count + 1) : 0;
+  const int team_global = blockIdx.x * teams + team;
+  const int team_stride = gridDim.x * teams;
+  const int nhs = d >> 6;
+  const char* wbytes = reinterpret_cast<const char*>(w_decT);
+  const size_t row_bytes = static_cast<size_t>(d) * 2;
+  const int b4 = (lane >> 4) & 1, b3 = (lane >> 3) & 1;
+  const int c0 = 8 * chi + 4 * b4 + 2 * b3;
+  const uint32_t g_st = static_cast<uint32_t>(chi * 16 + (b4 + 2 * b3) * 4);
+  const int nB = lane >> 2;
+  const uint32_t g_ld = static_cast<uint32_t>(((nB & 1) * 4 + (lane & 3)) * 16 + ((nB >> 1) & 1) * 8);
+  const bool lowB = nB < 4;
+  const bool lead = tw == 0;                 // writes the row's residual, SSE and db_dec partials
+
+  float sse_local = 0.f;
+  unsigned int l0_local = 0;
+
+  auto load_meta = [&](int row, int32_t& mi, float& mv) {
+    mi = -1;
+    mv = 0.f;
+    if (row < B && entry < k) {
+      mi = __ldg(idx + static_cast<size_t>(row) * k + entry);
+      mv = __ldg(val + static_cast<size_t>(row) * k + entry);
+    }
+  };
+  auto gather_feature = [&](int32_t mi, int row) -> uint32_t {
+    return (mi >= 0 && mi < F) ? static_cast<uint32_t>(mi)
+                               : (static_cast<uint32_t>(row) * 37u + static_cast<uint32_t>(entry)) % static_cast<uint32_t>(F);
+  };
+  const char* wp[8];
+  auto set_row = [&](uint32_t feat) {
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const uint32_t f = __shfl_sync(0xffffffffu, feat, 4 * i + rho);
+      wp[i] = wbytes + static_cast<size_t>(f) * row_bytes + chi * 16;
+    }
+  };
+  const float* trow = target;
+  auto set_target = [&](int row) {
+    const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
+    trow = target + srow * d + c0;
+  };
+  auto gather = [&](uint4 (&w)[8], float2& x, int ahead) {
+#pragma unroll
+    for (int i = 0; i < 8; ++i) w[i] = ldg_nc_v4<false>(wp[i] + ahead * 128, pol_w);
+    x = ldg_stream_v2(trow + ahead * 64, pol_x);
+  };
+  auto advance = [&](int n) {
+#pragma unroll
+    for (int i = 0; i < 8; ++i) wp[i] += n * 128;
+    trow += n * 64;
+  };
+
+  int row = team_global;
+  int32_t cur_i, nxt_i;
+  float cur_v, nxt_v;
+  load_meta(row, cur_i, cur_v);
+  load_meta(row + team_stride, nxt_i, nxt_v);
+  uint4 w0[8], w1[8];
+  float2 x0 = make_float2(0.f, 0.f), x1 = x0;
+  if (row < B) {
+    set_row(gather_feature(cur_i, row));
+    set_target(row);
+    gather(w0, x0, 0);
+  }
+
+  for (; row < B; row += team_stride) {
+    const int32_t my_i = cur_i;
+    const bool fired = (my_i >= 0) && (my_i < F) && (cur_v > 0.f);
+    if (fired && last_activated != nullptr) {
+      if (stamp_words > 0) atomicOr(&s_fired[my_i >> 5], 1u << (my_i & 31));
+      else last_activated[my_i] = stamp;
+    }
+    const float my_v = fired ? cur_v : 0.f;
+    const uint32_t my_hb = static_cast<uint32_t>(__bfloat16_as_ushort(__float2bfloat16_rn(my_v)));
+    const uint32_t mask = __ballot_sync(0xffffffffu, fired);
+    l0_local += (lane == 0) ? __popc(mask) : 0;
+    uint32_t hp[4];
+#pragma unroll
+    for (int m = 0; m < 4; ++m) {
+      const uint32_t lo = __shfl_sync(0xffffffffu, my_hb, 8 * m + rho);
+      const uint32_t hi = __shfl_sync(0xffffffffu, my_hb, 8 * m + 4 + rho);
+      hp[m] = lo | (hi << 16);
+    }
+    const size_t orow = static_cast<size_t>(row) * d + c0;
+    int32_t nn_i = -1;
+    float nn_v = 0.f;
+    const bool more = row + team_stride < B;
+
+    float dacc[4][4];
+#pragma unroll
+    for (int p = 0; p < 4; ++p) dacc[p][0] = dacc[p][1] = dacc[p][2] = dacc[p][3] = 0.f;
+
+    auto compute = [&](const uint4 (&w)[8], const float2 x, int hs) {
+      float part[8];
+#pragma unroll
+      for (int c = 0; c < 8; ++c) part[c] = 0.f;
+#pragma unroll
+      for (int m = 0; m < 4; ++m) {
+        fhfma_row4(part, w[2 * m].x, w[2 * m].y, hp[m]);
+        fhfma_row4(part + 4, w[2 * m].z, w[2 * m].w, hp[m]);
+        fhfma_row4_hi(part, w[2 * m + 1].x, w[2 * m + 1].y, hp[m]);
+        fhfma_row4_hi(part + 4, w[2 * m + 1].z, w[2 * m + 1].w, hp[m]);
+      }
+      {
+        const bool up = b4 != 0;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const float send = up ? part[c] : part[c + 4];
+          const float keep = up ? part[c + 4] : part[c];
+          part[c] = keep + __shfl_xor_sync(0xffffffffu, send, 16);
+        }
+      }
+      {
+        const bool up = b3 != 0;
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+          const float send = up ? part[c] : part[c + 2];
+          const float keep = up ? part[c + 2] : part[c];
+          part[c] = keep + __shfl_xor_sync(0xffffffffu, send, 8);
+        }
+      }
+      // ---- team exchange: this warp's 32 entries -> the row's reconstruction of the 64 columns ----
+      float* pbuf = s_part + (hs & 1) * nwarps * 64;
+      *reinterpret_cast<float2*>(pbuf + warp * 64 + c0) = make_float2(part[0], part[1]);
+      team_sync(bar_id, bar_n);
+      float2 rec = make_float2(0.f, 0.f);
+      for (int t = 0; t < tsize; ++t) {
+        const float2 p = *reinterpret_cast<const float2*>(pbuf + (team * tsize + t) * 64 + c0);
+        rec.x += p.x;
+        rec.y += p.y;
+      }
+      const int col = hs * 64 + c0;
+      const float2 bias = *reinterpret_cast<const float2*>(s_bias + col);
+      const float r0 = rec.x + bias.x - x.x;
+      const float r1 = rec.y + bias.y - x.y;
+      __nv_bfloat162 rb2 = __floats2bfloat162_rn(r0, r1);
+      const uint32_t rb = *reinterpret_cast<uint32_t*>(&rb2);
+      if (lead) {
+        sse_local = fmaf(r0, r0, sse_local);
+        sse_local = fmaf(r1, r1, sse_local);
+        float2 gs = *reinterpret_cast<float2*>(s_g + col);
+        gs.x += r0;
+        gs.y += r1;
+        *reinterpret_cast<float2*>(s_g + col) = gs;
+        if (resid != nullptr) *reinterpret_cast<float2*>(resid + orow + hs * 64) = make_float2(r0, r1);
+        if (resid_bf16 != nullptr) *reinterpret_cast<uint32_t*>(resid_bf16 + orow + hs * 64) = rb;
+      }
+      const uint32_t gb = gbuf + (hs & 1) * 128;
+      asm volatile("st.shared.u32 [%0], %1;" ::"r"(gb + g_st), "r"(rb) : "memory");
+      __syncwarp();
+      uint32_t ge0, ge1, go0, go1;
+      asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(ge0), "=r"(ge1) : "r"(lowB ? gb + g_ld : zbuf));
+      asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(go0), "=r"(go1) : "r"(lowB ? zbuf : gb + g_ld));
+#pragma unroll
+      for (int p = 0; p < 4; ++p) {
+        mma_bf16_16816(dacc[p], w[2 * p].x, w[2 * p].y, w[2 * p].z, w[2 * p].w, ge0, ge1);
+        mma_bf16_16816(dacc[p], w[2 * p + 1].x, w[2 * p + 1].y, w[2 * p + 1].z, w[2 * p + 1].w, go0, go1);
+      }
+    };
+
+    for (int hs = 0; hs < nhs; hs += 2) {
+      gather(w1, x1, 1);
+      if (hs == 0) load_meta(row + 2 * team_stride, nn_i, nn_v);
+      compute(w0, x0, hs);
+      const bool last = hs + 2 >= nhs;
+      if (!last) {
+        gather(w0, x0, 2);
+      } else if (more) {
+        set_row(gather_feature(nxt_i, row + team_stride));
+        set_target(row + team_stride);
+        gather(w0, x0, 0);
+      }
+      compute(w1, x1, hs + 1);
+      if (!last) advance(2);
+    }
+
+    // dot products: the tensor form's reduction (lane j ends with the dot product of its entry)
+    const bool beta = (lane & 4) != 0, gam = (lane & 1) != 0;
+    const int src = 8 * (lane & 3) + 2 * ((lane >> 2) & 1);
+    float dot = 0.f;
+#pragma unroll
+    for (int p = 0; p < 4; ++p) {
+      float t = gam ? (beta ? dacc[p][3] : dacc[p][2]) : (beta ? dacc[p][1] : dacc[p][0]);
+      t += __shfl_xor_sync(0xffffffffu, t, 4);
+      t += __shfl_xor_sync(0xffffffffu, t, 1);
+      const float v = __shfl_sync(0xffffffffu, t, src);
+      if ((lane >> 3) == p) dot = v;
+    }
+    const float my_dv = fired ? s * dot : 0.f;
+    if (entry < k) {
+      if (dpre_val != nullptr) dpre_val[static_cast<size_t>(row) * k + entry] = my_dv;
+      if (fired && d_b_enc != nullptr) atomicAdd(d_b_enc + my_i, my_dv);
+    }
+    cur_i = nxt_i; cur_v = nxt_v;
+    nxt_i = nn_i; nxt_v = nn_v;
+  }
+
+  __shared__ float s_sse[kWideMaxWarps];
+  __shared__ unsigned int s_l0[kWideMaxWarps];
+  const float wsum = warp_sum(sse_local);
+  if (lane == 0) {
+    s_sse[warp] = wsum;
+    s_l0[warp] = l0_local;
+  }
+  __syncthreads();
+  if (stamp_words > 0 && last_activated != nullptr)
+    for (int f = threadIdx.x; f < F; f += blockDim.x)
+      if ((s_fired[f >> 5] >> (f & 31)) & 1u) last_activated[f] = stamp;
+  if (d_b_dec != nullptr)
+    for (int i = threadIdx.x; i < d; i += blockDim.x) {
+      float t = 0.f;
+      for (int tm = 0; tm < teams; ++tm) t += fsm[d + tm * d + i];
+      atomicAdd(d_b_dec + i, s * t);
+    }
+  if (threadIdx.x == 0 && stats != nullptr) {
+    double tsum = 0.0;
+    unsigned long long c = 0;
+    for (int w = 0; w < nwarps; ++w) {
+      tsum += static_cast<double>(s_sse[w]);
+      c += s_l0[w];
+    }
+    atomicAdd(&stats->sse, tsum);
+    atomicAdd(&stats->l0_count, c);
+  }
+}
+
 // det_ws (see kDetScale*) -> d_b_enc += s * sum, d_b_dec += s * sum, stats->sse += sum
 __global__ void __launch_bounds__(256)
 det_finish_kernel(const long long* __restrict__ det_ws, int F, int d, const float* __restrict__ grad_out,
@@ -1084,8 +1385,50 @@ using namespace wsae;
 
 extern "C" int wsae_debug_decode_backward_general(int on) { g_decode_backward_general = on; return 0; }
 
-// See include/wsae.h.  Returns WSAE_E_UNSUPPORTED for shapes the fused kernel does not cover
-// (fp32 decoder, k > 32, d % 8 != 0): callers then use K2 + K3.
+// The wide form (32 < k <= 256, d % 128 == 0, no deterministic workspace).  Teams of ceil(k / 32)
+// warps, two teams per block while they fit in 4 warps, else one.
+static int decode_backward_wide(const float* target, const float* const* target_at,
+                                const long long* const* rows_at, const __nv_bfloat16* w_decT,
+                                const float* b_dec, const float* b_pre, const int32_t* idx,
+                                const float* val, const float* grad_out, float coef, int B, int d,
+                                int F, int k, float* resid, __nv_bfloat16* resid_bf16, FusedStats* stats,
+                                long long* last_activated, const long long* step_count, float* d_b_enc,
+                                float* d_b_dec, float* dpre_val, cudaStream_t stream) {
+  int dev = 0, sms = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  const int tsize = ceil_div(k, 32);
+  const int teams = tsize <= 2 ? 4 / tsize : 1;
+  const int nwarps = teams * tsize;
+  const int stamp_words = (last_activated != nullptr && F <= 65536) ? ceil_div(F, 32) : 0;
+  const size_t smem = ((1 + teams) * static_cast<size_t>(d) + 2 * nwarps * 64) * sizeof(float) +
+                      static_cast<size_t>(nwarps) * kTcGBytes + 16 + static_cast<size_t>(stamp_words) * 4;
+  if (smem > 200 * 1024) return kUnsupported;
+  static bool attr_set[64] = {};
+  if (dev >= 64 || !attr_set[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(decode_backward_wide_kernel,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    if (e != cudaSuccess) return static_cast<int>(e);
+    if (dev < 64) attr_set[dev] = true;
+  }
+  int per = 0;
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, decode_backward_wide_kernel,
+                                                                nwarps * 32, smem);
+  if (e != cudaSuccess) return static_cast<int>(e);
+  if (per < 1) per = 1;
+  int nblk = ceil_div(B, teams);
+  if (nblk > sms * per) nblk = sms * per;
+  // L2 hints as in the tensor form: decoder rows evict_last while the bf16 decoder fits in 48 MB
+  const int l2hint = static_cast<long long>(F) * d * 2 <= (48LL << 20) ? 3 : 1;
+  launch_pdl(decode_backward_wide_kernel, nblk, nwarps * 32, smem, stream, target, w_decT, b_dec, b_pre, idx,
+             val, grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated, step_count, d_b_enc,
+             d_b_dec, dpre_val, target_at, rows_at, stamp_words, l2hint);
+  return static_cast<int>(cudaGetLastError());
+}
+
+// See include/wsae.h.  Returns WSAE_E_UNSUPPORTED for shapes the fused kernels do not cover
+// (fp32 decoder, d % 8 != 0, k > 256, 32 < k with d % 128 != 0 or a deterministic workspace):
+// callers then use K2 + K3.
 static int decode_backward_impl(const float* target, const float* const* target_at,
                                 const long long* const* rows_at, long long* det_ws, const void* w_decT, int w_is_bf16, const float* b_dec,
                                 const float* b_pre, const int32_t* idx, const float* val,
@@ -1096,8 +1439,15 @@ static int decode_backward_impl(const float* target, const float* const* target_
                                 cudaStream_t stream) {
   if ((!target && !target_at) || !w_decT || !b_dec || !idx || !val) return kBadArg;
   if (B <= 0 || d <= 0 || F <= 0 || k <= 0) return kBadArg;
-  if (!w_is_bf16 || k > 32 || d % 8 != 0 || d > 8192) return kUnsupported;
+  if (!w_is_bf16 || d % 8 != 0 || d > 8192) return kUnsupported;
   if (static_cast<long long>(F) * (d / 4) > 0x7fffffffLL) return kUnsupported;
+  if (k > 32) {
+    if (k > kWideMaxK || d % 128 != 0 || det_ws != nullptr) return kUnsupported;
+    return decode_backward_wide(target, target_at, rows_at, static_cast<const __nv_bfloat16*>(w_decT), b_dec,
+                                b_pre, idx, val, grad_out, coef, B, d, F, k, resid,
+                                static_cast<__nv_bfloat16*>(resid_bf16), static_cast<FusedStats*>(stats),
+                                last_activated, step_count, d_b_enc, d_b_dec, dpre_val, stream);
+  }
   int dev = 0, sms = 0;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);

@@ -2197,6 +2197,32 @@ extern "C" int wsae_encode_topk_dense(const void* a_packed, const void* w_packed
   return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
 }
 
+// K1 for k > 64 at any batch: wsae_encode_topk_dense over row chunks of chunk_rows (a multiple of 128)
+// with one [chunk_rows, F] scratch.  The fused epilogues hold a row's candidates in registers and stop
+// at k = 64; the radix select does not.  Per chunk the GEMM reads the packed rows from a tensor map
+// based at the chunk's first row, so every 128 x 256 tile runs the same MMA sequence as in one
+// unchunked call: the results are bit-identical to it.  Chunks the size of a few tens of MB keep the
+// scratch in L2 between the GEMM that writes it and the select that reads it.
+extern "C" int wsae_encode_topk_chunked(const void* a_packed, const void* w_packed, int B, int Bp, int F,
+                                        int Fp, int Kp, int k_used_cols, int k, int chunk_rows,
+                                        float* pre_ws, float* out_val, int32_t* out_idx,
+                                        cudaStream_t stream) {
+  if (!a_packed || !out_val || !out_idx || !pre_ws) return kBadArg;
+  if (B <= 0 || Bp < B || Bp % kBM != 0 || Kp % kBK != 0) return kBadArg;
+  if (chunk_rows <= 0 || chunk_rows % kBM != 0) return kBadArg;
+  const size_t row_bytes = static_cast<size_t>(Kp) * 2;
+  for (int r0 = 0; r0 < B; r0 += chunk_rows) {
+    const int rows = B - r0 < chunk_rows ? B - r0 : chunk_rows;
+    const int rows_p = Bp - r0 < chunk_rows ? Bp - r0 : chunk_rows;
+    const int rc = wsae_encode_topk_dense(static_cast<const char*>(a_packed) + r0 * row_bytes, w_packed, rows,
+                                          rows_p, F, Fp, Kp, k_used_cols, k, pre_ws,
+                                          out_val + static_cast<size_t>(r0) * k,
+                                          out_idx + static_cast<size_t>(r0) * k, stream);
+    if (rc) return rc;
+  }
+  return kOk;
+}
+
 extern "C" int wsae_debug_encode_mode(int mode) { g_encode_dbg = mode; return 0; }
 
 // Number of F-splits wsae_encode_topk will actually use for a requested nsplit (so callers can

@@ -213,6 +213,30 @@ def choose_nsplit(B: int, F: int, k: int, num_sms: int) -> int:
 
 # rows up to which K1 runs as dense GEMM + row-wise select (wsae_encode_topk_dense); 0 switches it off
 _DENSE_ROWS = int(os.environ.get("WSAE_K1_DENSE_ROWS", "1024"))
+# the fused TopK epilogues of wsae_encode_topk keep at most 64 candidates per row
+ENCODE_FUSED_MAX_K = 64
+# fp32 scratch per chunk of the chunked route: written by the GEMM and read back by the select while
+# it is still in L2 (126 MB on a B200)
+_CHUNK_SCRATCH_BYTES = 40 << 20
+
+
+def encode_route(B: int, F: int, k: int, nsplit: int | None = None) -> str:
+    """The K1 form ``encode_topk`` runs: "dense" (one GEMM storing [B, F] + one block per row
+    selecting, batches <= WSAE_K1_DENSE_ROWS), "chunked" (the same over row chunks: k > 64 on larger
+    batches) or "fused" (the GEMM with the TopK in its epilogue, k <= 64)."""
+    dense_ok = F <= 49152 and F % 4 == 0
+    if nsplit is None and B <= _DENSE_ROWS and dense_ok:
+        return "dense"
+    if k > ENCODE_FUSED_MAX_K and dense_ok:
+        return "chunked"
+    return "fused"
+
+
+def encode_chunk_rows(B: int, F: int) -> int:
+    """Rows per chunk of the chunked K1 route: a multiple of 128 whose fp32 [rows, F] scratch fits
+    _CHUNK_SCRATCH_BYTES, no more than the batch needs."""
+    rows = max(128, _CHUNK_SCRATCH_BYTES // (F * 4) // 128 * 128)
+    return min(rows, _round_up(B, 128))
 
 
 def encode_topk(a_packed: Tensor, w_packed: Tensor, B: int, F: int, d: int, terms: int, k: int,
@@ -225,17 +249,23 @@ def encode_topk(a_packed: Tensor, w_packed: Tensor, B: int, F: int, d: int, term
     Bp, Fp = a_packed.shape[0], w_packed.shape[0]
     lib = _lib.load()
     dev = a_packed.device
-    nsplit_arg = nsplit
-    if nsplit is None:
-        nsplit = choose_nsplit(B, F, k, sm_count(dev))
-    nsplit = lib.wsae_encode_effective_splits(F, nsplit)
+    route = encode_route(B, F, k, nsplit)
     idx = torch.empty((B, k), dtype=torch.int32, device=dev)
     val = torch.empty((B, k), dtype=torch.float32, device=dev)
-    if nsplit_arg is None and B <= _DENSE_ROWS and F <= 49152 and F % 4 == 0:
+    if route == "dense":
         # small batches (the shipped YAML batch is 128 rows): dense pre-activations + one block per row
         pre = torch.empty((B, F), dtype=torch.float32, device=dev)
         _run("wsae_encode_topk", lib.wsae_encode_topk_dense, _ptr(a_packed), _ptr(w_packed), B, Bp, F, Fp, ps.kp, ps.used_cols, k, _ptr(pre), _ptr(val), _ptr(idx), _stream(), launches=2)
         return idx, val
+    if route == "chunked":
+        # the scratch is allocated per call: inside a captured train step it belongs to the graph
+        rows = encode_chunk_rows(B, F)
+        pre = torch.empty((rows, F), dtype=torch.float32, device=dev)
+        _run("wsae_encode_topk_chunked", lib.wsae_encode_topk_chunked, _ptr(a_packed), _ptr(w_packed), B, Bp, F, Fp, ps.kp, ps.used_cols, k, rows, _ptr(pre), _ptr(val), _ptr(idx), _stream(), launches=2 * ((B + rows - 1) // rows))
+        return idx, val
+    if nsplit is None:
+        nsplit = choose_nsplit(B, F, k, sm_count(dev))
+    nsplit = lib.wsae_encode_effective_splits(F, nsplit)
     pv = pi = None
     if nsplit > 1:
         pv = torch.empty((B, nsplit * k), dtype=torch.float32, device=dev)
@@ -355,9 +385,21 @@ def row_step(pre: Tensor, target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: 
     return idx, val
 
 
+# largest k of the team-of-warps K23 (wsae_decode_backward.cu, wide form)
+DECODE_BACKWARD_MAX_K = 256
+
+
 def decode_backward_supported(d: int, k: int, bf16: bool) -> bool:
-    """Shapes covered by the fused K23 kernel (else: decode_mse + backward_sparse)."""
-    return bf16 and k <= 32 and d % 8 == 0 and os.environ.get("WSAE_FUSED_DECODE", "1") != "0"
+    """Shapes covered by the fused K23 kernels (else: decode_mse + backward_sparse): k <= 32 with
+    d % 8 == 0, and 64 < k <= 256 with d % 128 == 0 (the team-of-warps form).  33 <= k <= 64 stays on
+    K2 + K3 unless WSAE_WIDE_K23=1 routes it to the team form too."""
+    if not (bf16 and d % 8 == 0 and os.environ.get("WSAE_FUSED_DECODE", "1") != "0"):
+        return False
+    if k <= 32:
+        return True
+    if d % 128 != 0 or k > DECODE_BACKWARD_MAX_K:
+        return False
+    return k > 64 or os.environ.get("WSAE_WIDE_K23", "0") == "1"
 
 
 def decode_backward(target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: Tensor | None,
@@ -422,6 +464,12 @@ def bucket_cells(B: int, F: int) -> tuple[int, int]:
     nc, nf = ctypes.c_int(), ctypes.c_int()
     _lib.check(lib.wsae_bucket_cells(B, F, ctypes.byref(nc), ctypes.byref(nf)), "wsae_bucket_cells")
     return nc.value, nf.value
+
+
+def bucket_supported(F: int, k: int) -> bool:
+    """wsae_bucket_by_tile stages one 64-row chunk (64 * k entries of 12 bytes) and the per-tile counts
+    in at most 200 KB of shared memory: k <= 256 at every Whisper width.  Larger k: K3's scatter."""
+    return (F + 127) // 128 * 4 + 64 * k * 12 <= 200 * 1024
 
 
 def bucket_by_tile(idx: Tensor, val: Tensor, dpre_val: Tensor, F: int,

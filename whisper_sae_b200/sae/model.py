@@ -227,7 +227,8 @@ class _FusedTopKSAE(torch.autograd.Function):
             d_b_dec = d_b_dec * go
             if needs[3]:
                 dpre = dpre * go
-        elif ctx.bf16 and ops.wgrad_gemm_supported(d_in) and ops.wgrad_gemm_supported(d_out):
+        elif (ctx.bf16 and ops.wgrad_gemm_supported(d_in) and ops.wgrad_gemm_supported(d_out)
+              and ops.bucket_supported(F, st.idx.shape[1])):
             resid_bf = torch.empty(st.resid.shape, dtype=torch.bfloat16, device=dev)
             ops.backward_sparse(st.resid, None, None, st.w_dec_used, st.idx, st.val, go, coef,
                                 d_w_enc=None, d_w_decT=None, d_b_enc=d_b_enc, d_b_dec=d_b_dec,

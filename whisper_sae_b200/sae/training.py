@@ -41,6 +41,12 @@ from ..data.feature_cache import IndexedBatch
 from .model import SAEOutput, TopKSAE, _fp32_terms, _SparseState
 
 
+# largest k the graphed train step (and with it data_parallel=True) serves: K1 runs fused (k <= 64)
+# or chunked, K23 up to 256 (ops.decode_backward_supported), the K4 bucketing up to ~265.  Larger k
+# trains through the autograd node, eagerly.
+GRAPH_MAX_K = 256
+
+
 @dataclass
 class TrainingMetrics:
     """Per-step metrics (training.py:19-29)."""
@@ -234,7 +240,7 @@ class _GraphedStep:
         self.state = _SparseState()
         # deterministic mode workspaces (bf16 step with K23 + K4 only)
         self.det = bool(trainer.deterministic) and self.bf16 and ops.wgrad_gemm_supported(d_in) \
-            and ops.decode_backward_supported(d_in, k_sel, True)
+            and k_sel <= 32 and ops.decode_backward_supported(d_in, k_sel, True)
         if trainer.deterministic and not self.det:
             raise RuntimeError("deterministic=True covers the bf16 (use_amp) graphed step with d % 8 == 0, k <= 32")
         self.det_k23 = self.det_k4 = self.det_sumsq = self.det_bpre = None
@@ -940,7 +946,8 @@ class SAETrainer:
         m = self.model
         if not (self.cuda_graph and isinstance(m, TopKSAE) and type(m).forward is TopKSAE.forward
                 and batch.dim() == 2 and batch.shape[1] == m.input_dim and m.input_dim % 4 == 0
-                and batch.dtype == torch.float32 and m.k <= 64 and m.precision is None):
+                and batch.dtype == torch.float32 and m.k <= GRAPH_MAX_K
+                and ops.bucket_supported(m.hidden_dim, m.k) and m.precision is None):
             return False
         # the five parameters by attribute (Module.parameters() walks the module tree: ~10 us per call)
         return (m.b_pre.requires_grad and m.encoder.weight.requires_grad and m.encoder.bias.requires_grad
