@@ -35,7 +35,15 @@ typedef void* wsae_stream_t; /* cudaStream_t */
 
 /* Library / build identification: returns 100 * major + minor of the ABI (currently 111: + wsae_encode_topk_dense, wsae_encode_dense, wsae_row_step with the fused counters, wsae_graph_launch, wsae_memcpy_async; later
  * additions that change no existing behaviour keep the number: wsae_encode_topk_chunked, and k up to 256 in
- * wsae_decode_backward / _at / _rows_at). */
+ * wsae_decode_backward / _at / _rows_at; the half-precision activation forms wsae_pack_activations_typed,
+ * wsae_decode_backward_typed, wsae_row_step_typed and wsae_layernorm_rows_typed, whose dtype 0 is the
+ * existing entry point).
+ *
+ * Activation dtype codes (x_dtype / in_dtype / out_dtype): 0 = float32, 1 = bfloat16, 2 = float16.  A
+ * bf16 / fp16 activation matrix is converted to fp32 as it is loaded, and everything after the load is
+ * the fp32 arithmetic: a half matrix Xh gives bit for bit what its fp32 copy Xh.float() gives.  A form
+ * that cannot read the given dtype returns WSAE_E_UNSUPPORTED (it never reinterprets the bytes); an
+ * unknown code is WSAE_E_BADARG. */
 int wsae_abi_version(void);
 
 /* cudaGraphLaunch(graph_exec, stream) for an instantiated CUDA graph of the calls below (the host mirror
@@ -68,6 +76,11 @@ int wsae_pack_activations_at(const float* const* x_at, const float* b_pre /*null
 int wsae_pack_activations_rows_at(const float* const* x_at, const long long* const* rows_at,
                                   const float* b_pre /*nullable*/, int B, int Bp, int d, int terms,
                                   void* a_packed /*bf16 [Bp,Kp]*/, wsae_stream_t stream);
+/* Slot form for any activation dtype: *x_at holds B x d elements of type x_dtype (16-byte aligned);
+ * rows_at nullable (and *rows_at == NULL: identity).  terms == 1 and d % 8 == 0 only. */
+int wsae_pack_activations_typed(const void* const* x_at, const long long* const* rows_at /*nullable*/,
+                                int x_dtype, const float* b_pre /*nullable*/, int B, int Bp, int d, int terms,
+                                void* a_packed /*bf16 [Bp,Kp]*/, wsae_stream_t stream);
 int wsae_pack_encoder(const float* w_enc /*[F,d]*/, const float* b_enc /*[F] nullable*/, int F,
                       int Fp, int d, int terms, void* w_packed /*bf16 [Fp,Kp]*/,
                       wsae_stream_t stream);
@@ -128,6 +141,15 @@ int wsae_row_step(const float* pre, const float* target, const float* const* tar
                   float* d_w_decT, float* resid, float* dpre_val, const float* w_enc, float* d_b_pre,
                   unsigned int* ticket, long long dead_threshold, long long* dead_count,
                   const long long* seq, long long* mailbox, wsae_stream_t stream);
+/* As wsae_row_step, with target / *target_at of element type x_dtype. */
+int wsae_row_step_typed(const float* pre, const void* target, const void* const* target_at,
+                        const long long* const* rows_at, int x_dtype, const void* w_decT_bf16, const float* b_dec,
+                        const float* b_pre, const float* grad_out, float coef, int B, int d, int F, int k,
+                        float* out_val, int32_t* out_idx, void* stats, long long* last_activated,
+                        long long* step_count, float* d_b_enc, float* d_b_dec, float* d_w_enc,
+                        float* d_w_decT, float* resid, float* dpre_val, const float* w_enc, float* d_b_pre,
+                        unsigned int* ticket, long long dead_threshold, long long* dead_count,
+                        const long long* seq, long long* mailbox, wsae_stream_t stream);
 
 /* ---- K2: k-sparse decode + MSE + L0 + fired stamps (sae/model.py:116,129,145,148,174-181) -----
  * recon = sum_j relu(val_j) * W_decT[idx_j,:] + b_dec (+ b_pre);  resid = recon - target.
@@ -191,6 +213,17 @@ int wsae_decode_backward_rows_at(const float* const* target_at, const long long*
                                  int k, float* resid, void* resid_bf16, void* stats,
                                  long long* last_activated, const long long* step_count,
                                  float* d_b_enc, float* d_b_dec, float* dpre_val, wsae_stream_t stream);
+/* Slot form for any target dtype: *target_at holds elements of type x_dtype (16-byte aligned); rows_at
+ * nullable (as in wsae_decode_backward_rows_at); det_ws nullable (non-NULL: wsae_decode_backward_det's
+ * deterministic accumulation, finished by wsae_det_finish).  Covers every K23 form (warp, staged, tensor,
+ * team). */
+int wsae_decode_backward_typed(const void* const* target_at, const long long* const* rows_at /*nullable*/,
+                               int x_dtype, const void* w_decT, int w_is_bf16, const float* b_dec,
+                               const float* b_pre /*nullable*/, const int32_t* idx, const float* val,
+                               const float* grad_out /*nullable*/, float coef, int B, int d, int F, int k,
+                               float* resid, void* resid_bf16, void* stats, long long* last_activated,
+                               const long long* step_count, float* d_b_enc, float* d_b_dec, float* dpre_val,
+                               long long* det_ws /*nullable*/, wsae_stream_t stream);
 /* out[idx[b,j], :] += vals[b,j] * (rows[b,:] - center): the encoder weight gradient as a sparse
  * scatter when the input width differs from the decoder width (transcoders); dr % 4 == 0. */
 int wsae_scatter_rows(const float* rows, const float* center /*nullable*/, const int32_t* idx,
@@ -307,6 +340,11 @@ int wsae_feature_topk_update(const int32_t* feat, const float* val, const int32_
 int wsae_layernorm_rows(const void* x, int in_dtype, long long rows, int d, long long in_pitch_elems,
                         const float* gamma /*nullable*/, const float* beta /*nullable*/, float eps,
                         float* out, long long out_pitch_elems, wsae_stream_t stream);
+/* As wsae_layernorm_rows, writing elements of type out_dtype: the statistics and the normalised value are
+ * fp32 as above, rounded to nearest at the store. */
+int wsae_layernorm_rows_typed(const void* x, int in_dtype, long long rows, int d, long long in_pitch_elems,
+                              const float* gamma /*nullable*/, const float* beta /*nullable*/, float eps,
+                              void* out, int out_dtype, long long out_pitch_elems, wsae_stream_t stream);
 
 /* ---- deterministic accumulation mode (SAETrainer(..., deterministic=True)) ----------------------
  * The default kernels add their cross-row / split-K partial sums with float atomics in arrival

@@ -63,6 +63,7 @@ _SIGNATURES = {
     "wsae_pack_activations": ([c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p], c_int),
     "wsae_pack_activations_at": ([c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p], c_int),
     "wsae_pack_activations_rows_at": ([c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p], c_int),
+    "wsae_pack_activations_typed": ([c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p], c_int),
     "wsae_pack_encoder": ([c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p], c_int),
     "wsae_encode_effective_splits": ([c_int, c_int], c_int),
     "wsae_encode_topk": (
@@ -87,6 +88,13 @@ _SIGNATURES = {
     ),
     "wsae_row_step": (
         [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
+         c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p,
+         c_void_p, c_void_p],
+        c_int,
+    ),
+    "wsae_row_step_typed": (
+        [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
          c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_longlong, c_void_p, c_void_p,
          c_void_p, c_void_p],
@@ -128,6 +136,12 @@ _SIGNATURES = {
          c_void_p, c_void_p, c_void_p, c_void_p],
         c_int,
     ),
+    "wsae_decode_backward_typed": (
+        [c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float,
+         c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_void_p, c_void_p],
+        c_int,
+    ),
     "wsae_det_finish": ([c_void_p, c_int, c_int, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p], c_int),
     "wsae_wgrad_gemm_workspace": ([c_int, c_int, c_int, POINTER(c_ulonglong)], c_int),
     "wsae_wgrad_gemm_det": (
@@ -164,6 +178,8 @@ _SIGNATURES = {
     "wsae_sumsq": ([c_void_p, c_longlong, c_void_p, c_void_p], c_int),
     "wsae_layernorm_rows": ([c_void_p, c_int, c_longlong, c_int, c_longlong, c_void_p, c_void_p, c_float,
                              c_void_p, c_longlong, c_void_p], c_int),
+    "wsae_layernorm_rows_typed": ([c_void_p, c_int, c_longlong, c_int, c_longlong, c_void_p, c_void_p, c_float,
+                                   c_void_p, c_int, c_longlong, c_void_p], c_int),
     "wsae_feature_topk_workspace": ([c_longlong, c_int, POINTER(c_ulonglong)], c_int),
     "wsae_feature_topk_update": (
         [c_void_p, c_void_p, c_void_p, c_longlong, c_int, c_void_p, c_longlong, c_void_p, c_int, c_int,

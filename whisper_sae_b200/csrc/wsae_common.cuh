@@ -6,8 +6,10 @@
 
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <cstdlib>
+#include <type_traits>
 
 #ifndef WSAE_SPIN_LIMIT
 // Bounded spin on mbarrier waits: a broken pipeline traps (CUDA error) instead of hanging the GPU.
@@ -332,6 +334,51 @@ __device__ __forceinline__ float4 bf16x4_to_float4(uint2 u) {
   f.z = __uint_as_float(u.y << 16);
   f.w = __uint_as_float(u.y & 0xFFFF0000u);
   return f;
+}
+
+// ----------------------------------------------------------------------------------------------
+// activation element types: the kernels that read the activation matrix (K0, K23, the row step) are
+// templated on its element type TX = float / __nv_bfloat16 / __half (dtype code 0 / 1 / 2, as in
+// wsae_layernorm_rows).  A half value converts to fp32 exactly, and the conversion happens at the
+// load: the arithmetic after it is the fp32 kernel's, so a half matrix trains bit for bit like its
+// fp32 copy.  The loads below are the fp32 kernels' loads for TX = float.
+// ----------------------------------------------------------------------------------------------
+__device__ __forceinline__ float2 x2_to_float2(uint32_t u, const __nv_bfloat16*) {
+  return make_float2(__uint_as_float(u << 16), __uint_as_float(u & 0xFFFF0000u));
+}
+__device__ __forceinline__ float2 x2_to_float2(uint32_t u, const __half*) {
+  return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
+template <typename TX>
+__device__ __forceinline__ float4 x4_to_float4(uint2 u) {
+  const float2 lo = x2_to_float2(u.x, static_cast<const TX*>(nullptr));
+  const float2 hi = x2_to_float2(u.y, static_cast<const TX*>(nullptr));
+  return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
+
+// 4 consecutive elements (16-byte aligned for fp32, 8-byte for half types), read-only path
+__device__ __forceinline__ float4 ldg_x4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+template <typename TX>
+__device__ __forceinline__ float4 ldg_x4(const TX* p) {
+  return x4_to_float4<TX>(__ldg(reinterpret_cast<const uint2*>(p)));
+}
+// 2 consecutive elements, plain load
+__device__ __forceinline__ float2 ld_x2(const float* p) { return *reinterpret_cast<const float2*>(p); }
+template <typename TX>
+__device__ __forceinline__ float2 ld_x2(const TX* p) {
+  return x2_to_float2(*reinterpret_cast<const uint32_t*>(p), p);
+}
+
+// Host side: fn(static_cast<const TX*>(nullptr)) for the element type of dtype code x_dtype;
+// kBadArg for a code that names none.
+template <typename Fn>
+inline int with_x_dtype(int x_dtype, Fn&& fn) {
+  switch (x_dtype) {
+    case 0: return fn(static_cast<const float*>(nullptr));
+    case 1: return fn(static_cast<const __nv_bfloat16*>(nullptr));
+    case 2: return fn(static_cast<const __half*>(nullptr));
+    default: return kBadArg;
+  }
 }
 
 }  // namespace wsae

@@ -111,9 +111,10 @@ constexpr int kDotScratch = 32 * 9;   // floats per warp: 32 dot products x 8 pa
 // partial dot product over block g.  Sixteen HMMA per slice replace 128 FHFMA, the accumulators
 // stay in registers across the slices, and the diagonal is summed through 1.1 KB of shared memory
 // per warp instead of a 31-step shuffle transpose.
-template <bool kFast>
+// TX: element type of the target matrix (float / __nv_bfloat16 / __half, converted at the load).
+template <bool kFast, typename TX>
 __global__ void __launch_bounds__(kFusedWarps * 32, kFast ? 3 : 4)
-decode_backward_kernel(const float* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
+decode_backward_kernel(const TX* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
                        const float* __restrict__ b_dec, const float* __restrict__ b_pre,
                        const int32_t* __restrict__ idx, const float* __restrict__ val,
                        const float* __restrict__ grad_out, float coef, int B, int d, int F, int k,
@@ -121,7 +122,7 @@ decode_backward_kernel(const float* __restrict__ target, const __nv_bfloat16* __
                        FusedStats* __restrict__ stats, long long* __restrict__ last_activated,
                        const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
                        float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
-                       const float* const* __restrict__ target_at,
+                       const TX* const* __restrict__ target_at,
                        const long long* const* __restrict__ rows_at, int stamp_words,
                        long long* __restrict__ det_ws) {
   extern __shared__ __align__(16) float fsm[];   // [dp] bias (b_dec + b_pre), then one [dp] db_dec accumulator per warp
@@ -189,7 +190,7 @@ decode_backward_kernel(const float* __restrict__ target, const __nv_bfloat16* __
       for (int p = 0; p < 16; ++p) acc[p][0] = acc[p][1] = acc[p][2] = acc[p][3] = 0.f;
       const uint2* lane_base = wbase + lane;
       const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
-      const float* trow = target + srow * d + lane * 4;
+      const TX* trow = target + srow * d + lane * 4;
       for (int c0 = 0; c0 < d; c0 += 128) {
         const uint2* sb = lane_base + (c0 >> 2);
         uint2 w[32];
@@ -198,7 +199,7 @@ decode_backward_kernel(const float* __restrict__ target, const __nv_bfloat16* __
           const uint32_t off = __shfl_sync(0xffffffffu, static_cast<uint32_t>(my_off), j);
           w[j] = __ldg(sb + off);
         }
-        const float4 t = __ldg(reinterpret_cast<const float4*>(trow + c0));
+        const float4 t = ldg_x4(trow + c0);
         float4 a = *reinterpret_cast<const float4*>(s_bias + c0 + lane * 4);
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
@@ -273,7 +274,7 @@ decode_backward_kernel(const float* __restrict__ target, const __nv_bfloat16* __
       float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
       if (ok) {
         const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
-        t = __ldg(reinterpret_cast<const float4*>(target + srow * d + col));
+        t = ldg_x4(target + srow * d + col);
       }
       float4 acc = *reinterpret_cast<const float4*>(s_bias + col);
       // ---- reconstruction of this slice (fp32) ----
@@ -392,9 +393,9 @@ __device__ __forceinline__ void cp_async_wait() {
 
 constexpr int kSliceBytes = 32 * 256;   // one staged slice: 32 gathered rows x 128 bf16 columns
 
-template <int STAGES>
+template <int STAGES, typename TX>
 __global__ void __launch_bounds__(kFusedWarps * 32, STAGES == 2 ? 3 : 2)
-decode_backward_staged_kernel(const float* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
+decode_backward_staged_kernel(const TX* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
                               const float* __restrict__ b_dec, const float* __restrict__ b_pre,
                               const int32_t* __restrict__ idx, const float* __restrict__ val,
                               const float* __restrict__ grad_out, float coef, int B, int d, int F, int k,
@@ -402,7 +403,7 @@ decode_backward_staged_kernel(const float* __restrict__ target, const __nv_bfloa
                               FusedStats* __restrict__ stats, long long* __restrict__ last_activated,
                               const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
                               float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
-                              const float* const* __restrict__ target_at,
+                              const TX* const* __restrict__ target_at,
                               const long long* const* __restrict__ rows_at, int stamp_words,
                               long long* __restrict__ det_ws, int dbg) {
   extern __shared__ __align__(16) float fsm[];   // [d] bias, [warps][d] db_dec partials, the slice rings, the fired bitmap
@@ -499,7 +500,7 @@ decode_backward_staged_kernel(const float* __restrict__ target, const __nv_bfloa
     const uint32_t mask = __ballot_sync(0xffffffffu, fired);
     l0_local += (lane == 0) ? __popc(mask) : 0;
     const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
-    const float* trow = target + srow * d + lane * 4;
+    const TX* trow = target + srow * d + lane * 4;
     int32_t nn_i = -1;     // metadata two rows ahead: requested after the first slice's copies are
     float nn_v = 0.f;      // out (not at the top of the row, where ptxas made the target address wait
                            // for it: 11 % of all stall samples), consumed when this row is done
@@ -510,7 +511,7 @@ decode_backward_staged_kernel(const float* __restrict__ target, const __nv_bfloa
 
     for (int sl = 0; sl < nsl; ++sl) {
       float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (!(dbg & 1)) t = __ldg(reinterpret_cast<const float4*>(trow + sl * 128));
+      if (!(dbg & 1)) t = ldg_x4(trow + sl * 128);
       cp_async_wait<STAGES - 2>();             // slice (row, sl) has landed (this lane's copies)
       __syncwarp();                            // ... and every other lane's; the stage consumed last is free
       {   // keep the ring full: slice sl + STAGES - 1 of this row, or of the next one
@@ -699,6 +700,28 @@ __device__ __forceinline__ float2 ldg_stream_v2(const float* p, uint64_t pol) {
                : "l"(p), "l"(pol));
   return v;
 }
+// The 2 target columns a lane of the tensor / team forms holds in flight, as loaded: fp32 pairs are
+// loaded as float2 (8 bytes), half pairs as their raw 4 bytes and converted where they are used, so the
+// load never waits on its own conversion.
+template <typename TX>
+struct XPair {
+  using type = uint32_t;
+};
+template <>
+struct XPair<float> {
+  using type = float2;
+};
+__device__ __forceinline__ float2 ldg_stream_x2(const float* p, uint64_t pol) { return ldg_stream_v2(p, pol); }
+template <typename TX>
+__device__ __forceinline__ uint32_t ldg_stream_x2(const TX* p, uint64_t pol) {
+  uint32_t v;
+  asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+  return v;
+}
+__device__ __forceinline__ float2 xpair_to_float2(float2 v, const float*) { return v; }
+template <typename TX>
+__device__ __forceinline__ float2 xpair_to_float2(uint32_t v, const TX* tag) { return x2_to_float2(v, tag); }
+
 // acc[0..3] += bf16x2(w0).{lo,hi}, bf16x2(w1).{lo,hi} times bf16(h.lo)
 __device__ __forceinline__ void fhfma_row4(float* acc, uint32_t w0, uint32_t w1, uint32_t h) {
   asm("{\n\t"
@@ -733,9 +756,9 @@ __device__ __forceinline__ void fhfma_row4_hi(float* acc, uint32_t w0, uint32_t 
 
 // STAGES half slices live in registers: one being multiplied, STAGES - 1 in flight (d / 64 must be a
 // multiple of STAGES).
-template <int kMinBlocks, int STAGES, bool PF>
+template <int kMinBlocks, int STAGES, bool PF, typename TX>
 __global__ void __launch_bounds__(kFusedWarps * 32, kMinBlocks)
-decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
+decode_backward_tc_kernel(const TX* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
                           const float* __restrict__ b_dec, const float* __restrict__ b_pre,
                           const int32_t* __restrict__ idx, const float* __restrict__ val,
                           const float* __restrict__ grad_out, float coef, int B, int d, int F, int k,
@@ -743,7 +766,7 @@ decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16*
                           FusedStats* __restrict__ stats, long long* __restrict__ last_activated,
                           const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
                           float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
-                          const float* const* __restrict__ target_at,
+                          const TX* const* __restrict__ target_at,
                           const long long* const* __restrict__ rows_at, int stamp_words,
                           long long* __restrict__ det_ws, int pf_dist, int l2hint) {
   static_assert(STAGES == 2 || STAGES == 3, "two or three half slices in registers");
@@ -819,15 +842,16 @@ decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16*
       wp[i] = wbytes + static_cast<size_t>(f) * row_bytes + chi * 16;
     }
   };
-  const float* trow = target;                // this lane's 2 target columns, at the current half slice
+  using XP = typename XPair<TX>::type;
+  const TX* trow = target;                   // this lane's 2 target columns, at the current half slice
   auto set_target = [&](int row) {
     const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
     trow = target + srow * d + c0;
   };
-  auto gather = [&](uint4 (&w)[8], float2& x, int ahead) {     // `ahead` half slices past the current one
+  auto gather = [&](uint4 (&w)[8], XP& x, int ahead) {     // `ahead` half slices past the current one
 #pragma unroll
     for (int i = 0; i < 8; ++i) w[i] = ldg_nc_v4<PF>(wp[i] + ahead * 128, pol_w);
-    x = ldg_stream_v2(trow + ahead * 64, pol_x);
+    x = ldg_stream_x2(trow + ahead * 64, pol_x);
   };
   // PF: every lane asks for ONE 128-byte line of ITS entry's row, pf_dist half slices past the one
   // being gathered - a single instruction per half slice brings all 32 lines (4 KB) into L1 without
@@ -855,7 +879,7 @@ decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16*
   load_meta(row, cur_i, cur_v);
   load_meta(row + warp_stride, nxt_i, nxt_v);
   uint4 w0[8], w1[8], w2[8];   // w2: three-stage form only (dead otherwise)
-  float2 x0 = make_float2(0.f, 0.f), x1 = x0, x2 = x0;
+  XP x0{}, x1 = x0, x2 = x0;
   if (row < B) {
     set_row(gather_feature(cur_i, row));
     set_target(row);
@@ -895,7 +919,8 @@ decode_backward_tc_kernel(const float* __restrict__ target, const __nv_bfloat16*
 #pragma unroll
     for (int p = 0; p < 4; ++p) dacc[p][0] = dacc[p][1] = dacc[p][2] = dacc[p][3] = 0.f;
 
-    auto compute = [&](const uint4 (&w)[8], const float2 x, int hs) {
+    auto compute = [&](const uint4 (&w)[8], const XP xp, int hs) {
+      const float2 x = xpair_to_float2(xp, static_cast<const TX*>(nullptr));
       // ---- reconstruction partials: 8 entries x 8 columns in this lane ----
       float part[8];
 #pragma unroll
@@ -1085,8 +1110,9 @@ __device__ __forceinline__ void team_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
+template <typename TX>
 __global__ void __maxnreg__(160)   // 156 registers, no spills: the tensor form's budget
-decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
+decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
                             const float* __restrict__ b_dec, const float* __restrict__ b_pre,
                             const int32_t* __restrict__ idx, const float* __restrict__ val,
                             const float* __restrict__ grad_out, float coef, int B, int d, int F, int k,
@@ -1094,7 +1120,7 @@ decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat1
                             FusedStats* __restrict__ stats, long long* __restrict__ last_activated,
                             const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
                             float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
-                            const float* const* __restrict__ target_at,
+                            const TX* const* __restrict__ target_at,
                             const long long* const* __restrict__ rows_at, int stamp_words, int l2hint) {
   const uint64_t pol_x = l2_policy((l2hint & 1) ? 1 : 0);
   const uint64_t pol_w = l2_policy((l2hint & 2) ? 2 : 0);
@@ -1169,15 +1195,16 @@ decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat1
       wp[i] = wbytes + static_cast<size_t>(f) * row_bytes + chi * 16;
     }
   };
-  const float* trow = target;
+  using XP = typename XPair<TX>::type;
+  const TX* trow = target;
   auto set_target = [&](int row) {
     const size_t srow = perm != nullptr ? static_cast<size_t>(__ldg(perm + row)) : static_cast<size_t>(row);
     trow = target + srow * d + c0;
   };
-  auto gather = [&](uint4 (&w)[8], float2& x, int ahead) {
+  auto gather = [&](uint4 (&w)[8], XP& x, int ahead) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) w[i] = ldg_nc_v4<false>(wp[i] + ahead * 128, pol_w);
-    x = ldg_stream_v2(trow + ahead * 64, pol_x);
+    x = ldg_stream_x2(trow + ahead * 64, pol_x);
   };
   auto advance = [&](int n) {
 #pragma unroll
@@ -1191,7 +1218,7 @@ decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat1
   load_meta(row, cur_i, cur_v);
   load_meta(row + team_stride, nxt_i, nxt_v);
   uint4 w0[8], w1[8];
-  float2 x0 = make_float2(0.f, 0.f), x1 = x0;
+  XP x0{}, x1 = x0;
   if (row < B) {
     set_row(gather_feature(cur_i, row));
     set_target(row);
@@ -1225,7 +1252,8 @@ decode_backward_wide_kernel(const float* __restrict__ target, const __nv_bfloat1
 #pragma unroll
     for (int p = 0; p < 4; ++p) dacc[p][0] = dacc[p][1] = dacc[p][2] = dacc[p][3] = 0.f;
 
-    auto compute = [&](const uint4 (&w)[8], const float2 x, int hs) {
+    auto compute = [&](const uint4 (&w)[8], const XP xp, int hs) {
+      const float2 x = xpair_to_float2(xp, static_cast<const TX*>(nullptr));
       float part[8];
 #pragma unroll
       for (int c = 0; c < 8; ++c) part[c] = 0.f;
@@ -1387,7 +1415,8 @@ extern "C" int wsae_debug_decode_backward_general(int on) { g_decode_backward_ge
 
 // The wide form (32 < k <= 256, d % 128 == 0, no deterministic workspace).  Teams of ceil(k / 32)
 // warps, two teams per block while they fit in 4 warps, else one.
-static int decode_backward_wide(const float* target, const float* const* target_at,
+template <typename TX>
+static int decode_backward_wide(const TX* target, const TX* const* target_at,
                                 const long long* const* rows_at, const __nv_bfloat16* w_decT,
                                 const float* b_dec, const float* b_pre, const int32_t* idx,
                                 const float* val, const float* grad_out, float coef, int B, int d,
@@ -1406,13 +1435,13 @@ static int decode_backward_wide(const float* target, const float* const* target_
   if (smem > 200 * 1024) return kUnsupported;
   static bool attr_set[64] = {};
   if (dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(decode_backward_wide_kernel,
+    cudaError_t e = cudaFuncSetAttribute(decode_backward_wide_kernel<TX>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return static_cast<int>(e);
     if (dev < 64) attr_set[dev] = true;
   }
   int per = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, decode_backward_wide_kernel,
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, decode_backward_wide_kernel<TX>,
                                                                 nwarps * 32, smem);
   if (e != cudaSuccess) return static_cast<int>(e);
   if (per < 1) per = 1;
@@ -1420,7 +1449,7 @@ static int decode_backward_wide(const float* target, const float* const* target_
   if (nblk > sms * per) nblk = sms * per;
   // L2 hints as in the tensor form: decoder rows evict_last while the bf16 decoder fits in 48 MB
   const int l2hint = static_cast<long long>(F) * d * 2 <= (48LL << 20) ? 3 : 1;
-  launch_pdl(decode_backward_wide_kernel, nblk, nwarps * 32, smem, stream, target, w_decT, b_dec, b_pre, idx,
+  launch_pdl(decode_backward_wide_kernel<TX>, nblk, nwarps * 32, smem, stream, target, w_decT, b_dec, b_pre, idx,
              val, grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated, step_count, d_b_enc,
              d_b_dec, dpre_val, target_at, rows_at, stamp_words, l2hint);
   return static_cast<int>(cudaGetLastError());
@@ -1428,15 +1457,16 @@ static int decode_backward_wide(const float* target, const float* const* target_
 
 // See include/wsae.h.  Returns WSAE_E_UNSUPPORTED for shapes the fused kernels do not cover
 // (fp32 decoder, d % 8 != 0, k > 256, 32 < k with d % 128 != 0 or a deterministic workspace):
-// callers then use K2 + K3.
-static int decode_backward_impl(const float* target, const float* const* target_at,
-                                const long long* const* rows_at, long long* det_ws, const void* w_decT, int w_is_bf16, const float* b_dec,
-                                const float* b_pre, const int32_t* idx, const float* val,
-                                const float* grad_out, float coef, int B, int d, int F, int k,
-                                float* resid, void* resid_bf16, void* stats,
-                                long long* last_activated, const long long* step_count,
-                                float* d_b_enc, float* d_b_dec, float* dpre_val,
-                                cudaStream_t stream) {
+// callers then use K2 + K3.  TX: element type of the target matrix.
+template <typename TX>
+static int decode_backward_launch(const TX* target, const TX* const* target_at,
+                                  const long long* const* rows_at, long long* det_ws, const void* w_decT, int w_is_bf16, const float* b_dec,
+                                  const float* b_pre, const int32_t* idx, const float* val,
+                                  const float* grad_out, float coef, int B, int d, int F, int k,
+                                  float* resid, void* resid_bf16, void* stats,
+                                  long long* last_activated, const long long* step_count,
+                                  float* d_b_enc, float* d_b_dec, float* dpre_val,
+                                  cudaStream_t stream) {
   if ((!target && !target_at) || !w_decT || !b_dec || !idx || !val) return kBadArg;
   if (B <= 0 || d <= 0 || F <= 0 || k <= 0) return kBadArg;
   if (!w_is_bf16 || d % 8 != 0 || d > 8192) return kUnsupported;
@@ -1462,10 +1492,10 @@ static int decode_backward_impl(const float* target, const float* const* target_
   if (smem > 48 * 1024) {      // d > 2432: opt in to the large dynamic shared-memory carve-out (once per device)
     static bool attr_set[64] = {};
     if (dev >= 64 || !attr_set[dev]) {
-      cudaError_t e = cudaFuncSetAttribute(decode_backward_kernel<true>,
+      cudaError_t e = cudaFuncSetAttribute(decode_backward_kernel<true, TX>,
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
       if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(decode_backward_kernel<false>,
+        e = cudaFuncSetAttribute(decode_backward_kernel<false, TX>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
       if (e != cudaSuccess) return static_cast<int>(e);
       if (dev < 64) attr_set[dev] = true;
@@ -1520,16 +1550,16 @@ static int decode_backward_impl(const float* target, const float* const* target_
       return e ? std::atoi(e) : -1;
     }();
     const int l2hint = l2_env >= 0 ? l2_env : (static_cast<long long>(F) * d * 2 <= (48LL << 20) ? 3 : 1);
-    using KernT = decltype(&decode_backward_tc_kernel<3, 2, false>);
-    KernT kern = stages == 3 ? decode_backward_tc_kernel<3, 3, false>
-                             : (per_want == 4 ? (pf_dist > 0 ? decode_backward_tc_kernel<4, 2, true> : decode_backward_tc_kernel<4, 2, false>)
-                                              : (pf_dist > 0 ? decode_backward_tc_kernel<3, 2, true> : decode_backward_tc_kernel<3, 2, false>));
+    using KernT = decltype(&decode_backward_tc_kernel<3, 2, false, TX>);
+    KernT kern = stages == 3 ? decode_backward_tc_kernel<3, 3, false, TX>
+                             : (per_want == 4 ? (pf_dist > 0 ? decode_backward_tc_kernel<4, 2, true, TX> : decode_backward_tc_kernel<4, 2, false, TX>)
+                                              : (pf_dist > 0 ? decode_backward_tc_kernel<3, 2, true, TX> : decode_backward_tc_kernel<3, 2, false, TX>));
     static bool attr_tc[64] = {};
     if (dev >= 64 || !attr_tc[dev]) {
       cudaError_t e = cudaSuccess;
-      for (KernT kf : {decode_backward_tc_kernel<4, 2, false>, decode_backward_tc_kernel<4, 2, true>,
-                       decode_backward_tc_kernel<3, 2, false>, decode_backward_tc_kernel<3, 2, true>,
-                       decode_backward_tc_kernel<3, 3, false>})
+      for (KernT kf : {decode_backward_tc_kernel<4, 2, false, TX>, decode_backward_tc_kernel<4, 2, true, TX>,
+                       decode_backward_tc_kernel<3, 2, false, TX>, decode_backward_tc_kernel<3, 2, true, TX>,
+                       decode_backward_tc_kernel<3, 3, false, TX>})
         if (e == cudaSuccess)
           e = cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
       if (e != cudaSuccess) return static_cast<int>(e);
@@ -1564,10 +1594,10 @@ static int decode_backward_impl(const float* target, const float* const* target_
     const size_t smem_s = base + static_cast<size_t>(kFusedWarps) * stages * kSliceBytes;
     static bool attr_staged[64] = {};
     if (dev >= 64 || !attr_staged[dev]) {
-      cudaError_t e = cudaFuncSetAttribute(decode_backward_staged_kernel<3>,
+      cudaError_t e = cudaFuncSetAttribute(decode_backward_staged_kernel<3, TX>,
                                            cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
       if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(decode_backward_staged_kernel<2>,
+        e = cudaFuncSetAttribute(decode_backward_staged_kernel<2, TX>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
       if (e != cudaSuccess) return static_cast<int>(e);
       if (dev < 64) attr_staged[dev] = true;
@@ -1579,11 +1609,11 @@ static int decode_backward_impl(const float* target, const float* const* target_
       int nblk = ceil_div(B, kFusedWarps);
       if (nblk > sms * per) nblk = sms * per;
       if (stages == 3)
-        launch_pdl(decode_backward_staged_kernel<3>, nblk, kFusedWarps * 32, smem_s, stream, target, wd, b_dec,
+        launch_pdl(decode_backward_staged_kernel<3, TX>, nblk, kFusedWarps * 32, smem_s, stream, target, wd, b_dec,
                    b_pre, idx, val, grad_out, coef, B, d, F, k, resid, rbf, st, last_activated, step_count,
                    d_b_enc, d_b_dec, dpre_val, target_at, rows_at, stamp_words, det_ws, dbg);
       else
-        launch_pdl(decode_backward_staged_kernel<2>, nblk, kFusedWarps * 32, smem_s, stream, target, wd, b_dec,
+        launch_pdl(decode_backward_staged_kernel<2, TX>, nblk, kFusedWarps * 32, smem_s, stream, target, wd, b_dec,
                    b_pre, idx, val, grad_out, coef, B, d, F, k, resid, rbf, st, last_activated, step_count,
                    d_b_enc, d_b_dec, dpre_val, target_at, rows_at, stamp_words, det_ws, dbg);
       return static_cast<int>(cudaGetLastError());
@@ -1591,16 +1621,33 @@ static int decode_backward_impl(const float* target, const float* const* target_
   }
   const bool fast = (d % 128 == 0) && (mode == 2 || (mode == 0 && d <= 1024));
   if (fast)
-    launch_pdl(decode_backward_kernel<true>, blocks, kFusedWarps * 32, smem, stream, target,
+    launch_pdl(decode_backward_kernel<true, TX>, blocks, kFusedWarps * 32, smem, stream, target,
                static_cast<const __nv_bfloat16*>(w_decT), b_dec, b_pre, idx, val, grad_out, coef, B, d,
                F, k, resid, static_cast<__nv_bfloat16*>(resid_bf16), static_cast<FusedStats*>(stats),
                last_activated, step_count, d_b_enc, d_b_dec, dpre_val, target_at, rows_at, stamp_words, det_ws);
   else
-    launch_pdl(decode_backward_kernel<false>, blocks, kFusedWarps * 32, smem, stream, target,
+    launch_pdl(decode_backward_kernel<false, TX>, blocks, kFusedWarps * 32, smem, stream, target,
                static_cast<const __nv_bfloat16*>(w_decT), b_dec, b_pre, idx, val, grad_out, coef, B, d,
                F, k, resid, static_cast<__nv_bfloat16*>(resid_bf16), static_cast<FusedStats*>(stats),
                last_activated, step_count, d_b_enc, d_b_dec, dpre_val, target_at, rows_at, stamp_words, det_ws);
   return static_cast<int>(cudaGetLastError());
+}
+
+// x_dtype (0 = fp32, 1 = bf16, 2 = fp16) names the element type of the target matrix.
+static int decode_backward_impl(const void* target, const void* const* target_at, int x_dtype,
+                                const long long* const* rows_at, long long* det_ws, const void* w_decT,
+                                int w_is_bf16, const float* b_dec, const float* b_pre, const int32_t* idx,
+                                const float* val, const float* grad_out, float coef, int B, int d, int F, int k,
+                                float* resid, void* resid_bf16, void* stats, long long* last_activated,
+                                const long long* step_count, float* d_b_enc, float* d_b_dec, float* dpre_val,
+                                cudaStream_t stream) {
+  return with_x_dtype(x_dtype, [&](auto tag) {
+    using TX = std::remove_cv_t<std::remove_pointer_t<decltype(tag)>>;
+    return decode_backward_launch<TX>(static_cast<const TX*>(target), reinterpret_cast<const TX* const*>(target_at),
+                                      rows_at, det_ws, w_decT, w_is_bf16, b_dec, b_pre, idx, val, grad_out, coef,
+                                      B, d, F, k, resid, resid_bf16, stats, last_activated, step_count, d_b_enc,
+                                      d_b_dec, dpre_val, stream);
+  });
 }
 
 extern "C" int wsae_decode_backward(const float* target, const void* w_decT, int w_is_bf16,
@@ -1611,7 +1658,7 @@ extern "C" int wsae_decode_backward(const float* target, const void* w_decT, int
                                     const long long* step_count, float* d_b_enc, float* d_b_dec,
                                     float* dpre_val, cudaStream_t stream) {
   if (!target) return kBadArg;
-  return decode_backward_impl(target, nullptr, nullptr, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val, grad_out,
+  return decode_backward_impl(target, nullptr, 0, nullptr, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val, grad_out,
                               coef, B, d, F, k, resid, resid_bf16, stats, last_activated, step_count,
                               d_b_enc, d_b_dec, dpre_val, stream);
 }
@@ -1626,7 +1673,7 @@ extern "C" int wsae_decode_backward_at(const float* const* target_at, const void
                                        const long long* step_count, float* d_b_enc, float* d_b_dec,
                                        float* dpre_val, cudaStream_t stream) {
   if (!target_at) return kBadArg;
-  return decode_backward_impl(nullptr, target_at, nullptr, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val,
+  return decode_backward_impl(nullptr, reinterpret_cast<const void* const*>(target_at), 0, nullptr, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val,
                               grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated,
                               step_count, d_b_enc, d_b_dec, dpre_val, stream);
 }
@@ -1643,7 +1690,7 @@ extern "C" int wsae_decode_backward_rows_at(const float* const* target_at,
                                             float* d_b_enc, float* d_b_dec, float* dpre_val,
                                             cudaStream_t stream) {
   if (!target_at || !rows_at) return kBadArg;
-  return decode_backward_impl(nullptr, target_at, rows_at, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val,
+  return decode_backward_impl(nullptr, reinterpret_cast<const void* const*>(target_at), 0, rows_at, nullptr, w_decT, w_is_bf16, b_dec, b_pre, idx, val,
                               grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated,
                               step_count, d_b_enc, d_b_dec, dpre_val, stream);
 }
@@ -1661,7 +1708,22 @@ extern "C" int wsae_decode_backward_det(const float* target, const float* const*
                                         const long long* step_count, float* d_b_enc, float* d_b_dec,
                                         float* dpre_val, long long* det_ws, cudaStream_t stream) {
   if ((!target && !target_at) || !det_ws) return kBadArg;
-  return decode_backward_impl(target, target_at, rows_at, det_ws, w_decT, w_is_bf16, b_dec, b_pre, idx,
+  return decode_backward_impl(target, reinterpret_cast<const void* const*>(target_at), 0, rows_at, det_ws, w_decT, w_is_bf16, b_dec, b_pre, idx,
+                              val, grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated,
+                              step_count, d_b_enc, d_b_dec, dpre_val, stream);
+}
+
+// Slot form for any target element type (x_dtype 0 = fp32, 1 = bf16, 2 = fp16; *target_at then points
+// at that type): rows_at nullable, det_ws nullable (non-NULL: the deterministic form above).
+extern "C" int wsae_decode_backward_typed(const void* const* target_at, const long long* const* rows_at,
+                                          int x_dtype, const void* w_decT, int w_is_bf16, const float* b_dec,
+                                          const float* b_pre, const int32_t* idx, const float* val,
+                                          const float* grad_out, float coef, int B, int d, int F, int k,
+                                          float* resid, void* resid_bf16, void* stats, long long* last_activated,
+                                          const long long* step_count, float* d_b_enc, float* d_b_dec,
+                                          float* dpre_val, long long* det_ws, cudaStream_t stream) {
+  if (!target_at) return kBadArg;
+  return decode_backward_impl(nullptr, target_at, x_dtype, rows_at, det_ws, w_decT, w_is_bf16, b_dec, b_pre, idx,
                               val, grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated,
                               step_count, d_b_enc, d_b_dec, dpre_val, stream);
 }

@@ -30,11 +30,16 @@ __device__ __forceinline__ float ln_load<__nv_bfloat16>(const __nv_bfloat16* p, 
 template <>
 __device__ __forceinline__ float ln_load<__half>(const __half* p, size_t i) { return __half2float(p[i]); }
 
-template <typename TIn, int PER>
+// fp32 result -> output element, rounded to nearest
+__device__ __forceinline__ void ln_store(float* p, float v) { *p = v; }
+__device__ __forceinline__ void ln_store(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
+__device__ __forceinline__ void ln_store(__half* p, float v) { *p = __float2half_rn(v); }
+
+template <typename TIn, typename TOut, int PER>
 __global__ void __launch_bounds__(256)
 layernorm_rows_kernel(const TIn* __restrict__ x, long long rows, int d, long long in_pitch,
                       const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
-                      float* __restrict__ out, long long out_pitch) {
+                      TOut* __restrict__ out, long long out_pitch) {
   const int lane = threadIdx.x & 31;
   const long long row = static_cast<long long>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= rows) return;
@@ -56,28 +61,29 @@ layernorm_rows_kernel(const TIn* __restrict__ x, long long rows, int d, long lon
     sq = fmaf(t, t, sq);
   }
   const float rstd = rsqrtf(warp_sum(sq) / static_cast<float>(d) + eps);
-  float* orow = out + row * out_pitch;
+  TOut* orow = out + row * out_pitch;
 #pragma unroll
   for (int j = 0; j < PER; ++j) {
     const int c = j * 32 + lane;
     if (c < d) {
       const float g = gamma != nullptr ? gamma[c] : 1.f;
       const float b = beta != nullptr ? beta[c] : 0.f;
-      orow[c] = (v[j] - mean) * rstd * g + b;
+      ln_store(orow + c, (v[j] - mean) * rstd * g + b);
     }
   }
 }
 
-template <typename TIn>
+template <typename TIn, typename TOut>
 static int launch_layernorm(const void* x, long long rows, int d, long long in_pitch, const float* gamma,
-                            const float* beta, float eps, float* out, long long out_pitch,
+                            const float* beta, float eps, void* out_v, long long out_pitch,
                             cudaStream_t stream) {
+  TOut* out = static_cast<TOut*>(out_v);
   const int warps = 8;
   const unsigned blocks = static_cast<unsigned>((rows + warps - 1) / warps);
   const TIn* xi = static_cast<const TIn*>(x);
   const int per = ceil_div(d, 32);
 #define WSAE_LN_CASE(P)                                                                        \
-  layernorm_rows_kernel<TIn, P><<<blocks, warps * 32, 0, stream>>>(xi, rows, d, in_pitch, gamma, \
+  layernorm_rows_kernel<TIn, TOut, P><<<blocks, warps * 32, 0, stream>>>(xi, rows, d, in_pitch, gamma, \
                                                                    beta, eps, out, out_pitch)
   if (per <= 4) WSAE_LN_CASE(4);
   else if (per <= 12) WSAE_LN_CASE(12);
@@ -95,20 +101,30 @@ static int launch_layernorm(const void* x, long long rows, int d, long long in_p
 
 using namespace wsae;
 
-// See include/wsae.h.  in_dtype: 0 = float32, 1 = bfloat16, 2 = float16.
+// See include/wsae.h.  in_dtype / out_dtype: 0 = float32, 1 = bfloat16, 2 = float16.
+extern "C" int wsae_layernorm_rows_typed(const void* x, int in_dtype, long long rows, int d,
+                                         long long in_pitch_elems, const float* gamma, const float* beta,
+                                         float eps, void* out, int out_dtype, long long out_pitch_elems,
+                                         cudaStream_t stream) {
+  if (!x || !out || rows < 0 || d <= 0) return kBadArg;
+  if (in_pitch_elems < d || out_pitch_elems < d) return kBadArg;
+  if (d > 32 * kLnMaxPerLane) return kUnsupported;
+  if (out_dtype < 0 || out_dtype > 2) return kBadArg;
+  if (rows == 0) return kOk;
+  if (rows > 0x7fffffffLL * 8) return kUnsupported;
+  return with_x_dtype(in_dtype, [&](auto in_tag) {
+    using TIn = std::remove_cv_t<std::remove_pointer_t<decltype(in_tag)>>;
+    return with_x_dtype(out_dtype, [&](auto out_tag) {
+      using TOut = std::remove_cv_t<std::remove_pointer_t<decltype(out_tag)>>;
+      return launch_layernorm<TIn, TOut>(x, rows, d, in_pitch_elems, gamma, beta, eps, out, out_pitch_elems, stream);
+    });
+  });
+}
+
 extern "C" int wsae_layernorm_rows(const void* x, int in_dtype, long long rows, int d,
                                    long long in_pitch_elems, const float* gamma, const float* beta,
                                    float eps, float* out, long long out_pitch_elems,
                                    cudaStream_t stream) {
-  if (!x || !out || rows < 0 || d <= 0) return kBadArg;
-  if (in_pitch_elems < d || out_pitch_elems < d) return kBadArg;
-  if (d > 32 * kLnMaxPerLane) return kUnsupported;
-  if (rows == 0) return kOk;
-  if (rows > 0x7fffffffLL * 8) return kUnsupported;
-  switch (in_dtype) {
-    case 0: return launch_layernorm<float>(x, rows, d, in_pitch_elems, gamma, beta, eps, out, out_pitch_elems, stream);
-    case 1: return launch_layernorm<__nv_bfloat16>(x, rows, d, in_pitch_elems, gamma, beta, eps, out, out_pitch_elems, stream);
-    case 2: return launch_layernorm<__half>(x, rows, d, in_pitch_elems, gamma, beta, eps, out, out_pitch_elems, stream);
-    default: return kBadArg;
-  }
+  return wsae_layernorm_rows_typed(x, in_dtype, rows, d, in_pitch_elems, gamma, beta, eps, out, 0, out_pitch_elems,
+                                   stream);
 }

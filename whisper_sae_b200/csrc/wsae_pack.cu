@@ -84,11 +84,25 @@ pack_rows_kernel(const float* __restrict__ src, const float* __restrict__ center
       *reinterpret_cast<const uint4*>(out);
 }
 
+// 8 consecutive activations (16-byte aligned), streamed: fp32 is two 16-byte loads, a half type one
+__device__ __forceinline__ void ldcs_x8(const float* p, float4& a, float4& b) {
+  const float4* src = reinterpret_cast<const float4*>(p);
+  a = __ldcs(src);
+  b = __ldcs(src + 1);
+}
+template <typename TX>
+__device__ __forceinline__ void ldcs_x8(const TX* p, float4& a, float4& b) {
+  const uint4 u = __ldcs(reinterpret_cast<const uint4*>(p));
+  a = x4_to_float4<TX>(make_uint2(u.x, u.y));
+  b = x4_to_float4<TX>(make_uint2(u.z, u.w));
+}
+
 // bf16 fast path for activations (T = 1, d % 8 == 0): one thread converts 8 consecutive columns with
-// two 16-byte loads and one 16-byte store; the bias block and the K padding are written by the same
-// grid.  HBM bound: reads B*d*4, writes Bp*Kp*2 bytes.
+// two 16-byte loads (fp32 input; one for bf16 / fp16 input) and one 16-byte store; the bias block and
+// the K padding are written by the same grid.  HBM bound: reads B*d*sizeof(TX), writes Bp*Kp*2 bytes.
+template <typename TX>
 __global__ void __launch_bounds__(256)
-pack_activations_bf16_kernel(const float* __restrict__ x, const float* const* __restrict__ x_at,
+pack_activations_bf16_kernel(const TX* __restrict__ x, const TX* const* __restrict__ x_at,
                              const long long* const* __restrict__ rows_at,
                              const float* __restrict__ center, int rows, int rows_p, int d, int Kp,
                              __nv_bfloat16* __restrict__ dst) {
@@ -108,8 +122,8 @@ pack_activations_bf16_kernel(const float* __restrict__ x, const float* const* __
   if (r < rows) {
     if (c0 < d) {
       const size_t sr = perm != nullptr ? static_cast<size_t>(__ldg(perm + r)) : static_cast<size_t>(r);
-      const float4* src = reinterpret_cast<const float4*>(x + sr * d + c0);
-      float4 a = __ldcs(src), b = __ldcs(src + 1);        // streamed once: do not keep in L2/L1
+      float4 a, b;
+      ldcs_x8(x + sr * d + c0, a, b);                     // streamed once: do not keep in L2/L1
       if (center != nullptr) {
         const float4 ca = __ldg(reinterpret_cast<const float4*>(center + c0));
         const float4 cb = __ldg(reinterpret_cast<const float4*>(center + c0 + 4));
@@ -157,10 +171,14 @@ extern "C" int wsae_packed_k(int d, int terms, int* dp_out, int* used_cols_out, 
   return kOk;
 }
 
+// x_dtype: element type of the activations (0 = fp32, 1 = bf16, 2 = fp16); half types are read by the
+// single-term fast path only (src / src_at then point at that type).
 static int pack_common(int kind, const float* src, const float* center, const float* bias,
                        int rows, int rows_p, int d, int terms, void* dst, cudaStream_t stream,
-                       const float* const* src_at = nullptr, const long long* const* rows_at = nullptr) {
+                       const void* const* src_at = nullptr, const long long* const* rows_at = nullptr,
+                       int x_dtype = 0) {
   if ((!src && !src_at) || !dst || rows <= 0 || rows_p < rows) return kBadArg;
+  if (x_dtype < 0 || x_dtype > 2) return kBadArg;
   int dp, used, Kp;
   if (wsae_packed_k(d, terms, &dp, &used, &Kp)) return kBadArg;
   PieceSchedule s;
@@ -171,11 +189,17 @@ static int pack_common(int kind, const float* src, const float* center, const fl
   const bool fast = kind == 0 && terms == 1 && d % 8 == 0 &&
                     (reinterpret_cast<uintptr_t>(src) & 15u) == 0 &&
                     (center == nullptr || (reinterpret_cast<uintptr_t>(center) & 15u) == 0);
-  if (src_at != nullptr && !fast) return kUnsupported;   // the slot form exists for the bf16 path only
+  // the slot form and half-precision input exist for the bf16 path only
+  if ((src_at != nullptr || x_dtype != 0) && !fast) return kUnsupported;
   if (fast)
-    launch_pdl(pack_activations_bf16_kernel, blocks, threads, 0, stream, src, src_at, rows_at, center,
-               rows, rows_p, d, Kp, static_cast<__nv_bfloat16*>(dst));
-  else if (kind == 0)
+    return with_x_dtype(x_dtype, [&](auto tag) {
+      using TX = std::remove_cv_t<std::remove_pointer_t<decltype(tag)>>;
+      launch_pdl(pack_activations_bf16_kernel<TX>, blocks, threads, 0, stream,
+                 reinterpret_cast<const TX*>(src), reinterpret_cast<const TX* const*>(src_at), rows_at,
+                 center, rows, rows_p, d, Kp, static_cast<__nv_bfloat16*>(dst));
+      return static_cast<int>(cudaGetLastError());
+    });
+  if (kind == 0)
     launch_pdl(pack_rows_kernel<0>, blocks, threads, 0, stream, src, center, bias, rows, rows_p, d,
                dp, terms, Kp, s, static_cast<__nv_bfloat16*>(dst));
   else
@@ -194,7 +218,8 @@ extern "C" int wsae_pack_activations(const float* x, const float* b_pre, int B, 
 extern "C" int wsae_pack_activations_at(const float* const* x_at, const float* b_pre, int B, int Bp,
                                         int d, int terms, void* a_packed, cudaStream_t stream) {
   if (!x_at) return kBadArg;
-  return pack_common(0, nullptr, b_pre, nullptr, B, Bp, d, terms, a_packed, stream, x_at);
+  return pack_common(0, nullptr, b_pre, nullptr, B, Bp, d, terms, a_packed, stream,
+                     reinterpret_cast<const void* const*>(x_at));
 }
 
 // Slot form with a row-index indirection: batch row r = (*x_at)[(*rows_at)[r], :]; *rows_at == 0 means
@@ -203,7 +228,16 @@ extern "C" int wsae_pack_activations_rows_at(const float* const* x_at, const lon
                                              const float* b_pre, int B, int Bp, int d, int terms,
                                              void* a_packed, cudaStream_t stream) {
   if (!x_at || !rows_at) return kBadArg;
-  return pack_common(0, nullptr, b_pre, nullptr, B, Bp, d, terms, a_packed, stream, x_at, rows_at);
+  return pack_common(0, nullptr, b_pre, nullptr, B, Bp, d, terms, a_packed, stream,
+                     reinterpret_cast<const void* const*>(x_at), rows_at);
+}
+
+// Slot form for any activation element type (x_dtype 0 = fp32, 1 = bf16, 2 = fp16); rows_at nullable.
+extern "C" int wsae_pack_activations_typed(const void* const* x_at, const long long* const* rows_at, int x_dtype,
+                                           const float* b_pre, int B, int Bp, int d, int terms, void* a_packed,
+                                           cudaStream_t stream) {
+  if (!x_at) return kBadArg;
+  return pack_common(0, nullptr, b_pre, nullptr, B, Bp, d, terms, a_packed, stream, x_at, rows_at, x_dtype);
 }
 
 extern "C" int wsae_pack_encoder(const float* w_enc, const float* b_enc, int F, int Fp, int d,

@@ -33,9 +33,11 @@ __device__ __forceinline__ void red_add_v2(float* addr, float a, float b) {
 
 __device__ __forceinline__ float bf16_round(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 
+// TX: element type of the activation matrix (float / __nv_bfloat16 / __half, converted at the load).
+template <typename TX>
 __global__ void __launch_bounds__(kRowTopkThreads)
-row_step_kernel(const float* __restrict__ pre, const float* __restrict__ target,
-                const float* const* __restrict__ target_at, const long long* const* __restrict__ rows_at,
+row_step_kernel(const float* __restrict__ pre, const TX* __restrict__ target,
+                const TX* const* __restrict__ target_at, const long long* const* __restrict__ rows_at,
                 const __nv_bfloat16* __restrict__ w_decT, const float* __restrict__ b_dec,
                 const float* __restrict__ b_pre, const float* __restrict__ grad_out, float coef, int B, int d,
                 int F, int k, float* __restrict__ out_val, int32_t* __restrict__ out_idx,
@@ -82,7 +84,7 @@ row_step_kernel(const float* __restrict__ pre, const float* __restrict__ target,
   if (target_at != nullptr) target = *target_at;
   const long long* perm = rows_at != nullptr ? *rows_at : nullptr;
   const size_t srow = perm != nullptr ? static_cast<size_t>(perm[row]) : static_cast<size_t>(row);
-  const float* trow = target + srow * d;
+  const TX* trow = target + srow * d;
   const float s = coef * (grad_out != nullptr ? *grad_out : 1.f);
   const long long stamp = (last_activated != nullptr && step_count != nullptr) ? (*step_count + 1) : 0;
   const uint32_t* wrows = reinterpret_cast<const uint32_t*>(w_decT);     // bf16 pairs
@@ -112,7 +114,7 @@ row_step_kernel(const float* __restrict__ pre, const float* __restrict__ target,
       a0 = fmaf(h, __uint_as_float(w[j] << 16), a0);
       a1 = fmaf(h, __uint_as_float(w[j] & 0xffff0000u), a1);
     }
-    const float2 t = *reinterpret_cast<const float2*>(trow + c);
+    const float2 t = ld_x2(trow + c);
     const float r0 = a0 - t.x, r1 = a1 - t.y;
     s_res[c] = r0;
     s_res[c + 1] = r1;
@@ -254,6 +256,44 @@ row_step_kernel(const float* __restrict__ pre, const float* __restrict__ target,
 using namespace wsae;
 
 // See include/wsae.h.  stats = { double sse; uint64 l0_count } (caller-zeroed, as for wsae_decode_mse).
+// x_dtype (0 = fp32, 1 = bf16, 2 = fp16): element type of target / *target_at.
+extern "C" int wsae_row_step_typed(const float* pre, const void* target, const void* const* target_at,
+                                   const long long* const* rows_at, int x_dtype, const void* w_decT_bf16,
+                                   const float* b_dec, const float* b_pre, const float* grad_out, float coef, int B,
+                                   int d, int F, int k, float* out_val, int32_t* out_idx, void* stats,
+                                   long long* last_activated, long long* step_count, float* d_b_enc, float* d_b_dec,
+                                   float* d_w_enc, float* d_w_decT, float* resid, float* dpre_val, const float* w_enc,
+                                   float* d_b_pre, unsigned int* ticket, long long dead_threshold,
+                                   long long* dead_count, const long long* seq, long long* mailbox,
+                                   cudaStream_t stream) {
+  if (!pre || (!target && !target_at) || !w_decT_bf16 || !b_dec || !out_val || !out_idx) return kBadArg;
+  if (B <= 0 || d <= 0 || F <= 0 || k <= 0 || k > F) return kBadArg;
+  if (k > kRowStepMaxK || d % 2 != 0) return kUnsupported;
+  if (ticket != nullptr && (!step_count || !last_activated || (mailbox != nullptr && !seq))) return kBadArg;
+  const size_t smem = (static_cast<size_t>(F) + 2 * static_cast<size_t>(d)) * 4;
+  if (smem > 200 * 1024) return kUnsupported;
+  return with_x_dtype(x_dtype, [&](auto tag) {
+    using TX = std::remove_cv_t<std::remove_pointer_t<decltype(tag)>>;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    static bool attr_set[64] = {};
+    if (dev >= 64 || !attr_set[dev]) {
+      cudaError_t e = cudaFuncSetAttribute(row_step_kernel<TX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+      if (e != cudaSuccess) return static_cast<int>(e);
+      if (dev < 64) attr_set[dev] = true;
+    }
+    double* sse = stats ? static_cast<double*>(stats) : nullptr;
+    unsigned long long* l0 = stats ? reinterpret_cast<unsigned long long*>(static_cast<char*>(stats) + 8) : nullptr;
+    cudaError_t e = launch_pdl(row_step_kernel<TX>, B, kRowTopkThreads, smem, stream, pre,
+                               static_cast<const TX*>(target), reinterpret_cast<const TX* const*>(target_at), rows_at,
+                               static_cast<const __nv_bfloat16*>(w_decT_bf16), b_dec, b_pre, grad_out, coef, B, d, F,
+                               k, out_val, out_idx, sse, l0, last_activated, step_count, d_b_enc, d_b_dec, d_w_enc,
+                               d_w_decT, resid, dpre_val, w_enc, d_b_pre, ticket, dead_threshold, dead_count, seq,
+                               mailbox);
+    return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
+  });
+}
+
 extern "C" int wsae_row_step(const float* pre, const float* target, const float* const* target_at,
                              const long long* const* rows_at, const void* w_decT_bf16, const float* b_dec,
                              const float* b_pre, const float* grad_out, float coef, int B, int d, int F, int k,
@@ -262,25 +302,8 @@ extern "C" int wsae_row_step(const float* pre, const float* target, const float*
                              float* d_w_decT, float* resid, float* dpre_val, const float* w_enc, float* d_b_pre,
                              unsigned int* ticket, long long dead_threshold, long long* dead_count,
                              const long long* seq, long long* mailbox, cudaStream_t stream) {
-  if (!pre || (!target && !target_at) || !w_decT_bf16 || !b_dec || !out_val || !out_idx) return kBadArg;
-  if (B <= 0 || d <= 0 || F <= 0 || k <= 0 || k > F) return kBadArg;
-  if (k > kRowStepMaxK || d % 2 != 0) return kUnsupported;
-  if (ticket != nullptr && (!step_count || !last_activated || (mailbox != nullptr && !seq))) return kBadArg;
-  const size_t smem = (static_cast<size_t>(F) + 2 * static_cast<size_t>(d)) * 4;
-  if (smem > 200 * 1024) return kUnsupported;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static bool attr_set[64] = {};
-  if (dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(row_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    if (dev < 64) attr_set[dev] = true;
-  }
-  double* sse = stats ? static_cast<double*>(stats) : nullptr;
-  unsigned long long* l0 = stats ? reinterpret_cast<unsigned long long*>(static_cast<char*>(stats) + 8) : nullptr;
-  cudaError_t e = launch_pdl(row_step_kernel, B, kRowTopkThreads, smem, stream, pre, target, target_at, rows_at,
-                             static_cast<const __nv_bfloat16*>(w_decT_bf16), b_dec, b_pre, grad_out, coef, B, d, F,
-                             k, out_val, out_idx, sse, l0, last_activated, step_count, d_b_enc, d_b_dec, d_w_enc,
-                             d_w_decT, resid, dpre_val, w_enc, d_b_pre, ticket, dead_threshold, dead_count, seq, mailbox);
-  return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
+  return wsae_row_step_typed(pre, target, reinterpret_cast<const void* const*>(target_at), rows_at, 0, w_decT_bf16,
+                             b_dec, b_pre, grad_out, coef, B, d, F, k, out_val, out_idx, stats, last_activated,
+                             step_count, d_b_enc, d_b_dec, d_w_enc, d_w_decT, resid, dpre_val, w_enc, d_b_pre, ticket,
+                             dead_threshold, dead_count, seq, mailbox, stream);
 }

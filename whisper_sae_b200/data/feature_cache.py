@@ -3,6 +3,7 @@
 
 Files (byte-compatible with the reference, so caches are interchangeable):
   ``{model_short}_{component}_layer{N}.pt``        one float32 tensor [num_tokens, d_model]
+                                                   (bfloat16 / float16 when extracted with ``dtype=``)
   ``{model_short}_{component}_layer{N}_meta.json`` the 8 ``CacheMetadata`` fields
 
 ``get_dataloader`` keeps the reference signature and default behaviour (a ``DataLoader`` over a
@@ -164,6 +165,8 @@ class FeatureCache:
                 and self._get_metadata_path(component, layer_idx).exists())
 
     def load(self, component: Component, layer_idx: int) -> tuple[Tensor, CacheMetadata]:
+        """The cached matrix in its stored dtype (a bf16 / fp16 cache stays half precision: the graphed
+        train step reads it in place) and its metadata."""
         features = torch.load(self._get_cache_path(component, layer_idx), weights_only=True)
         meta = CacheMetadata.from_json(self._get_metadata_path(component, layer_idx).read_text())
         return features, meta
@@ -185,6 +188,7 @@ class FeatureCache:
     def get_dataloader(self, component: Component, layer_idx: int, batch_size: int,
                        shuffle: bool = True, num_workers: int = 0, *,
                        device: torch.device | str | None = None):
+        """Batches of the cached matrix in its stored dtype; a bf16 / fp16 cache trains in place."""
         features, _ = self.load(component, layer_idx)
         if device is not None:
             return ResidentBatches(features, batch_size, shuffle, device)
@@ -196,7 +200,8 @@ def extract_and_cache_features(whisper_model, processor, audio_dataloader, cache
                                encoder_layers: list[int], decoder_layers: list[int],
                                device: torch.device | str = "cuda",
                                max_samples: int | None = None, *,
-                               device_budget_bytes: int = 8 << 30) -> None:
+                               device_budget_bytes: int = 8 << 30,
+                               dtype: torch.dtype = torch.float32) -> None:
     """Run Whisper over ``audio_dataloader`` and write one cache file per hooked layer
     (feature_cache.py:200-306; same signature, ``processor`` is unused there too).
 
@@ -205,16 +210,24 @@ def extract_and_cache_features(whisper_model, processor, audio_dataloader, cache
     ``cache.save`` writes the ``[N, d]`` fp32 tensor in the reference's file format - unless the
     hooked layers together would hold more than ``device_budget_bytes`` on the GPU, in which case full
     chunks are spilled to pinned host memory as they fill (the reference accumulates on the host).
+
+    ``dtype`` (extension): ``torch.bfloat16`` or ``torch.float16`` writes half-precision cache files,
+    the fp32 LayerNorm result rounded to nearest - half the bytes on disk, in host memory, on PCIe and
+    in HBM.  The file format and the metadata are otherwise unchanged; ``SAETrainer`` trains on such a
+    matrix in place, while the reference's trainer needs ``.float()`` to read it.
     """
+    if dtype not in (torch.float32, torch.bfloat16, torch.float16):
+        raise ValueError(f"cache dtype must be float32, bfloat16 or float16, not {dtype}")
     from ..sae.hooks import ActivationMatrix, _hidden_of, run_whisper
 
     whisper_model = whisper_model.to(device)
     whisper_model.eval()
     d = whisper_model.config.d_model
     n_sinks = max(1, len(encoder_layers) + len(decoder_layers))
-    cap_rows = max(4096, device_budget_bytes // (n_sinks * d * 4))
-    enc = {layer: ActivationMatrix(d, device, max_device_rows=cap_rows) for layer in encoder_layers}
-    dec = {layer: ActivationMatrix(d, device, max_device_rows=cap_rows) for layer in decoder_layers}
+    elem = torch.empty((), dtype=dtype).element_size()
+    cap_rows = max(4096, device_budget_bytes // (n_sinks * d * elem))
+    enc = {layer: ActivationMatrix(d, device, max_device_rows=cap_rows, dtype=dtype) for layer in encoder_layers}
+    dec = {layer: ActivationMatrix(d, device, max_device_rows=cap_rows, dtype=dtype) for layer in decoder_layers}
     enc_ln, dec_ln = whisper_model.model.encoder.layer_norm, whisper_model.model.decoder.layer_norm
     handles = []
     for layer, sink in enc.items():

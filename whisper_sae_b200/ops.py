@@ -50,6 +50,21 @@ def _f32c(t: Tensor | None, name: str) -> None:
         raise RuntimeError(f"{name} must be a contiguous float32 tensor")
 
 
+# activation element types the kernels read, by the C ABI's dtype code (include/wsae.h)
+_LN_DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
+
+
+def _x_dtype_code(dtype: torch.dtype) -> int:
+    if dtype not in _LN_DTYPES:
+        raise RuntimeError(f"unsupported activation dtype {dtype} (float32, bfloat16 or float16)")
+    return _LN_DTYPES[dtype]
+
+
+def _check_slot(slot: Tensor, name: str) -> None:
+    if slot.dtype != torch.int64 or slot.numel() != 1 or not slot.is_cuda:
+        raise RuntimeError(f"{name} must be a one-element int64 CUDA tensor holding a device address")
+
+
 def _count(n: int = 1) -> None:
     global GPU_LAUNCHES
     GPU_LAUNCHES += n
@@ -123,31 +138,25 @@ def pack_activations(x: Tensor, b_pre: Tensor | None, terms: int, out: Tensor | 
 
 
 def pack_activations_at(x_at: Tensor, B: int, d: int, b_pre: Tensor | None,
-                        out: Tensor | None = None, rows_at: Tensor | None = None) -> Tensor:
-    """``pack_activations`` (bf16, one term) of the ``[B, d]`` fp32 matrix whose device address the
-    int64 slot ``x_at`` holds WHEN THE KERNEL RUNS (graph replay on batches in place).  ``rows_at``:
-    a second int64 slot holding the address of an int64 row-index array (0 = identity): batch row r is
-    row ``rows[r]`` of the matrix (shuffled batches of a resident matrix, never materialised)."""
+                        out: Tensor | None = None, rows_at: Tensor | None = None,
+                        x_dtype: torch.dtype = torch.float32) -> Tensor:
+    """``pack_activations`` (bf16, one term) of the ``[B, d]`` matrix whose device address the int64
+    slot ``x_at`` holds WHEN THE KERNEL RUNS (graph replay on batches in place).  ``x_dtype``: its
+    element type (float32, bfloat16 or float16; a slot holds only an address).  ``rows_at``: a second
+    int64 slot holding the address of an int64 row-index array (0 = identity): batch row r is row
+    ``rows[r]`` of the matrix (shuffled batches of a resident matrix, never materialised)."""
     _need_cuda(x_at, b_pre, rows_at)
     _f32c(b_pre, "b_pre")
-    if x_at.dtype != torch.int64 or x_at.numel() != 1:
-        raise RuntimeError("x_at must be a one-element int64 CUDA tensor holding a device address")
+    _check_slot(x_at, "x_at")
     if rows_at is not None:
-        if rows_at.dtype != torch.int64 or rows_at.numel() != 1:
-            raise RuntimeError("rows_at must be a one-element int64 CUDA tensor holding a device address")
-        ps = packed_shape(d, 1)
-        Bp = _round_up(B, 128)
-        if out is None or out.shape != (Bp, ps.kp):
-            out = torch.empty((Bp, ps.kp), dtype=torch.bfloat16, device=x_at.device)
-        lib = _lib.load()
-        _run("wsae_pack_activations", lib.wsae_pack_activations_rows_at, _ptr(x_at), _ptr(rows_at), _ptr(b_pre), B, Bp, d, 1, _ptr(out), _stream())
-        return out
+        _check_slot(rows_at, "rows_at")
     ps = packed_shape(d, 1)
     Bp = _round_up(B, 128)
     if out is None or out.shape != (Bp, ps.kp):
         out = torch.empty((Bp, ps.kp), dtype=torch.bfloat16, device=x_at.device)
     lib = _lib.load()
-    _run("wsae_pack_activations", lib.wsae_pack_activations_at, _ptr(x_at), _ptr(b_pre), B, Bp, d, 1, _ptr(out), _stream())
+    _run("wsae_pack_activations", lib.wsae_pack_activations_typed, _ptr(x_at), _ptr(rows_at), _x_dtype_code(x_dtype),
+         _ptr(b_pre), B, Bp, d, 1, _ptr(out), _stream())
     return out
 
 
@@ -353,9 +362,11 @@ def row_step(pre: Tensor, target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: 
              resid: Tensor | None = None, dpre_val: Tensor | None = None, target_is_slot: bool = False,
              rows_at: Tensor | None = None, w_enc: Tensor | None = None,
              d_b_pre: Tensor | None = None,
-             finish: tuple[Tensor, int, Tensor | None, Tensor, Tensor] | None = None) -> tuple[Tensor, Tensor]:
+             finish: tuple[Tensor, int, Tensor | None, Tensor, Tensor] | None = None,
+             x_dtype: torch.dtype = torch.float32) -> tuple[Tensor, Tensor]:
     """Small-batch step, one block per row: TopK of ``pre`` + sparse decode + MSE + stamps + dv + bias
-    gradients + both weight-gradient rows (fp32 atomics).  Returns (idx int32 [B,k], val fp32 [B,k])."""
+    gradients + both weight-gradient rows (fp32 atomics).  Returns (idx int32 [B,k], val fp32 [B,k]).
+    The target is float32, bfloat16 or float16: its own dtype, or ``x_dtype`` when it is a slot."""
     _need_cuda(pre, target, w_decT, b_dec, b_pre, grad_out)
     _f32c(pre, "pre")
     B, F = pre.shape
@@ -363,12 +374,12 @@ def row_step(pre: Tensor, target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: 
     if w_decT.dtype != torch.bfloat16 or not w_decT.is_contiguous() or w_decT.shape[0] != F:
         raise RuntimeError("w_decT must be contiguous [F, d] bfloat16")
     if target_is_slot:
-        if target.dtype != torch.int64 or target.numel() != 1:
-            raise RuntimeError("target slot must be a one-element int64 CUDA tensor")
+        _check_slot(target, "target slot")
         tgt, tgt_at = None, target
     else:
-        _f32c(target, "target")
-        tgt, tgt_at = target, None
+        if not target.is_contiguous():
+            raise RuntimeError("target must be contiguous")
+        tgt, tgt_at, x_dtype = target, None, target.dtype
     idx = torch.empty((B, k), dtype=torch.int32, device=pre.device)
     val = torch.empty((B, k), dtype=torch.float32, device=pre.device)
     lib = _lib.load()
@@ -378,7 +389,7 @@ def row_step(pre: Tensor, target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: 
     if finish is not None:
         ticket, thr, dead, seq, mailbox = finish
         fin = (_ptr(ticket), int(thr), _ptr(dead), _ptr(seq), _ptr(mailbox))
-    _run("wsae_row_step", lib.wsae_row_step, _ptr(pre), _ptr(tgt), _ptr(tgt_at), _ptr(rows_at), _ptr(w_decT),
+    _run("wsae_row_step", lib.wsae_row_step_typed, _ptr(pre), _ptr(tgt), _ptr(tgt_at), _ptr(rows_at), _x_dtype_code(x_dtype), _ptr(w_decT),
          _ptr(b_dec), _ptr(b_pre), _ptr(grad_out), float(coef), B, d, F, k, _ptr(val), _ptr(idx), _ptr(stats),
          _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(d_w_enc), _ptr(d_w_decT),
          _ptr(resid), _ptr(dpre_val), _ptr(w_enc), _ptr(d_b_pre), *fin, _stream())
@@ -408,45 +419,38 @@ def decode_backward(target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: Tensor
                     last_activated: Tensor | None, step_count: Tensor | None,
                     d_b_enc: Tensor | None, d_b_dec: Tensor | None, dpre_val: Tensor | None,
                     target_is_slot: bool = False, rows_at: Tensor | None = None,
-                    det_ws: Tensor | None = None) -> None:
+                    det_ws: Tensor | None = None, x_dtype: torch.dtype = torch.float32) -> None:
     """K23: sparse decode + MSE + L0 + fired stamps + dv / bias gradients in one pass.
     ``target_is_slot``: ``target`` is a one-element int64 tensor holding the device address of the
-    ``[B, d]`` fp32 target, read when the kernel runs (see ``pack_activations_at``)."""
+    ``[B, d]`` target, read when the kernel runs (see ``pack_activations_at``); ``x_dtype`` is that
+    matrix's element type (float32, bfloat16 or float16)."""
     _need_cuda(target, w_decT, b_dec, b_pre, idx, val, grad_out)
     F, d = w_decT.shape
+    B, k = idx.shape
     if det_ws is not None:
         # deterministic accumulation: fixed-point int64 sums in det_ws [F + d + 1] (zeroed by the caller),
         # converted by det_finish; the float atomics on d_b_enc / d_b_dec / stats.sse are not issued
         if det_ws.dtype != torch.int64 or det_ws.numel() < F + d + 1 or not det_ws.is_cuda:
             raise RuntimeError("det_ws must be an int64 CUDA tensor of >= F + d + 1 elements")
-        if w_decT.dtype != torch.bfloat16 or not w_decT.is_contiguous():
-            raise RuntimeError("w_decT must be contiguous [F, d] bfloat16")
-        B, k = idx.shape
-        lib = _lib.load()
-        tgt, tgt_at = (None, target) if target_is_slot else (target, None)
-        _run("wsae_decode_backward", lib.wsae_decode_backward_det, _ptr(tgt), _ptr(tgt_at), _ptr(rows_at), _ptr(w_decT), 1, _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _ptr(det_ws), _stream())
-        _run("wsae_det_finish", lib.wsae_det_finish, _ptr(det_ws), F, d, _ptr(grad_out), float(coef), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(stats), _stream())
-        return
+    lib = _lib.load()
     if target_is_slot:
-        if target.dtype != torch.int64 or target.numel() != 1:
-            raise RuntimeError("target slot must be a one-element int64 CUDA tensor")
-        B, k = idx.shape
+        _check_slot(target, "target slot")
+        if rows_at is not None:
+            _check_slot(rows_at, "rows_at")
         if not w_decT.is_contiguous() or w_decT.dtype != torch.bfloat16:
             raise RuntimeError("w_decT must be contiguous [F, d] bfloat16")
-        lib = _lib.load()
-        if rows_at is not None:
-            if rows_at.dtype != torch.int64 or rows_at.numel() != 1 or not rows_at.is_cuda:
-                raise RuntimeError("rows_at must be a one-element int64 CUDA tensor holding a device address")
-            _run("wsae_decode_backward", lib.wsae_decode_backward_rows_at, _ptr(target), _ptr(rows_at), _ptr(w_decT), 1, _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _stream())
-            return
-        _run("wsae_decode_backward", lib.wsae_decode_backward_at, _ptr(target), _ptr(w_decT), 1, _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _stream())
-        return
-    _f32c(target, "target")
-    B, k = idx.shape
-    if not w_decT.is_contiguous() or w_decT.dtype not in (torch.float32, torch.bfloat16):
-        raise RuntimeError("w_decT must be contiguous [F, d] float32 or bfloat16")
-    lib = _lib.load()
-    _run("wsae_decode_backward", lib.wsae_decode_backward, _ptr(target), _ptr(w_decT), int(w_decT.dtype == torch.bfloat16), _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _stream())
+        _run("wsae_decode_backward", lib.wsae_decode_backward_typed, _ptr(target), _ptr(rows_at), _x_dtype_code(x_dtype), _ptr(w_decT), 1, _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _ptr(det_ws), _stream())
+    elif det_ws is not None:
+        if w_decT.dtype != torch.bfloat16 or not w_decT.is_contiguous():
+            raise RuntimeError("w_decT must be contiguous [F, d] bfloat16")
+        _run("wsae_decode_backward", lib.wsae_decode_backward_det, _ptr(target), None, _ptr(rows_at), _ptr(w_decT), 1, _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _ptr(det_ws), _stream())
+    else:
+        _f32c(target, "target")
+        if not w_decT.is_contiguous() or w_decT.dtype not in (torch.float32, torch.bfloat16):
+            raise RuntimeError("w_decT must be contiguous [F, d] float32 or bfloat16")
+        _run("wsae_decode_backward", lib.wsae_decode_backward, _ptr(target), _ptr(w_decT), int(w_decT.dtype == torch.bfloat16), _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(grad_out), float(coef), B, d, F, k, _ptr(resid), _ptr(resid_bf16), _ptr(stats), _ptr(last_activated), _ptr(step_count), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(dpre_val), _stream())
+    if det_ws is not None:
+        _run("wsae_det_finish", lib.wsae_det_finish, _ptr(det_ws), F, d, _ptr(grad_out), float(coef), _ptr(d_b_enc), _ptr(d_b_dec), _ptr(stats), _stream())
 
 
 @dataclass
@@ -675,14 +679,12 @@ def feature_topk_update(feat: Tensor, val: Tensor, rows: Tensor | None, k: int,
          _ptr(top_pos), _ptr(top_count), _ptr(total), _ptr(ws), need.value, _stream(), launches=4)
 
 
-_LN_DTYPES = {torch.float32: 0, torch.bfloat16: 1, torch.float16: 2}
-
-
 def layernorm_rows_(x: Tensor, gamma: Tensor | None, beta: Tensor | None, eps: float, out: Tensor,
                     row0: int = 0) -> None:
-    """out[row0 : row0 + n, :] = LayerNorm(x.reshape(n, d)) in fp32 (wsae_layernorm_rows;
+    """out[row0 : row0 + n, :] = LayerNorm(x.reshape(n, d)) (wsae_layernorm_rows_typed;
     sae/hooks.py:85-86,213-230: final LayerNorm of hooked hidden states + flatten, appended to the
-    activation matrix ``out``)."""
+    activation matrix ``out``).  Computed in fp32; ``out`` is float32, bfloat16 or float16, and a half
+    ``out`` receives the fp32 result rounded to nearest."""
     _need_cuda(x, gamma, beta, out)
     if x.dtype not in _LN_DTYPES:
         raise RuntimeError(f"unsupported activation dtype {x.dtype}")
@@ -698,11 +700,11 @@ def layernorm_rows_(x: Tensor, gamma: Tensor | None, beta: Tensor | None, eps: f
         beta = beta.to(torch.float32)
     _f32c(gamma, "layer_norm.weight")
     _f32c(beta, "layer_norm.bias")
-    if out.dtype != torch.float32 or out.dim() != 2 or out.shape[1] != d or out.stride(1) != 1:
-        raise RuntimeError("out must be a float32 [N, d] matrix with unit column stride")
+    if out.dtype not in _LN_DTYPES or out.dim() != 2 or out.shape[1] != d or out.stride(1) != 1:
+        raise RuntimeError("out must be a float32, bfloat16 or float16 [N, d] matrix with unit column stride")
     if row0 < 0 or row0 + n > out.shape[0]:
         raise RuntimeError(f"rows [{row0}, {row0 + n}) do not fit the [{out.shape[0]}, {d}] activation matrix")
     lib = _lib.load()
-    dst = out.data_ptr() + row0 * out.stride(0) * 4
-    _run("wsae_layernorm_rows", lib.wsae_layernorm_rows, _ptr(x2), _LN_DTYPES[x.dtype], n, d, x2.stride(0),
-         _ptr(gamma), _ptr(beta), float(eps), dst, out.stride(0), _stream())
+    dst = out.data_ptr() + row0 * out.stride(0) * out.element_size()
+    _run("wsae_layernorm_rows", lib.wsae_layernorm_rows_typed, _ptr(x2), _LN_DTYPES[x.dtype], n, d, x2.stride(0),
+         _ptr(gamma), _ptr(beta), float(eps), dst, _LN_DTYPES[out.dtype], out.stride(0), _stream())

@@ -52,7 +52,8 @@ class ActivationCache:
 
 
 class ActivationMatrix:
-    """Growable fp32 ``[N, d]`` matrix that hooked batches are normalised INTO, on the device.
+    """Growable ``[N, d]`` matrix (fp32, or bf16 / fp16 with ``dtype=``) that hooked batches are normalised
+    INTO, on the device.
 
     ``max_device_rows`` bounds the device-resident part: when the next batch would not fit, the rows
     gathered so far are spilled to pinned host memory (one D2H copy per spill, the reference copies
@@ -62,20 +63,21 @@ class ActivationMatrix:
     """
 
     def __init__(self, d: int, device: torch.device | str, capacity: int = 1 << 16,
-                 max_device_rows: int | None = None):
+                 max_device_rows: int | None = None, dtype: torch.dtype = torch.float32):
         self.d = d
+        self.dtype = dtype                 # float32, or bfloat16 / float16: the LayerNorm result rounded
         self.rows = 0                      # total rows appended (device part + spilled part)
         self._dev_rows = 0
         self._max = max_device_rows
         if max_device_rows is not None:
             capacity = min(capacity, max_device_rows)
-        self._buf = torch.empty((max(capacity, 1), d), dtype=torch.float32, device=device)
+        self._buf = torch.empty((max(capacity, 1), d), dtype=dtype, device=device)
         self._spilled: list[Tensor] = []
 
     def _spill(self) -> None:
         if self._dev_rows == 0:
             return
-        host = torch.empty((self._dev_rows, self.d), dtype=torch.float32, pin_memory=True)
+        host = torch.empty((self._dev_rows, self.d), dtype=self.dtype, pin_memory=True)
         host.copy_(self._buf[: self._dev_rows])
         self._spilled.append(host)
         self._dev_rows = 0
@@ -92,7 +94,7 @@ class ActivationMatrix:
         cap = max(need, 2 * self._buf.shape[0])
         if self._max is not None:
             cap = max(need, min(cap, self._max))
-        grown = torch.empty((cap, self.d), dtype=torch.float32, device=self._buf.device)
+        grown = torch.empty((cap, self.d), dtype=self.dtype, device=self._buf.device)
         if self._dev_rows:
             grown[: self._dev_rows].copy_(self._buf[: self._dev_rows])
         self._buf = grown

@@ -45,6 +45,8 @@ from .model import SAEOutput, TopKSAE, _fp32_terms, _SparseState
 # or chunked, K23 up to 256 (ops.decode_backward_supported), the K4 bucketing up to ~265.  Larger k
 # trains through the autograd node, eagerly.
 GRAPH_MAX_K = 256
+# batch dtypes the graphed step trains on (half batches are read in place or staged to fp32, exactly)
+_X_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
 
 
 @dataclass
@@ -191,6 +193,16 @@ class _GraphedStep:
         self._w_packed_buf: Tensor | None = None
         self._w_used_buf: Tensor | None = None
         self._x: Tensor | None = None     # staging buffer, allocated on first use
+        # Half-precision batches: the kernels that read the batch through x_slot (K0, K23, the row step)
+        # convert each element to fp32 as they load it, and their element type is baked into the captured
+        # graph.  So there is one captured graph per dtype the slot has named: `graph` / `_exec` /
+        # `kernels_per_replay` belong to the current `x_dtype`, the others wait in `_captured`.  Routes
+        # that do not read through the slot stage every batch into the fp32 `x` (an exact conversion).
+        self.x_dtype = torch.float32
+        self._captured: dict = {}         # dtype -> (graph, exec handle, kernels_per_replay)
+        self._warm: set = set()           # dtypes whose step has run eagerly once (loads their kernels)
+        self._xh: dict = {}               # per half dtype: staging buffer of host batches on in-place routes
+        self.captures = 0
         self._live: Tensor | None = None  # the batch the slot names (kept alive until the next step)
         self.one = torch.ones((), dtype=torch.float32, device=dev)
         self.params = [m.b_pre, m.encoder.weight, m.encoder.bias, m.decoder.weight, m.decoder.bias]
@@ -389,7 +401,8 @@ class _GraphedStep:
                 with torch.cuda.stream(self._side2):
                     w_used = ops.cast_bf16(w_decT, out=self._w_used_buf)
         if self.in_place:
-            a_packed = ops.pack_activations_at(self.x_slot, B, d, m.b_pre.data, rows_at=self.rows_slot)
+            a_packed = ops.pack_activations_at(self.x_slot, B, d, m.b_pre.data, rows_at=self.rows_slot,
+                                               x_dtype=self.x_dtype)
         else:
             a_packed = ops.pack_activations(x, m.b_pre.data, terms)
         if self.fork:
@@ -412,7 +425,8 @@ class _GraphedStep:
                                     d_w_enc=self.g_w_enc, d_w_decT=self.g_w_decT, target_is_slot=True,
                                     rows_at=self.rows_slot, w_enc=m.encoder.weight.data, d_b_pre=self.g_b_pre,
                                     finish=(self.ticket, m.dead_feature_threshold, self.stats[2:], self.seq_dev,
-                                            self.mailbox))      # counters + metrics mailbox by the last block
+                                            self.mailbox),      # counters + metrics mailbox by the last block
+                                    x_dtype=self.x_dtype)
             self._k4_forked = False
             self._mid = dict(use_gemm=False, buckets=None, resid_bf=None, B=B, d=d, coef=coef)
             st = self.state
@@ -434,7 +448,8 @@ class _GraphedStep:
                                 last_activated=m.feature_last_activated, step_count=m.step_count,
                                 d_b_enc=self.g_b_enc, d_b_dec=self.g_b_dec, dpre_val=dpre,
                                 target_is_slot=self.in_place,
-                                rows_at=self.rows_slot if self.in_place else None, det_ws=self.det_k23)
+                                rows_at=self.rows_slot if self.in_place else None, det_ws=self.det_k23,
+                                x_dtype=self.x_dtype)
         else:
             resid, _ = ops.decode_mse(x, w_used, m.decoder.bias.data, m.b_pre.data, idx, val,
                                       stats=self.stats, last_activated=m.feature_last_activated,
@@ -573,7 +588,7 @@ class _GraphedStep:
         rows_ptr = 0
         if isinstance(batch, IndexedBatch):
             f, r = batch.features, batch.rows
-            if (self.in_place and f.is_cuda and f.device == self.ctl.device and f.dtype == torch.float32
+            if (self.in_place and f.is_cuda and f.device == self.ctl.device and f.dtype in _X_DTYPES
                     and f.is_contiguous() and f.data_ptr() % 16 == 0 and r.is_cuda and r.is_contiguous()
                     and r.device == f.device):
                 src, rows_ptr = f, r.data_ptr()      # rows gathered inside K0 / K23
@@ -583,12 +598,23 @@ class _GraphedStep:
         if rows_ptr:
             pass
         elif (self.in_place and batch.is_cuda and batch.device == self.ctl.device
-                and batch.dtype == torch.float32 and batch.is_contiguous()
+                and batch.dtype in _X_DTYPES and batch.is_contiguous()
                 and batch.data_ptr() % 16 == 0):
             src = batch                      # trained on where it lies
+        elif self.in_place and batch.dtype != torch.float32:
+            # a half batch from the host: staged in its own dtype (2 bytes per element over PCIe)
+            src = self._xh.get(batch.dtype)
+            if src is None:
+                src = self._xh[batch.dtype] = torch.empty(tuple(batch.shape), dtype=batch.dtype,
+                                                          device=self.ctl.device)
+            src.copy_(batch, non_blocking=True)
         else:
-            self.x.copy_(batch, non_blocking=True)
+            self.x.copy_(batch, non_blocking=True)   # converts a half batch to fp32 exactly
             src = self.x
+        if src.dtype != self.x_dtype:        # switch to the captured graph of this dtype (if any)
+            self._captured[self.x_dtype] = (self.graph, self._exec, self.kernels_per_replay)
+            self.graph, self._exec, self.kernels_per_replay = self._captured.pop(src.dtype, (None, None, 0))
+            self.x_dtype = src.dtype
         self._live = src                     # the caller may drop its reference before the replay runs
         self.x_slot_np[0] = src.data_ptr()
         self.rows_slot_np[0] = rows_ptr
@@ -606,6 +632,7 @@ class _GraphedStep:
                 self._step_views.append((t, None if t.is_cuda else t.numpy()))
             self.graph = None             # new state tensors: the captured moment pointers are void
             self._exec = None
+            self._captured.clear()
         t0, v0 = self._step_views[0]
         step_t = float(v0 if v0 is not None else t0) + 1.0
         beta1, beta2 = group["betas"]
@@ -623,6 +650,7 @@ class _GraphedStep:
         if key != self._ptrs:      # storage was swapped behind our back (.data = ..., load): re-capture
             self.graph = None
             self._exec = None
+            self._captured.clear()
             if self._ptrs:
                 tr._dp_operands_fresh = False      # new weights: the gathered bf16 operands are void
             self._ptrs = key
@@ -635,7 +663,9 @@ class _GraphedStep:
                                        "fp32 rows were stale - call trainer.consolidate_weights() first")
                 self._refresh_operands()
             tr._dp_weights_stale = True      # after this step the fp32 rows of other ranks are one step behind
-        if self.calls > 1 and tr.cuda_graph == "segments":
+        fresh = self.x_dtype not in self._warm     # this dtype's kernels have not run yet: one eager step
+        self._warm.add(self.x_dtype)
+        if self.calls > 1 and not fresh and tr.cuda_graph == "segments":
             # data parallel: the kernels between the collectives are four CUDA graphs (compute up to
             # dW_enc | dW_dec + b_pre gradient | counters + gradient norm | optimizer), the NCCL calls
             # stay eager between them (capturing them into one graph hung on the 2-GPU box in round 1)
@@ -652,6 +682,7 @@ class _GraphedStep:
                 self.kernels_per_replay = ops.GPU_LAUNCHES - before
                 ops.GPU_LAUNCHES = before
                 self.graph = segs
+                self.captures += 1
             if not self._exec:        # raw cudaGraphExec_t handles of the four segments (see _launch_graph)
                 self._exec = [self._raw_exec(g) for g in self.graph]
             launch = self._launch_one
@@ -668,7 +699,7 @@ class _GraphedStep:
             if self.shard:
                 self._gather_weights()
             ops.GPU_LAUNCHES += self.kernels_per_replay
-        elif self.calls == 1 or tr.cuda_graph in ("eager", "segments"):
+        elif self.calls == 1 or fresh or tr.cuda_graph in ("eager", "segments"):
             self._body()
         else:
             if self.graph is None:
@@ -683,6 +714,7 @@ class _GraphedStep:
                 self.kernels_per_replay = ops.GPU_LAUNCHES - before   # captured, not yet executed
                 ops.GPU_LAUNCHES = before
                 self.graph = g
+                self.captures += 1
                 self._exec = None
             self._launch_graph()
             ops.GPU_LAUNCHES += self.kernels_per_replay
@@ -946,7 +978,7 @@ class SAETrainer:
         m = self.model
         if not (self.cuda_graph and isinstance(m, TopKSAE) and type(m).forward is TopKSAE.forward
                 and batch.dim() == 2 and batch.shape[1] == m.input_dim and m.input_dim % 4 == 0
-                and batch.dtype == torch.float32 and m.k <= GRAPH_MAX_K
+                and batch.dtype in _X_DTYPES and m.k <= GRAPH_MAX_K
                 and ops.bucket_supported(m.hidden_dim, m.k) and m.precision is None):
             return False
         # the five parameters by attribute (Module.parameters() walks the module tree: ~10 us per call)
@@ -1088,6 +1120,7 @@ class SAETrainer:
         for gs in self._graphs.values():
             gs.graph = None
             gs._exec = None
+            gs._captured.clear()
         self._graphs.clear()
         gc.collect()
         if str(self.device).startswith("cuda"):
