@@ -188,7 +188,8 @@ int wsae_backward_sparse(const float* resid, const float* x /*nullable if !d_w_e
  * k ranges: k <= 32 one warp per row; 32 < k <= 256 (d % 128 == 0 only) a team of ceil(k / 32)
  * warps per row, each holding 32 of the k gathered rows, meeting once per 64 columns to form the
  * residual.  Returns WSAE_E_UNSUPPORTED for an fp32 decoder, d % 8 != 0, k > 256, or k > 32 with
- * d % 128 != 0 or with wsae_decode_backward_det's workspace: use K2 + K3 then. */
+ * d % 128 != 0: use K2 + K3 then.  The deterministic form (wsae_decode_backward_det, or a non-NULL
+ * det_ws) covers the same shapes. */
 int wsae_decode_backward(const float* target, const void* w_decT, int w_is_bf16,
                          const float* b_dec, const float* b_pre /*nullable*/, const int32_t* idx,
                          const float* val, const float* grad_out /*nullable*/, float coef, int B,
@@ -353,6 +354,9 @@ int wsae_layernorm_rows_typed(const void* x, int in_dtype, long long rows, int d
  *       det_ws [F + d + 1] (caller-zeroed; addends are the unscaled dot products, |.| < 2^10);
  *       wsae_det_finish converts: d_b_enc += s*sum, d_b_dec += s*sum, stats.sse += sum,
  *       s = coef * (*grad_out).  target (direct) or target_at (slot) names the matrix; rows_at nullable.
+ *       Shapes: k <= 32 with d % 8 == 0, and 32 < k <= 256 with d % 128 == 0 (the team form: db_dec
+ *       and SSE are summed per block in team / warp order before the fixed-point add).  A feature
+ *       gets at most one db_enc addend per row at any k, so the int64 headroom does not depend on k.
  *   wsae_wgrad_gemm_det      : K4 with one partial slab per k split in ws (wsae_wgrad_gemm_workspace
  *       bytes; 0 = no split) and an ordered reduction instead of red.global.add.
  *   wsae_sumsq_det           : per-block partials in ws (wsae_sumsq_det_blocks() doubles), ordered sum.

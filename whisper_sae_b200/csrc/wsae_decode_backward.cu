@@ -1102,6 +1102,13 @@ decode_backward_tc_kernel(const TX* __restrict__ target, const __nv_bfloat16* __
 // tensor form is one shared-memory exchange and one barrier per half slice.  Entries past k (the tail
 // of the last warp) get activation 0 and gather a spread-out row, like the tensor form's invalid
 // entries: they add nothing and get no dv.
+//
+// kDet (deterministic form, det_ws as in wsae_decode_backward_det): the three cross-row sums go to
+// det_ws with det_add instead of float atomics - db_enc one unscaled dot product per fired entry,
+// db_dec the block's per-team partials summed in team order, the SSE the block's per-warp partials
+// summed in warp order.  A feature appears at most once among a row's k entries, so it still gets at
+// most one db_enc addend per row whatever k is, and the int64 headroom of kDetScaleEnc holds as at
+// k <= 32.  kDet = false is the default form, unchanged (det_ws unused).
 // ================================================================================================
 constexpr int kWideMaxK = 256;
 constexpr int kWideMaxWarps = 8;
@@ -1110,7 +1117,7 @@ __device__ __forceinline__ void team_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-template <typename TX>
+template <bool kDet, typename TX>
 __global__ void __maxnreg__(160)   // 156 registers, no spills: the tensor form's budget
 decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* __restrict__ w_decT,
                             const float* __restrict__ b_dec, const float* __restrict__ b_pre,
@@ -1121,7 +1128,8 @@ decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* 
                             const long long* __restrict__ step_count, float* __restrict__ d_b_enc,
                             float* __restrict__ d_b_dec, float* __restrict__ dpre_val,
                             const TX* const* __restrict__ target_at,
-                            const long long* const* __restrict__ rows_at, int stamp_words, int l2hint) {
+                            const long long* const* __restrict__ rows_at, int stamp_words, int l2hint,
+                            long long* __restrict__ det_ws) {
   const uint64_t pol_x = l2_policy((l2hint & 1) ? 1 : 0);
   const uint64_t pol_w = l2_policy((l2hint & 2) ? 2 : 0);
   // [d] bias | [teams][d] db_dec partials | [2][warps][64] partial reconstructions |
@@ -1352,7 +1360,10 @@ decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* 
     const float my_dv = fired ? s * dot : 0.f;
     if (entry < k) {
       if (dpre_val != nullptr) dpre_val[static_cast<size_t>(row) * k + entry] = my_dv;
-      if (fired && d_b_enc != nullptr) atomicAdd(d_b_enc + my_i, my_dv);
+      if (fired && d_b_enc != nullptr) {
+        if constexpr (kDet) det_add(det_ws + my_i, static_cast<double>(dot), kDetScaleEnc);
+        else atomicAdd(d_b_enc + my_i, my_dv);
+      }
     }
     cur_i = nxt_i; cur_v = nxt_v;
     nxt_i = nn_i; nxt_v = nn_v;
@@ -1373,7 +1384,8 @@ decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* 
     for (int i = threadIdx.x; i < d; i += blockDim.x) {
       float t = 0.f;
       for (int tm = 0; tm < teams; ++tm) t += fsm[d + tm * d + i];
-      atomicAdd(d_b_dec + i, s * t);
+      if constexpr (kDet) det_add(det_ws + F + i, static_cast<double>(t), kDetScaleDec);
+      else atomicAdd(d_b_dec + i, s * t);
     }
   if (threadIdx.x == 0 && stats != nullptr) {
     double tsum = 0.0;
@@ -1382,7 +1394,8 @@ decode_backward_wide_kernel(const TX* __restrict__ target, const __nv_bfloat16* 
       tsum += static_cast<double>(s_sse[w]);
       c += s_l0[w];
     }
-    atomicAdd(&stats->sse, tsum);
+    if constexpr (kDet) det_add(det_ws + F + d, tsum, kDetScaleSse);
+    else atomicAdd(&stats->sse, tsum);
     atomicAdd(&stats->l0_count, c);
   }
 }
@@ -1413,11 +1426,11 @@ using namespace wsae;
 
 extern "C" int wsae_debug_decode_backward_general(int on) { g_decode_backward_general = on; return 0; }
 
-// The wide form (32 < k <= 256, d % 128 == 0, no deterministic workspace).  Teams of ceil(k / 32)
-// warps, two teams per block while they fit in 4 warps, else one.
+// The wide form (32 < k <= 256, d % 128 == 0; det_ws non-null: its deterministic form).  Teams of
+// ceil(k / 32) warps, two teams per block while they fit in 4 warps, else one.
 template <typename TX>
 static int decode_backward_wide(const TX* target, const TX* const* target_at,
-                                const long long* const* rows_at, const __nv_bfloat16* w_decT,
+                                const long long* const* rows_at, long long* det_ws, const __nv_bfloat16* w_decT,
                                 const float* b_dec, const float* b_pre, const int32_t* idx,
                                 const float* val, const float* grad_out, float coef, int B, int d,
                                 int F, int k, float* resid, __nv_bfloat16* resid_bf16, FusedStats* stats,
@@ -1433,31 +1446,32 @@ static int decode_backward_wide(const TX* target, const TX* const* target_at,
   const size_t smem = ((1 + teams) * static_cast<size_t>(d) + 2 * nwarps * 64) * sizeof(float) +
                       static_cast<size_t>(nwarps) * kTcGBytes + 16 + static_cast<size_t>(stamp_words) * 4;
   if (smem > 200 * 1024) return kUnsupported;
+  const auto kern = det_ws != nullptr ? decode_backward_wide_kernel<true, TX> : decode_backward_wide_kernel<false, TX>;
   static bool attr_set[64] = {};
   if (dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(decode_backward_wide_kernel<TX>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaError_t e = cudaSuccess;
+    for (auto kf : {decode_backward_wide_kernel<false, TX>, decode_backward_wide_kernel<true, TX>})
+      if (e == cudaSuccess) e = cudaFuncSetAttribute(kf, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     if (e != cudaSuccess) return static_cast<int>(e);
     if (dev < 64) attr_set[dev] = true;
   }
   int per = 0;
-  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, decode_backward_wide_kernel<TX>,
-                                                                nwarps * 32, smem);
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, kern, nwarps * 32, smem);
   if (e != cudaSuccess) return static_cast<int>(e);
   if (per < 1) per = 1;
   int nblk = ceil_div(B, teams);
   if (nblk > sms * per) nblk = sms * per;
   // L2 hints as in the tensor form: decoder rows evict_last while the bf16 decoder fits in 48 MB
   const int l2hint = static_cast<long long>(F) * d * 2 <= (48LL << 20) ? 3 : 1;
-  launch_pdl(decode_backward_wide_kernel<TX>, nblk, nwarps * 32, smem, stream, target, w_decT, b_dec, b_pre, idx,
+  launch_pdl(kern, nblk, nwarps * 32, smem, stream, target, w_decT, b_dec, b_pre, idx,
              val, grad_out, coef, B, d, F, k, resid, resid_bf16, stats, last_activated, step_count, d_b_enc,
-             d_b_dec, dpre_val, target_at, rows_at, stamp_words, l2hint);
+             d_b_dec, dpre_val, target_at, rows_at, stamp_words, l2hint, det_ws);
   return static_cast<int>(cudaGetLastError());
 }
 
 // See include/wsae.h.  Returns WSAE_E_UNSUPPORTED for shapes the fused kernels do not cover
-// (fp32 decoder, d % 8 != 0, k > 256, 32 < k with d % 128 != 0 or a deterministic workspace):
-// callers then use K2 + K3.  TX: element type of the target matrix.
+// (fp32 decoder, d % 8 != 0, k > 256, 32 < k with d % 128 != 0): callers then use K2 + K3.
+// A deterministic workspace is accepted at every covered shape.  TX: element type of the target matrix.
 template <typename TX>
 static int decode_backward_launch(const TX* target, const TX* const* target_at,
                                   const long long* const* rows_at, long long* det_ws, const void* w_decT, int w_is_bf16, const float* b_dec,
@@ -1472,8 +1486,8 @@ static int decode_backward_launch(const TX* target, const TX* const* target_at,
   if (!w_is_bf16 || d % 8 != 0 || d > 8192) return kUnsupported;
   if (static_cast<long long>(F) * (d / 4) > 0x7fffffffLL) return kUnsupported;
   if (k > 32) {
-    if (k > kWideMaxK || d % 128 != 0 || det_ws != nullptr) return kUnsupported;
-    return decode_backward_wide(target, target_at, rows_at, static_cast<const __nv_bfloat16*>(w_decT), b_dec,
+    if (k > kWideMaxK || d % 128 != 0) return kUnsupported;
+    return decode_backward_wide(target, target_at, rows_at, det_ws, static_cast<const __nv_bfloat16*>(w_decT), b_dec,
                                 b_pre, idx, val, grad_out, coef, B, d, F, k, resid,
                                 static_cast<__nv_bfloat16*>(resid_bf16), static_cast<FusedStats*>(stats),
                                 last_activated, step_count, d_b_enc, d_b_dec, dpre_val, stream);

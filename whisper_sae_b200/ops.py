@@ -400,17 +400,19 @@ def row_step(pre: Tensor, target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: 
 DECODE_BACKWARD_MAX_K = 256
 
 
-def decode_backward_supported(d: int, k: int, bf16: bool) -> bool:
+def decode_backward_supported(d: int, k: int, bf16: bool, deterministic: bool = False) -> bool:
     """Shapes covered by the fused K23 kernels (else: decode_mse + backward_sparse): k <= 32 with
     d % 8 == 0, and 64 < k <= 256 with d % 128 == 0 (the team-of-warps form).  33 <= k <= 64 stays on
-    K2 + K3 unless WSAE_WIDE_K23=1 routes it to the team form too."""
+    K2 + K3 unless WSAE_WIDE_K23=1 routes it to the team form too.  ``deterministic``: the shapes of
+    the deterministic form (``det_ws``), which has no K2 + K3 counterpart, so 33 <= k <= 64 takes the
+    team form whatever WSAE_WIDE_K23 says."""
     if not (bf16 and d % 8 == 0 and os.environ.get("WSAE_FUSED_DECODE", "1") != "0"):
         return False
     if k <= 32:
         return True
     if d % 128 != 0 or k > DECODE_BACKWARD_MAX_K:
         return False
-    return k > 64 or os.environ.get("WSAE_WIDE_K23", "0") == "1"
+    return deterministic or k > 64 or os.environ.get("WSAE_WIDE_K23", "0") == "1"
 
 
 def decode_backward(target: Tensor, w_decT: Tensor, b_dec: Tensor, b_pre: Tensor | None,

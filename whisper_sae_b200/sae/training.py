@@ -170,8 +170,10 @@ class _GraphedStep:
         self.seq_np = self.seq_host.numpy()
         self._step_views: list = []       # (optimizer `step` tensor, its 0-d numpy view) per parameter
         d_in, k_sel = m.input_dim, m.k
+        # the deterministic step takes K23 wherever its deterministic form exists (33 <= k <= 64 included),
+        # so staging and the K23 / K2 + K3 choice in _compute_a follow the same predicate
         self.in_place = (self.bf16 and d_in % 8 == 0 and ops.wgrad_gemm_supported(d_in)
-                         and ops.decode_backward_supported(d_in, k_sel, True))
+                         and ops.decode_backward_supported(d_in, k_sel, True, bool(trainer.deterministic)))
         # Single-GPU bf16 step: the small kernels that do not sit on the K0 -> K1 -> K23 -> K4 chain run
         # on a side stream (a forked branch of the captured graph): [encoder pack, decoder bf16 cast]
         # next to the activation pack, and [counters + mailbox, b_pre gradient] next to the bucketing
@@ -252,9 +254,10 @@ class _GraphedStep:
         self.state = _SparseState()
         # deterministic mode workspaces (bf16 step with K23 + K4 only)
         self.det = bool(trainer.deterministic) and self.bf16 and ops.wgrad_gemm_supported(d_in) \
-            and k_sel <= 32 and ops.decode_backward_supported(d_in, k_sel, True)
+            and ops.decode_backward_supported(d_in, k_sel, True, deterministic=True)
         if trainer.deterministic and not self.det:
-            raise RuntimeError("deterministic=True covers the bf16 (use_amp) graphed step with d % 8 == 0, k <= 32")
+            raise RuntimeError("deterministic=True covers the bf16 (use_amp) graphed step with d % 8 == 0 and "
+                               "k <= 32, or d % 128 == 0 and k <= 256")
         self.det_k23 = self.det_k4 = self.det_sumsq = self.det_bpre = None
         if self.det:
             self.det_k23 = torch.zeros(F + d + 1, dtype=torch.int64, device=dev)
@@ -438,7 +441,7 @@ class _GraphedStep:
             w_used = ops.cast_bf16(w_decT) if self.bf16 else w_decT
         dpre = torch.empty((B, k), dtype=torch.float32, device=dev)
         use_gemm = self.bf16 and ops.wgrad_gemm_supported(d)
-        if use_gemm and ops.decode_backward_supported(d, k, True):
+        if use_gemm and ops.decode_backward_supported(d, k, True, self.det):
             # K23: decode + MSE + stamps + dv + bias gradients in one pass over the gathered rows
             resid = None          # fp32 residual only on demand (SAEOutput.reconstructed, resampling)
             resid_bf = torch.empty((B, d), dtype=torch.bfloat16, device=dev)
