@@ -106,11 +106,15 @@ int wsae_encode_topk_dense(const void* a_packed, const void* w_packed, int B, in
                            int Kp, int k_used_cols, int k, float* pre_ws, float* out_val /*[B,k]*/,
                            int32_t* out_idx /*[B,k]*/, wsae_stream_t stream);
 
-/* K1 for k > 64 (the fused epilogue of wsae_encode_topk stops at k = 64): wsae_encode_topk_dense
- * over consecutive chunks of chunk_rows packed rows (a multiple of 128), one library call.  pre_ws is
- * chunk_rows * F floats of scratch, reused by every chunk (size it to stay in L2: ~32-48 MB).
- * Results bit-identical to one wsae_encode_topk_dense call over all B rows.  F <= 49152, F % 4 == 0,
- * k <= 65535. */
+/* K1 for k > 64 (the fused epilogue of wsae_encode_topk stops at k = 64): the GEMM and row select of
+ * wsae_encode_topk_dense over consecutive chunks of chunk_rows packed rows (a multiple of 128), one
+ * library call, at any F.  pre_ws is scratch reused by every chunk (size it to stay in L2: ~32-48 MB):
+ * chunk_rows * Fr floats with Fr = round_up(F, 4) when F <= 49152; above that the select runs on
+ * nslices = ceil(F / 49152) column slices, whose k candidates each are merged, and pre_ws needs
+ * chunk_rows * (Fr + 2 * nslices * k) floats.  Same values and tie rule as wsae_encode_topk_dense
+ * (bit-identical to one such call over all B rows where that call runs); output in ascending feature
+ * index.  k <= 65535, and ceil(nslices * k / 32) <= 64 (F up to 393216 at k = 256):
+ * WSAE_E_UNSUPPORTED otherwise. */
 int wsae_encode_topk_chunked(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
                              int Kp, int k_used_cols, int k, int chunk_rows, float* pre_ws,
                              float* out_val /*[B,k]*/, int32_t* out_idx /*[B,k]*/, wsae_stream_t stream);

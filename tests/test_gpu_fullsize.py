@@ -124,7 +124,8 @@ def test_fullsize_train_step_invariants(tmp_path):
         assert torch.isfinite(p).all() and not torch.equal(p, w0[n]), n
 
 
-@pytest.mark.parametrize("shape", [(75776, 384, 3072), (8192, 768, 6144), (2048, 1280, 40960)])
+@pytest.mark.parametrize("shape", [(75776, 384, 3072), (8192, 768, 6144), (2048, 1280, 40960), (16384, 512, 4096),
+                                   (8192, 1024, 8192)])
 def test_deterministic_mode_is_bit_reproducible(shape, tmp_path):
     """SAETrainer(deterministic=True): two runs of the bf16 graphed step from the same state on the
     same batches are BIT-identical (losses, every parameter, AdamW moments, counters) - split-K
@@ -166,16 +167,25 @@ def test_deterministic_mode_is_bit_reproducible(shape, tmp_path):
         assert rel < 1e-3, f"{n}: deterministic vs default rel-L2 {rel:.2e}"
 
 
-@pytest.mark.parametrize("rows,d,f", [(75776, 768, 6144), (37888, 1280, 40960)])
-def test_fullsize_step_gradients_small_and_large_v3(rows, d, f, tmp_path):
-    """BASELINE configs 3 / 4 at the bench's own batch sizes: loss, L0, fired set and the four gradient
-    tensors of ONE bf16 step against a dense fp32 statement with the same bf16 operand roundings in the
-    forward (the golden traces at these widths are 256-row batches)."""
+@pytest.mark.parametrize("rows,d,f,k", [
+    pytest.param(75776, 768, 6144, K, id="75776-768-6144"),
+    pytest.param(37888, 1280, 40960, K, id="37888-1280-40960"),
+    pytest.param(16384, 512, 4096, 32, id="base-16384-512-4096-k32"),
+    pytest.param(16384, 512, 4096, 128, id="base-16384-512-4096-k128"),
+    pytest.param(16384, 1024, 8192, 64, id="medium-16384-1024-8192-k64"),      # K2 + K3 + K4
+    pytest.param(4096, 1280, 81920, 128, id="large-4096-1280-81920-k128"),     # chunked K1 in column slices
+    pytest.param(2048, 1024, 65536, 256, id="medium-2048-1024-65536-k256"),
+])
+def test_fullsize_step_gradients_small_and_large_v3(rows, d, f, k, tmp_path):
+    """BASELINE configs 3 / 4 at the bench's own batch sizes, and the Whisper base / medium widths and
+    more than 65 536 features at k up to 256: loss, L0, fired set and the five gradient tensors of ONE
+    graphed bf16 step against a dense fp32 statement with the same bf16 operand roundings in the forward
+    (the golden traces at these widths are 256-row batches)."""
     from whisper_sae_b200.config import TrainingConfig
     from whisper_sae_b200.sae import SAETrainer, TopKSAE
 
     torch.manual_seed(42)
-    sae = TopKSAE(d, f, k=K, dead_feature_threshold=10_000)
+    sae = TopKSAE(d, f, k=k, dead_feature_threshold=10_000)
     tr = SAETrainer(sae, TrainingConfig(batch_size=rows, use_amp=True, num_workers=0), device="cuda", run_dir=tmp_path)
     tr.setup_scheduler(1000)
     x = O.synthetic_activations(rows, d, seed=17).cuda()
@@ -183,7 +193,7 @@ def test_fullsize_step_gradients_small_and_large_v3(rows, d, f, tmp_path):
     with torch.no_grad():
         xc = x - w["b_pre"]
         pre = xc.to(torch.bfloat16).float() @ w["encoder.weight"].to(torch.bfloat16).float().t() + w["encoder.bias"]
-        v, i = torch.topk(pre, K, dim=1)
+        v, i = torch.topk(pre, k, dim=1)
         del pre
         wd = w["decoder.weight"].t().to(torch.bfloat16).float()
         hidden = torch.zeros(rows, f, device="cuda").scatter_(1, i, torch.relu(v))
@@ -199,6 +209,7 @@ def test_fullsize_step_gradients_small_and_large_v3(rows, d, f, tmp_path):
         l0_ref = float((v > 0).sum()) / rows
         del hidden, dpre, resid, g
     m = tr.train_step(x)
+    assert rows in tr._graphs          # the step ran the graphed route's kernels (the first call is not captured)
     assert m.loss == pytest.approx(loss_ref, rel=1e-4)
     assert m.l0 == pytest.approx(l0_ref, abs=1e-3)
     assert torch.equal(sae.feature_last_activated > 0, fired)

@@ -136,7 +136,7 @@ def test_crosscoder_fp32_matches_reference(name):
 
 
 @pytest.mark.parametrize("precision,tol", [("fp32", 1e-5), ("bf16", 2e-2)])
-def test_crosscoder_whisper_tiny_shape(precision, tol):
+def test_crosscoder_whisper_tiny_shape(precision, tol, monkeypatch):
     """tests/test_crosscoder.py:421-436 shape (BASELINE config 5): d=384, 4 layers, 3072 features, k=32."""
     fx = load_golden("variants_crosscoder")["crosscoder_tiny_384x4_3072_k32"]
     r = fx["recipe"]
@@ -149,10 +149,27 @@ def test_crosscoder_whisper_tiny_shape(precision, tol):
     assert out.hidden.shape == (r["B"], r["F"])
     for n, p in m.named_parameters():
         g, dg = p.grad.detach().cpu(), fx["grads"][n]
-        assert abs(g.double().abs().sum().item() - dg["abs_sum"]) <= max(tol * 50, 1e-4) * dg["abs_sum"] + 1e-9
         if precision == "fp32":
+            assert abs(g.double().abs().sum().item() - dg["abs_sum"]) <= 5e-4 * dg["abs_sum"] + 1e-9
             torch.testing.assert_close(g.reshape(-1)[::997], dg["sample"], rtol=1e-3,
                                        atol=1e-5 * dg["sample"].abs().max().item() + 1e-12)
+        else:
+            # bf16 against the fp32 golden: the TopK sets differ where bf16 rounding reorders near ties, which
+            # moves whole weight-gradient rows (measured on a B200: rel L2 0.112 W_enc, 0.066 W_dec, 9e-4 b_enc)
+            sample = dg["sample"].double()
+            rel = ((g.reshape(-1)[::997].double() - sample).norm() / sample.norm()).item()
+            assert rel <= (0.15 if n in ("W_enc", "W_dec") else tol), (n, rel)
+    if precision == "bf16":
+        # d = 4 x 384 = 1536 runs K4 at nb_tile = 8 (two stages, a second MMA at N = 256, all 512 TMEM
+        # columns): its weight gradients must be those of K3's scatter on the same step (measured on a
+        # B200: rel L2 2.4e-3 W_enc, 2.5e-3 W_dec; both are bf16 products summed in different orders)
+        monkeypatch.setenv("WSAE_WGRAD", "scatter")
+        m2 = _build_crosscoder(r, precision)
+        m2(acts).loss.backward()
+        for n, p in m2.named_parameters():
+            ref, got = p.grad.detach().double(), dict(m.named_parameters())[n].grad.detach().double()
+            rel = ((got - ref).norm() / ref.norm()).item()
+            assert rel <= 1e-2, (n, rel)
 
 
 @pytest.mark.parametrize("kind", ["transcoder", "skip", "crosscoder"])

@@ -51,6 +51,8 @@ def _case(B, d, F, k, seed, pitch=None):
     (1000, 96, 1000, 16),       # d not a multiple of 64
     (512, 768, 6144, 32),       # whisper-small (N = 768: three MMAs per k-step? -> n tiles)
     (300, 1280, 2048, 32),      # large-v3 width (n tiles of 7*64 / 6*64 columns)
+    (300, 512, 4096, 32),       # whisper-base: 8 x 64-column n tiles, 2 stages, second MMA at N = 256
+    (200, 1024, 2176, 32),      # whisper-medium: the same n tiling, odd feature-tile count
 ])
 def test_wgrad_gemm_matches_dense(B, d, F, k):
     _case(B, d, F, k, seed=B + d)

@@ -28,7 +28,11 @@ def _ops():
     (512, 384, 3072, 128, True, "dense", True, True),         # small batch: the dense form, any k
     (4096, 392, 3072, 128, True, "chunked", False, True),     # d % 128 != 0: K2 + K3
     (4096, 384, 3072, 128, False, "chunked", False, True),    # fp32 decoder: K2 + K3
-    (2176, 1280, 65536, 128, True, "fused", True, True),      # F beyond the dense form's shared memory
+    (2176, 1280, 65536, 128, True, "chunked", True, True),    # F beyond one select's shared memory: slices
+    (4096, 1280, 81920, 128, True, "chunked", True, True),
+    (512, 1280, 81920, 128, True, "chunked", True, True),     # small batch, but too wide for "dense"
+    (4096, 384, 3002, 100, True, "chunked", True, True),      # F % 4 != 0: the scratch has a row pitch
+    (2176, 1280, 65536, 64, True, "fused", False, True),       # k <= 64 keeps the fused route
 ])
 def test_routing(B, d, F, k, bf16, k1, k23, graph, monkeypatch):
     monkeypatch.delenv("WSAE_WIDE_K23", raising=False)
@@ -38,6 +42,10 @@ def test_routing(B, d, F, k, bf16, k1, k23, graph, monkeypatch):
 
     ops = _ops()
     assert ops.encode_route(B, F, k) == k1
+    if k > ops.ENCODE_FUSED_MAX_K:      # the fused epilogue cannot run k > 64, with or without an F-split
+        assert ops.encode_route(B, F, k, nsplit=4) == "chunked"
+        for Bx, Fx in [(1, 3072), (1024, 49153), (1025, 3002), (75776, 393216), (100, 131072)]:
+            assert ops.encode_route(Bx, Fx, k) != "fused"
     assert ops.decode_backward_supported(d, k, bf16) == k23
     if k > 256:      # the bf16 backward then scatters through K3 instead of bucketing for K4
         assert ops.bucket_supported(F, k) == (k < 266)
@@ -62,10 +70,14 @@ def test_routing_wide_k23_switch(monkeypatch):
 
 def test_chunk_rows():
     ops = _ops()
-    for B, F in [(75776, 3072), (75776, 6144), (2176, 40960), (5000, 49152), (100, 3072)]:
-        r = ops.encode_chunk_rows(B, F)
+    for B, F, k in [(75776, 3072, 128), (75776, 6144, 256), (2176, 40960, 65), (5000, 49152, 128),
+                    (100, 3072, 65), (4096, 81920, 128), (4096, 3002, 100), (75776, 393216, 256)]:
+        r = ops.encode_chunk_rows(B, F, k)
         assert r % 128 == 0 and r >= 128 and r <= (B + 127) // 128 * 128
-        assert r == 128 or r * F * 4 <= 40 << 20
+        assert r == 128 or ops.encode_chunk_scratch_floats(F, k, r) * 4 <= 40 << 20
+    assert ops.encode_chunk_scratch_floats(49152, 256, 128) == 128 * 49152             # one slice: no lists
+    assert ops.encode_chunk_scratch_floats(3002, 65, 128) == 128 * 3004                 # row pitch
+    assert ops.encode_chunk_scratch_floats(81920, 128, 256) == 256 * (81920 + 2 * 2 * 128)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -80,7 +92,7 @@ def test_k1_chunked_matches_unchunked_dense(B, d, F, k):
     from whisper_sae_b200 import _lib
     ops = _ops()
     assert ops.encode_route(B, F, k) == "chunked"
-    assert (B + ops.encode_chunk_rows(B, F) - 1) // ops.encode_chunk_rows(B, F) >= 2
+    assert (B + ops.encode_chunk_rows(B, F, k) - 1) // ops.encode_chunk_rows(B, F, k) >= 2
     torch.manual_seed(B + k)
     state = O.init_state(d, F)
     state["b_pre"] = torch.randn(d) * 0.05
@@ -116,11 +128,11 @@ def test_k1_chunked_matches_unchunked_dense(B, d, F, k):
 # ------------------------------------------------------------------------------------------------
 # 3. K23, team-of-warps form, against the oracle
 # ------------------------------------------------------------------------------------------------
-_K23_F = {384: 3072, 768: 6144, 1280: 4096}
+_K23_F = {384: 3072, 512: 4096, 768: 6144, 1024: 8192, 1280: 4096}
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("d", [384, 768, 1280])
+@pytest.mark.parametrize("d", [384, 512, 768, 1024, 1280])
 @pytest.mark.parametrize("k", [33, 64, 65, 128, 256])
 def test_k23_wide_matches_oracle(k, d):
     """The test_decode_backward_fused recipe (tests/test_gpu_sparse.py) at 32 < k <= 256 on a ragged

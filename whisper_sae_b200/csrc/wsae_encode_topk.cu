@@ -1768,6 +1768,11 @@ topk_merge_kernel(const float* __restrict__ part_val, const int32_t* __restrict_
     }
     base += __popc(keep_mask);
   }
+  // fewer than k valid candidates (NaN rows): pad with (-inf, -1) as the unmerged lists are
+  for (int slot = base + lane; slot < k; slot += 32) {
+    out_val[static_cast<size_t>(row) * k + slot] = __uint_as_float(0xff800000u);
+    out_idx[static_cast<size_t>(row) * k + slot] = -1;
+  }
 }
 
 // ================================================================================================
@@ -1788,7 +1793,7 @@ topk_merge_kernel(const float* __restrict__ part_val, const int32_t* __restrict_
 template <int STAGES>
 __global__ void __launch_bounds__(256, 1)
 encode_dense_kernel(const __grid_constant__ CUtensorMap tmap_a,
-                    const __grid_constant__ CUtensorMap tmap_w, int B, int F, int ksteps,
+                    const __grid_constant__ CUtensorMap tmap_w, int B, int F, int ld, int ksteps,
                     int num_m_blocks, int num_n_tiles, float* __restrict__ pre) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1850,7 +1855,7 @@ encode_dense_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const int row = m_blk * kBM + row_in_blk;
       const int col0 = nt * kBN;
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * kBN;
-      float* out = pre + static_cast<size_t>(row < B ? row : 0) * F + col0;
+      float* out = pre + static_cast<size_t>(row < B ? row : 0) * ld + col0;
       uint32_t ra[16], rb[16];
       tmem_ld16(taddr, ra);
 #pragma unroll 1
@@ -1895,17 +1900,21 @@ encode_dense_kernel(const __grid_constant__ CUtensorMap tmap_a,
   }
 }
 
-// One block (256 threads) per row: the k largest of pre[row, 0:F] (block_row_topk, wsae_rowselect.cuh).
+// One block (256 threads) per (row, column slice): the k largest of pre[row, c0 : c0 + S] with
+// c0 = blockIdx.y * S (block_row_topk, wsae_rowselect.cuh), written with their feature indices to the
+// slice's k slots of the row's gridDim.y * k list.  One slice (S >= F) is the whole row.
 __global__ void __launch_bounds__(kRowTopkThreads)
-rowwise_topk_kernel(const float* __restrict__ pre, int B, int F, int k, float* __restrict__ out_val,
-                    int32_t* __restrict__ out_idx) {
-  extern __shared__ __align__(16) uint32_t s_key[];          // [F]
+rowwise_topk_kernel(const float* __restrict__ pre, int B, int F, int ld, int S, int k,
+                    float* __restrict__ out_val, int32_t* __restrict__ out_idx) {
+  extern __shared__ __align__(16) uint32_t s_key[];          // [S]
   __shared__ RowSelectSmem sm;
   pdl_prologue();
   const int row = blockIdx.x;
   if (row >= B) return;
-  block_row_topk(pre + static_cast<size_t>(row) * F, F, k, s_key, sm, out_val + static_cast<size_t>(row) * k,
-                 out_idx + static_cast<size_t>(row) * k);
+  const int c0 = blockIdx.y * S;
+  const size_t o = (static_cast<size_t>(row) * gridDim.y + blockIdx.y) * k;
+  block_row_topk(pre + static_cast<size_t>(row) * ld + c0, min(S, F - c0), k, s_key, sm, out_val + o,
+                 out_idx + o, c0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2137,14 +2146,15 @@ extern "C" int wsae_encode_topk(const void* a_packed, const void* w_packed, int 
 }
 
 
-// The GEMM half of the small-batch form: pre_ws[B, F] = A' x W'^T (bias included), nothing else.
-extern "C" int wsae_encode_dense(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
-                                 int Kp, int k_used_cols, float* pre_ws, cudaStream_t stream) {
-  if (!a_packed || !w_packed || !pre_ws) return kBadArg;
+// The GEMM half of the small-batch form: pre[B, F] = A' x W'^T (bias included) with row pitch ld
+// (a multiple of 4: the epilogue stores 16-byte vectors), nothing else.
+static int encode_dense_ld(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp, int Kp,
+                           int k_used_cols, int ld, float* pre, cudaStream_t stream) {
+  if (!a_packed || !w_packed || !pre) return kBadArg;
   if (B <= 0 || F <= 0) return kBadArg;
   if (Bp % kBM != 0 || Fp % kBN != 0 || Kp % kBK != 0 || Bp < B || Fp < F) return kBadArg;
   if (k_used_cols <= 0 || k_used_cols % 16 != 0 || k_used_cols > Kp) return kBadArg;
-  if (F % 4 != 0) return kUnsupported;
+  if (ld < F || ld % 4 != 0) return kBadArg;
   CUtensorMap ta, tw;
   int rc = make_tmap_bf16(&ta, a_packed, static_cast<uint64_t>(Bp), static_cast<uint64_t>(Kp), kBM);
   if (rc) return rc;
@@ -2166,9 +2176,55 @@ extern "C" int wsae_encode_dense(const void* a_packed, const void* w_packed, int
   const int num_n_tiles = ceil_div(F, kBN);
   const int total = num_m_blocks * num_n_tiles;
   const int grid = total < num_sms ? total : num_sms;
-  cudaError_t e = launch_pdl(encode_dense_kernel<kStages>, grid, 256, smem_g, stream, ta, tw, B, F,
-                             k_used_cols / 16, num_m_blocks, num_n_tiles, pre_ws);
+  cudaError_t e = launch_pdl(encode_dense_kernel<kStages>, grid, 256, smem_g, stream, ta, tw, B, F, ld,
+                             k_used_cols / 16, num_m_blocks, num_n_tiles, pre);
   return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
+}
+
+extern "C" int wsae_encode_dense(const void* a_packed, const void* w_packed, int B, int Bp, int F, int Fp,
+                                 int Kp, int k_used_cols, float* pre_ws, cudaStream_t stream) {
+  if (F > 0 && F % 4 != 0) return kUnsupported;
+  return encode_dense_ld(a_packed, w_packed, B, Bp, F, Fp, Kp, k_used_cols, F, pre_ws, stream);
+}
+
+// Column slices of the row select: the keys of one slice fill at most 192 KB of shared memory.
+constexpr int kSelectMaxCols = 49152;
+static int select_slices(int F) { return ceil_div(F, kSelectMaxCols); }
+static int select_slice_cols(int F) { return round_up(ceil_div(F, select_slices(F)), 4); }
+
+// The select half: per row of pre (pitch ld), the k largest of pre[row, 0:F] in ascending feature index.
+// One slice: one block per row, straight into out_*.  Several: one block per (row, slice) writes k
+// candidates per slice to part_* ([B, nslices * k], ascending feature index, short slices padded with
+// (-inf, -1)), and topk_merge_kernel keeps the k largest, ties to the earlier candidate, i.e. to the
+// lowest feature index, as one unsliced select does.
+static int rowwise_select(const float* pre, int B, int F, int ld, int k, float* part_val, int32_t* part_idx,
+                          float* out_val, int32_t* out_idx, cudaStream_t stream) {
+  const int ns = select_slices(F);
+  const int S = select_slice_cols(F);
+  int dev = 0;
+  cudaGetDevice(&dev);
+  static bool attr_set[64] = {};
+  if (dev >= 64 || !attr_set[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(rowwise_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    if (e != cudaSuccess) return static_cast<int>(e);
+    if (dev < 64) attr_set[dev] = true;
+  }
+  const size_t smem_t = static_cast<size_t>(S) * 4;
+  cudaError_t e = launch_pdl(rowwise_topk_kernel, dim3(B, ns), kRowTopkThreads, smem_t, stream, pre, B, F, ld, S,
+                             k, ns > 1 ? part_val : out_val, ns > 1 ? part_idx : out_idx);
+  if (e != cudaSuccess) return static_cast<int>(e);
+  if (ns > 1) {
+    const int warps = 8;
+    const int n = ns * k;
+    const dim3 grid(ceil_div(B, warps)), block(warps * 32);
+    const int per = ceil_div(n, 32);
+    if (per <= 8) e = launch_pdl(topk_merge_kernel<8>, grid, block, 0, stream, part_val, part_idx, B, n, k, out_val, out_idx);
+    else if (per <= 16) e = launch_pdl(topk_merge_kernel<16>, grid, block, 0, stream, part_val, part_idx, B, n, k, out_val, out_idx);
+    else if (per <= 32) e = launch_pdl(topk_merge_kernel<32>, grid, block, 0, stream, part_val, part_idx, B, n, k, out_val, out_idx);
+    else e = launch_pdl(topk_merge_kernel<64>, grid, block, 0, stream, part_val, part_idx, B, n, k, out_val, out_idx);
+    if (e != cudaSuccess) return static_cast<int>(e);
+  }
+  return static_cast<int>(cudaGetLastError());
 }
 
 // Small-batch form of wsae_encode_topk (see encode_dense_kernel): `pre_ws` is B * F floats of scratch.
@@ -2180,29 +2236,20 @@ extern "C" int wsae_encode_topk_dense(const void* a_packed, const void* w_packed
                                       float* out_val, int32_t* out_idx, cudaStream_t stream) {
   if (!out_val || !out_idx) return kBadArg;
   if (k <= 0 || k > F) return kBadArg;
-  if (F > 49152 || k > 0xFFFF) return kUnsupported;
+  if (F > kSelectMaxCols || k > 0xFFFF) return kUnsupported;
   int rc = wsae_encode_dense(a_packed, w_packed, B, Bp, F, Fp, Kp, k_used_cols, pre_ws, stream);
   if (rc) return rc;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  const size_t smem_t = static_cast<size_t>(F) * 4;
-  static bool attr_set[64] = {};
-  if (dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(rowwise_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return static_cast<int>(e);
-    if (dev < 64) attr_set[dev] = true;
-  }
-  cudaError_t e = launch_pdl(rowwise_topk_kernel, B, kRowTopkThreads, smem_t, stream, static_cast<const float*>(pre_ws), B, F,
-                             k, out_val, out_idx);
-  return static_cast<int>(e != cudaSuccess ? e : cudaGetLastError());
+  return rowwise_select(pre_ws, B, F, F, k, nullptr, nullptr, out_val, out_idx, stream);
 }
 
-// K1 for k > 64 at any batch: wsae_encode_topk_dense over row chunks of chunk_rows (a multiple of 128)
-// with one [chunk_rows, F] scratch.  The fused epilogues hold a row's candidates in registers and stop
-// at k = 64; the radix select does not.  Per chunk the GEMM reads the packed rows from a tensor map
-// based at the chunk's first row, so every 128 x 256 tile runs the same MMA sequence as in one
-// unchunked call: the results are bit-identical to it.  Chunks the size of a few tens of MB keep the
-// scratch in L2 between the GEMM that writes it and the select that reads it.
+// K1 for k > 64 at any batch: the dense GEMM and the row select over row chunks of chunk_rows (a multiple
+// of 128) with one scratch: [chunk_rows, round_up(F, 4)] fp32 pre-activations, then, when F > 49152, the
+// [chunk_rows, nslices * k] candidate values and indices of the sliced select.  The fused epilogues hold a row's candidates in
+// registers and stop at k = 64; the radix select does not.  Per chunk the GEMM reads the packed rows from
+// a tensor map based at the chunk's first row, so every 128 x 256 tile runs the same MMA sequence as in
+// one unchunked call: the values are bit-identical to it, and the selection is exact on them.  Chunks the
+// size of a few tens of MB keep the scratch in L2 between the GEMM that writes it and the select that
+// reads it.
 extern "C" int wsae_encode_topk_chunked(const void* a_packed, const void* w_packed, int B, int Bp, int F,
                                         int Fp, int Kp, int k_used_cols, int k, int chunk_rows,
                                         float* pre_ws, float* out_val, int32_t* out_idx,
@@ -2210,14 +2257,22 @@ extern "C" int wsae_encode_topk_chunked(const void* a_packed, const void* w_pack
   if (!a_packed || !out_val || !out_idx || !pre_ws) return kBadArg;
   if (B <= 0 || Bp < B || Bp % kBM != 0 || Kp % kBK != 0) return kBadArg;
   if (chunk_rows <= 0 || chunk_rows % kBM != 0) return kBadArg;
+  if (F <= 0 || k <= 0 || k > F) return kBadArg;
+  const int ns = select_slices(F);
+  if (k > 0xFFFF || (ns > 1 && (static_cast<long long>(ns) * k + 31) / 32 > kMergeMaxPerLane)) return kUnsupported;
+  const int ld = round_up(F, 4);
+  const size_t part_n = static_cast<size_t>(chunk_rows) * ns * k;
+  float* part_val = pre_ws + static_cast<size_t>(chunk_rows) * ld;
+  int32_t* part_idx = reinterpret_cast<int32_t*>(part_val + part_n);
   const size_t row_bytes = static_cast<size_t>(Kp) * 2;
   for (int r0 = 0; r0 < B; r0 += chunk_rows) {
     const int rows = B - r0 < chunk_rows ? B - r0 : chunk_rows;
     const int rows_p = Bp - r0 < chunk_rows ? Bp - r0 : chunk_rows;
-    const int rc = wsae_encode_topk_dense(static_cast<const char*>(a_packed) + r0 * row_bytes, w_packed, rows,
-                                          rows_p, F, Fp, Kp, k_used_cols, k, pre_ws,
-                                          out_val + static_cast<size_t>(r0) * k,
-                                          out_idx + static_cast<size_t>(r0) * k, stream);
+    int rc = encode_dense_ld(static_cast<const char*>(a_packed) + r0 * row_bytes, w_packed, rows, rows_p, F,
+                             Fp, Kp, k_used_cols, ld, pre_ws, stream);
+    if (rc) return rc;
+    rc = rowwise_select(pre_ws, rows, F, ld, k, part_val, part_idx, out_val + static_cast<size_t>(r0) * k,
+                        out_idx + static_cast<size_t>(r0) * k, stream);
     if (rc) return rc;
   }
   return kOk;

@@ -19,11 +19,12 @@ struct RowSelectSmem {
 // (s_key[F]).  Four passes of an 8-bit most-significant-digit radix select find the key T of the k-th
 // largest value and how many keys lie above it; then every thread walks a CONTIGUOUS chunk of
 // features, a block scan turns the per-thread counts into output slots, and ties at T are admitted in
-// ascending feature index.  Output: k (value, index) pairs in ascending feature index through the
-// generic pointers ov / oi (global or shared); fewer than k valid candidates: padded with (-inf, -1).
+// ascending feature index.  Output: k (value, f_base + index) pairs in ascending feature index through
+// the generic pointers ov / oi (global or shared); fewer than k valid candidates: padded with (-inf, -1).
 // Every thread of the kRowTopkThreads-wide block must call it; it ends with a __syncthreads().
 __device__ __forceinline__ void block_row_topk(const float* __restrict__ src, int F, int k, uint32_t* s_key,
-                                               RowSelectSmem& sm, float* ov, int32_t* oi) {
+                                               RowSelectSmem& sm, float* ov, int32_t* oi,
+                                               int f_base = 0) {
   uint32_t* s_hist = sm.hist;
   uint32_t* s_pick = sm.pick;
   uint32_t* s_scan = sm.scan;
@@ -138,7 +139,7 @@ __device__ __forceinline__ void block_row_topk(const float* __restrict__ src, in
       const uint32_t slot = gt_before + ties_kept_before;
       if (slot < static_cast<uint32_t>(k)) {
         ov[slot] = src[f];
-        oi[slot] = f;
+        oi[slot] = f_base + f;
       }
     }
     gt_before += gt ? 1u : 0u;

@@ -224,27 +224,42 @@ def choose_nsplit(B: int, F: int, k: int, num_sms: int) -> int:
 _DENSE_ROWS = int(os.environ.get("WSAE_K1_DENSE_ROWS", "1024"))
 # the fused TopK epilogues of wsae_encode_topk keep at most 64 candidates per row
 ENCODE_FUSED_MAX_K = 64
-# fp32 scratch per chunk of the chunked route: written by the GEMM and read back by the select while
-# it is still in L2 (126 MB on a B200)
+# scratch per chunk of the chunked route (fp32 pre-activations, plus the sliced select's candidate lists
+# above 49 152 features): written by the GEMM and read back by the select while it is still in L2 (126 MB
+# on a B200)
 _CHUNK_SCRATCH_BYTES = 40 << 20
+# the row select holds one row's keys in shared memory: wider rows are selected in column slices of at
+# most this many features, whose k candidates each a merge reduces to k (wsae_encode_topk_chunked)
+_SELECT_MAX_COLS = 49152
 
 
 def encode_route(B: int, F: int, k: int, nsplit: int | None = None) -> str:
     """The K1 form ``encode_topk`` runs: "dense" (one GEMM storing [B, F] + one block per row
-    selecting, batches <= WSAE_K1_DENSE_ROWS), "chunked" (the same over row chunks: k > 64 on larger
-    batches) or "fused" (the GEMM with the TopK in its epilogue, k <= 64)."""
-    dense_ok = F <= 49152 and F % 4 == 0
+    selecting, batches <= WSAE_K1_DENSE_ROWS, F <= 49152, F % 4 == 0), "chunked" (the same over row
+    chunks, at any F: every k > 64 that "dense" does not take) or "fused" (the GEMM with the TopK in its
+    epilogue, k <= 64)."""
+    dense_ok = F <= _SELECT_MAX_COLS and F % 4 == 0
     if nsplit is None and B <= _DENSE_ROWS and dense_ok:
         return "dense"
-    if k > ENCODE_FUSED_MAX_K and dense_ok:
+    if k > ENCODE_FUSED_MAX_K:
         return "chunked"
     return "fused"
 
 
-def encode_chunk_rows(B: int, F: int) -> int:
-    """Rows per chunk of the chunked K1 route: a multiple of 128 whose fp32 [rows, F] scratch fits
-    _CHUNK_SCRATCH_BYTES, no more than the batch needs."""
-    rows = max(128, _CHUNK_SCRATCH_BYTES // (F * 4) // 128 * 128)
+def encode_chunk_scratch_floats(F: int, k: int, rows: int) -> int:
+    """fp32 words of scratch the chunked route needs for ``rows`` rows per chunk: the pre-activations
+    at row pitch round_up(F, 4), and above 49 152 features the [rows, nslices * k] candidate values and
+    indices of the sliced select."""
+    nslices = (F + _SELECT_MAX_COLS - 1) // _SELECT_MAX_COLS
+    return rows * (_round_up(F, 4) + (2 * nslices * k if nslices > 1 else 0))
+
+
+def encode_chunk_rows(B: int, F: int, k: int = 256) -> int:
+    """Rows per chunk of the chunked K1 route: a multiple of 128 whose scratch fits
+    _CHUNK_SCRATCH_BYTES, no more than the batch needs.  ``k`` sizes the candidate lists of the sliced
+    select above 49 152 features (by default for k = 256, the largest k of the graphed step); at most
+    49 152 features the scratch does not depend on it."""
+    rows = max(128, _CHUNK_SCRATCH_BYTES // (4 * encode_chunk_scratch_floats(F, k, 1)) // 128 * 128)
     return min(rows, _round_up(B, 128))
 
 
@@ -268,8 +283,8 @@ def encode_topk(a_packed: Tensor, w_packed: Tensor, B: int, F: int, d: int, term
         return idx, val
     if route == "chunked":
         # the scratch is allocated per call: inside a captured train step it belongs to the graph
-        rows = encode_chunk_rows(B, F)
-        pre = torch.empty((rows, F), dtype=torch.float32, device=dev)
+        rows = encode_chunk_rows(B, F, k)
+        pre = torch.empty(encode_chunk_scratch_floats(F, k, rows), dtype=torch.float32, device=dev)
         _run("wsae_encode_topk_chunked", lib.wsae_encode_topk_chunked, _ptr(a_packed), _ptr(w_packed), B, Bp, F, Fp, ps.kp, ps.used_cols, k, rows, _ptr(pre), _ptr(val), _ptr(idx), _stream(), launches=2 * ((B + rows - 1) // rows))
         return idx, val
     if nsplit is None:
