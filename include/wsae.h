@@ -56,7 +56,8 @@ int wsae_memcpy_async(void* dst, const void* src, size_t bytes, wsae_stream_t st
 /* ---- K0: operand packing (sae/model.py:108 `x - b_pre`; bias of nn.Linear at :111) ------------
  * Packed row layout: `terms` blocks of dp = round_up(d, 8) bf16 columns (split-bf16 pieces), then
  * a 16-column bias block, zero-padded to Kp = round_up(terms*dp + 16, 64).  terms: 1 = bf16,
- * 3 = ~2^-16, 6 = fp32-grade.  Rows >= B (resp. F) up to Bp (Fp) are written as zeros.
+ * 3 = ~2^-16, 6 = fp32-grade.  Rows >= B up to Bp are written as zeros; encoder rows >= F up to Fp
+ * are zeros with a -inf bias, so their pre-activation is -inf and no TopK selects them.
  * Bp must be a multiple of 128 and Fp a multiple of 256 for wsae_encode_topk. */
 int wsae_packed_k(int d, int terms, int* dp_out, int* used_cols_out, int* kp_out);
 int wsae_pack_activations(const float* x, const float* b_pre /*nullable*/, int B, int Bp, int d,
@@ -88,8 +89,9 @@ int wsae_pack_encoder(const float* w_enc /*[F,d]*/, const float* b_enc /*[F] nul
 /* ---- K1: encoder GEMM + fused per-row TopK (sae/model.py:111 Linear, :114 torch.topk) ---------
  * pre = A' . W'^T on tcgen05 tensor cores (fp32 accumulate in TMEM); the [B,F] pre-activations
  * are never written.  Emits, per row, the k largest pre-activations (signed, pre-ReLU) and their
- * feature indices, unordered.  Ties at the k-th value resolve to the lowest feature index.
- * nsplit > 1 splits F across CTAs (latency at small B); part_* are [B, nsplit_eff*k] scratch
+ * feature indices, unordered.  Ties at the k-th value resolve to the lowest feature index; NaN is
+ * never selected; a row with fewer than k non-NaN pre-activations is padded with (-inf, -1), so every
+ * index is in [-1, F).  nsplit > 1 splits F across CTAs (latency at small B); part_* are [B, nsplit_eff*k] scratch
  * (nsplit_eff from wsae_encode_effective_splits) and may be NULL when nsplit == 1.  k <= 64
  * (larger k: wsae_encode_topk_dense or wsae_encode_topk_chunked). */
 int wsae_encode_effective_splits(int F, int nsplit);

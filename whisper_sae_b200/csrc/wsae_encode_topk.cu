@@ -163,7 +163,9 @@ __device__ __noinline__ void topk_compact(uint32_t wbase, uint32_t& waddr, float
     for (int s = 0; s < CAP; ++s) vmin = fminf(vmin, (v[s] == ninf) ? pinf : v[s]);
     lo = f2key(vmin) - 1u;                  // below every candidate: count == cnt
   } else {
-    lo = f2key(tau);                        // every candidate is > tau: count == cnt
+    // every candidate is >= tau (a tie-breaking compaction keeps entries EQUAL to the tau it sets):
+    // start just below it, so count == cnt
+    lo = f2key(tau) - 1u;
   }
   uint32_t hi = f2key(vmax);                // count == 0
   int c_lo = cnt;
@@ -224,7 +226,8 @@ __device__ __noinline__ void topk_compact(uint32_t wbase, uint32_t& waddr, float
 // After one ordinary compaction (<= k + kSlack survivors) the few surplus entries are removed by
 // repeated min-extraction in registers - much cheaper than bisecting down to adjacent float keys.
 // Ties at the k-th value keep the lowest feature index: among equal minima the LAST list slot
-// (highest index; the list is in ascending index order) is dropped first.
+// (highest index; the list is in ascending index order) is dropped first.  NaN marks a slot that holds
+// no candidate (no NaN ever enters the list), so a +inf candidate is kept like any other value.
 template <int CAP, int KMAX>
 __device__ __noinline__ void topk_finalize(uint32_t wbase, uint32_t waddr, float tau, int k,
                                            float* __restrict__ out_val,
@@ -232,6 +235,7 @@ __device__ __noinline__ void topk_finalize(uint32_t wbase, uint32_t waddr, float
   constexpr int NB = KMAX + kSlack;
   const float ninf = __uint_as_float(0xff800000u);
   const float pinf = __uint_as_float(0x7f800000u);
+  const float none = __uint_as_float(0x7fc00000u);
   if (__any_sync(0xffffffffu, waddr > wbase + static_cast<uint32_t>(k + kSlack) * (kBM * 4)))
     topk_compact<CAP>(wbase, waddr, tau, k, kSlack);
   const uint32_t used = waddr - wbase;
@@ -240,27 +244,27 @@ __device__ __noinline__ void topk_finalize(uint32_t wbase, uint32_t waddr, float
 #pragma unroll
   for (int s = 0; s < NB; ++s) {
     const float x = lds_f32(wbase + s * (kBM * 4));
-    v[s] = (static_cast<uint32_t>(s * (kBM * 4)) < used) ? x : pinf;   // +inf = not a candidate
+    v[s] = (static_cast<uint32_t>(s * (kBM * 4)) < used) ? x : none;
   }
   while (__any_sync(0xffffffffu, surplus > 0)) {
     float vmin = pinf;
     int pos = -1;
 #pragma unroll
     for (int s = 0; s < NB; ++s) {
-      const bool le = v[s] <= vmin && v[s] != pinf;
+      const bool le = v[s] <= vmin;    // false for NaN
       vmin = le ? v[s] : vmin;
       pos = le ? s : pos;
     }
     if (surplus <= 0) pos = -1;
 #pragma unroll
-    for (int s = 0; s < NB; ++s) v[s] = (s == pos) ? pinf : v[s];
+    for (int s = 0; s < NB; ++s) v[s] = (s == pos) ? none : v[s];
     --surplus;
   }
   if (write) {
     int w = 0;
 #pragma unroll
     for (int s = 0; s < NB; ++s) {
-      if (v[s] != pinf && w < k) {
+      if (v[s] == v[s] && w < k) {
         uint32_t ix;
         asm volatile("ld.shared.u32 %0, [%1];" : "=r"(ix) : "r"(wbase + s * (kBM * 4) + CAP * kBM * 4) : "memory");
         out_val[w] = v[s];
@@ -446,7 +450,7 @@ encode_topk_kernel(const __grid_constant__ CUtensorMap tmap_a,
         // fresh registers (a0 -> a1 -> a2 -> a3 -> a0') so that no address register is rewritten
         // while a store that reads it is still in flight (the read-after-write scoreboard wait
         // on an in-place `@p add` costs ~20 cycles per value).
-        // Zero-padded feature rows of W' carry a -3.4e38 bias (wsae_pack.cu), so they never pass.
+        // Zero-padded feature rows of W' carry a -inf bias (wsae_pack.cu), so they never pass.
         auto process = [&](uint32_t (&r)[16], int cbase) {
 #pragma unroll
           for (int j = 0; j < kChunk; j += 4) {
@@ -629,6 +633,23 @@ __device__ __forceinline__ uint32_t append4(uint32_t w, float thr, float v0, flo
   return wn;
 }
 
+// min.NaN.f32: unlike fminf, a NaN operand makes the result NaN
+__device__ __forceinline__ float fmin_nan(float a, float b) {
+  float r;
+  asm("min.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+  return r;
+}
+
+// Scanner threshold from the floor of a work item's first tile (the smallest of its 32 group maxima,
+// taken with fmin_nan).  Candidates must be strictly above the threshold, so it steps to the next float
+// below the floor, and below -0.0 when the floor is +0.0 or -0.0: every value equal to the floor still
+// passes.  A floor that is NaN (a group of 8 NaN columns has no maximum) or -inf (padding columns)
+// bounds nothing: tau stays where it is.
+__device__ __forceinline__ float floor_threshold(float floor_v, float tau) {
+  if (!(floor_v > __uint_as_float(0xff800000u))) return tau;
+  return fmaxf(tau, key2f(f2key(floor_v == 0.f ? -0.f : floor_v) - 1u));
+}
+
 __device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
   uint32_t v;
   asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
@@ -670,7 +691,7 @@ __device__ __forceinline__ float select_threshold(const float (&v)[N], int total
     const float vmin = fminf(fminf(n0, n1), fminf(n2, n3));
     lo = f2key(vmin) - 1u;
   } else {
-    lo = f2key(tau);
+    lo = f2key(tau) - 1u;   // survivors of a tie-breaking select equal tau: start just below it
   }
   uint32_t hi = f2key(vmax);
   bool done = keep_all;
@@ -853,7 +874,8 @@ encode_topk2_kernel(const __grid_constant__ CUtensorMap tmap_a,
         // its values instead of all of the first ~120 columns: about two hand-overs fewer per item,
         // in the part of the item where the selector is the bottleneck.  Costs one extra read of
         // the tile (16 tcgen05.ld) and ~0.6 instructions per value while the selector is idle.
-        // Padding columns (-3.39e38) only make the floor useless, never wrong.  (k <= 32 here.)
+        // A group of 8 NaN columns has no maximum: fmin_nan turns the floor into NaN, and padding
+        // columns (-inf) turn it into -inf; either leaves tau at -inf.  (k <= 32 here.)
         if (nt == t0 && !(DBG && mode >= 3)) {
           float floor_v = __uint_as_float(0x7f800000u);
           uint32_t rp[16];
@@ -869,11 +891,9 @@ encode_topk2_kernel(const __grid_constant__ CUtensorMap tmap_a,
                                          fmaxf(__uint_as_float(rp[10]), __uint_as_float(rp[11]))),
                                    fmaxf(fmaxf(__uint_as_float(rp[12]), __uint_as_float(rp[13])),
                                          fmaxf(__uint_as_float(rp[14]), __uint_as_float(rp[15]))));
-            floor_v = fminf(floor_v, fminf(m0, m1));
+            floor_v = fmin_nan(floor_v, fmin_nan(m0, m1));
           }
-          // candidates must be strictly above the threshold: step to the next float below the floor
-          // so that values EQUAL to it still pass.  NaN maxima (NaN rows) leave tau at -inf.
-          if (floor_v == floor_v) tau = fmaxf(tau, key2f(f2key(floor_v) - 1u));
+          tau = floor_threshold(floor_v, tau);
         }
 
         // ---- scan of one 128x256 accumulator tile, 32 columns (two tcgen05.ld.x16) per trip ----
@@ -1403,7 +1423,8 @@ encode_topk3_kernel(const __grid_constant__ CUtensorMap tmap_a,
         // its values instead of all of the first ~120 columns: about two hand-overs fewer per item,
         // in the part of the item where the selector is the bottleneck.  Costs one extra read of
         // the tile (16 tcgen05.ld) and ~0.6 instructions per value while the selector is idle.
-        // Padding columns (-3.39e38) only make the floor useless, never wrong.  (k <= 32 here.)
+        // A group of 8 NaN columns has no maximum: fmin_nan turns the floor into NaN, and padding
+        // columns (-inf) turn it into -inf; either leaves tau at -inf.  (k <= 32 here.)
         if (nt == t0 && !(DBG && mode >= 3)) {
           float floor_v = __uint_as_float(0x7f800000u);
           uint32_t rp[16];
@@ -1419,11 +1440,9 @@ encode_topk3_kernel(const __grid_constant__ CUtensorMap tmap_a,
                                          fmaxf(__uint_as_float(rp[10]), __uint_as_float(rp[11]))),
                                    fmaxf(fmaxf(__uint_as_float(rp[12]), __uint_as_float(rp[13])),
                                          fmaxf(__uint_as_float(rp[14]), __uint_as_float(rp[15]))));
-            floor_v = fminf(floor_v, fminf(m0, m1));
+            floor_v = fmin_nan(floor_v, fmin_nan(m0, m1));
           }
-          // candidates must be strictly above the threshold: step to the next float below the floor
-          // so that values EQUAL to it still pass.  NaN maxima (NaN rows) leave tau at -inf.
-          if (floor_v == floor_v) tau = fmaxf(tau, key2f(f2key(floor_v) - 1u));
+          tau = floor_threshold(floor_v, tau);
         }
 
         // ---- scan of one 128x256 accumulator tile, 32 columns (two tcgen05.ld.x16) per trip ----

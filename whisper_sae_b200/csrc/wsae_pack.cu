@@ -2,7 +2,7 @@
 //
 //   A'[r, :] = [ piece_a0(xc_r) | ... | piece_a(T-1)(xc_r) | 1 1 1 0 ... 0 | 0-pad ]   xc = x - b_pre
 //   W'[f, :] = [ piece_w0(W_f)  | ... | piece_w(T-1)(W_f)  | b1 b2 b3 0 .. | 0-pad ]   b1+b2+b3 = b_enc[f]
-//   W'[f >= F, :] = [ 0 ... 0 | -3.39e38 0 0 .. | 0-pad ]      (padding rows: pre-activation = -3.39e38)
+//   W'[f >= F, :] = [ 0 ... 0 | -inf 0 0 .. | 0-pad ]      (padding rows: pre-activation = -inf)
 //
 // (reference: x - b_pre is model.py:108; the encoder bias add is part of nn.Linear at model.py:111.)
 // Each of the T blocks is dp = round_up(d, 8) columns wide.  A split-bf16 "piece" p of a float v is
@@ -76,9 +76,11 @@ pack_rows_kernel(const float* __restrict__ src, const float* __restrict__ center
       }
     }
   } else if (KIND == 1 && c0 == T * dp) {
-    // zero-padded feature rows (F..Fp) get the most negative finite bf16 as their bias, so the
-    // TopK epilogue of K1 can scan whole tiles without a column guard: they never win.
-    out[0] = __ushort_as_bfloat16(static_cast<unsigned short>(0xFF7Fu));
+    // zero-padded feature rows (F..Fp) get a -inf bias, so the TopK epilogues of K1 can scan whole
+    // tiles without a column guard: no threshold admits -inf, even in a row with fewer than k valid
+    // (non-NaN) pre-activations.  (Rows >= B of A' are zero: 0 * -inf = NaN there, and those rows
+    // are never written.)
+    out[0] = __ushort_as_bfloat16(static_cast<unsigned short>(0xFF80u));
   }
   *reinterpret_cast<uint4*>(dst + static_cast<size_t>(r) * Kp + c0) =
       *reinterpret_cast<const uint4*>(out);
