@@ -37,7 +37,7 @@ typedef void* wsae_stream_t; /* cudaStream_t */
  * additions that change no existing behaviour keep the number: wsae_encode_topk_chunked, and k up to 256 in
  * wsae_decode_backward / _at / _rows_at; the half-precision activation forms wsae_pack_activations_typed,
  * wsae_decode_backward_typed, wsae_row_step_typed and wsae_layernorm_rows_typed, whose dtype 0 is the
- * existing entry point).
+ * existing entry point; wsae_splice_pack and wsae_splice_decode).
  *
  * Activation dtype codes (x_dtype / in_dtype / out_dtype): 0 = float32, 1 = bfloat16, 2 = float16.  A
  * bf16 / fp16 activation matrix is converted to fp32 as it is loaded, and everything after the load is
@@ -352,6 +352,38 @@ int wsae_layernorm_rows(const void* x, int in_dtype, long long rows, int d, long
 int wsae_layernorm_rows_typed(const void* x, int in_dtype, long long rows, int d, long long in_pitch_elems,
                               const float* gamma /*nullable*/, const float* beta /*nullable*/, float eps,
                               void* out, int out_dtype, long long out_pitch_elems, wsae_stream_t stream);
+
+/* ---- Splicing a TopK SAE into Whisper's forward pass (sae/splice.py) ---------------------------
+ * A site's layer output row h [d] (dtype h_dtype), its mean mu and biased variance var, r = rsqrt(var + eps):
+ *   x      = (h - mu) * r * gamma + beta                 (the fp32 formula of wsae_layernorm_rows)
+ *   (i, v) = TopK_k(pack(x - b_pre) . W'^T)             (wsae_encode_topk*, terms = 1)
+ *   a_j    = relu(v_j), rounded to bf16                  (K2's convention)
+ *   recon  = sum_j a_j W_dec[i_j] + b_dec + b_pre        (bf16 decoder shadow, fp32 accumulation)
+ *   recon' = sum_j gain[i_j] a_j W_dec[i_j] + b_dec + b_pre + steer
+ *   mode 0 (replace): h' = mu + ((recon' - beta) / gamma) / r
+ *   mode 1 (error)  : h' = h + ((recon' - recon) / gamma) / r; an element whose difference is exactly 0 is
+ *                     written back with h's bits.  recon' - recon is accumulated directly, as
+ *                     steer + sum (gain - 1) a_j W_dec[i_j] over the entries whose gain is not 1.
+ * h' is written in h's dtype, rounded to nearest.  Without the LayerNorm (row_stats == NULL in the decode;
+ * pack with wsae_pack_activations_typed) x = h and the inverse map is the identity.
+ *
+ * wsae_splice_pack: a_packed = pack_activations(LN(h), b_pre, terms = 1) bit for bit ([Bp, Kp] bf16, rows
+ *   >= N zero, Bp % 128 == 0) and row_stats [N, 2] = (mu, r) float32; h is [N, d] with row pitch d.
+ * wsae_splice_decode: out [N, d] (h's dtype; may not alias h).  idx / val [N, k] from K1, any k, padding
+ *   (-inf, -1) allowed.  gain [F] / steer [d] / gamma / beta nullable (1 / 0).  Accumulators, nullable,
+ *   caller-zeroed, added to: stats {double sse (unmodified recon against x); double sum x^2; uint64 l0},
+ *   x_sum double [d], feature_count int64 [F] (rows in which each feature fired).
+ * Both: d % 8 == 0, d <= 4096 (WSAE_E_UNSUPPORTED above), pointers 16-byte aligned. */
+int wsae_splice_pack(const void* h, int h_dtype, int N, int Bp, int d, const float* gamma /*nullable*/,
+                     const float* beta /*nullable*/, float eps, const float* b_pre /*nullable*/,
+                     void* a_packed /*bf16 [Bp,Kp]*/, float* row_stats /*[N,2]*/, wsae_stream_t stream);
+int wsae_splice_decode(const void* h, int h_dtype, const float* row_stats /*nullable*/,
+                       const float* gamma /*nullable*/, const float* beta /*nullable*/,
+                       const void* w_decT_bf16 /*[F,d]*/, const float* b_dec, const float* b_pre /*nullable*/,
+                       const int32_t* idx, const float* val, const float* gain /*nullable*/,
+                       const float* steer /*nullable*/, int N, int d, int F, int k, int mode, void* out,
+                       void* stats /*nullable*/, double* x_sum /*nullable*/,
+                       long long* feature_count /*nullable*/, wsae_stream_t stream);
 
 /* ---- deterministic accumulation mode (SAETrainer(..., deterministic=True)) ----------------------
  * The default kernels add their cross-row / split-K partial sums with float atomics in arrival

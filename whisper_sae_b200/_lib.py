@@ -180,6 +180,13 @@ _SIGNATURES = {
                              c_void_p, c_longlong, c_void_p], c_int),
     "wsae_layernorm_rows_typed": ([c_void_p, c_int, c_longlong, c_int, c_longlong, c_void_p, c_void_p, c_float,
                                    c_void_p, c_int, c_longlong, c_void_p], c_int),
+    "wsae_splice_pack": ([c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                          c_void_p, c_void_p], c_int),
+    "wsae_splice_decode": (
+        [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+         c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p],
+        c_int,
+    ),
     "wsae_feature_topk_workspace": ([c_longlong, c_int, POINTER(c_ulonglong)], c_int),
     "wsae_feature_topk_update": (
         [c_void_p, c_void_p, c_void_p, c_longlong, c_int, c_void_p, c_longlong, c_void_p, c_int, c_int,

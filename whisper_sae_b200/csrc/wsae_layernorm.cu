@@ -11,29 +11,9 @@
 // torch.nn.LayerNorm formula) and writes fp32 row `out_row0 + r` of a caller-owned [N, d] device
 // matrix, so flatten + concatenate are just the destination offset.
 // HBM bound: d * (in_bytes + 4) bytes per row.
-#include <cuda_fp16.h>
-
-#include "wsae_common.cuh"
+#include "wsae_rownorm.cuh"
 
 namespace wsae {
-
-constexpr int kLnMaxPerLane = 128;   // d <= 32 * 128 = 4096 keeps the row in registers
-
-template <typename TIn>
-__device__ __forceinline__ float ln_load(const TIn* p, size_t i);
-template <>
-__device__ __forceinline__ float ln_load<float>(const float* p, size_t i) { return p[i]; }
-template <>
-__device__ __forceinline__ float ln_load<__nv_bfloat16>(const __nv_bfloat16* p, size_t i) {
-  return __bfloat162float(p[i]);
-}
-template <>
-__device__ __forceinline__ float ln_load<__half>(const __half* p, size_t i) { return __half2float(p[i]); }
-
-// fp32 result -> output element, rounded to nearest
-__device__ __forceinline__ void ln_store(float* p, float v) { *p = v; }
-__device__ __forceinline__ void ln_store(__nv_bfloat16* p, float v) { *p = __float2bfloat16_rn(v); }
-__device__ __forceinline__ void ln_store(__half* p, float v) { *p = __float2half_rn(v); }
 
 template <typename TIn, typename TOut, int PER>
 __global__ void __launch_bounds__(256)
@@ -45,22 +25,13 @@ layernorm_rows_kernel(const TIn* __restrict__ x, long long rows, int d, long lon
   if (row >= rows) return;
   const TIn* xr = x + row * in_pitch;
   float v[PER];
-  float sum = 0.f;
 #pragma unroll
   for (int j = 0; j < PER; ++j) {
     const int c = j * 32 + lane;
     v[j] = c < d ? ln_load<TIn>(xr, c) : 0.f;
-    sum += v[j];
   }
-  const float mean = warp_sum(sum) / static_cast<float>(d);
-  float sq = 0.f;
-#pragma unroll
-  for (int j = 0; j < PER; ++j) {
-    const int c = j * 32 + lane;
-    const float t = c < d ? v[j] - mean : 0.f;
-    sq = fmaf(t, t, sq);
-  }
-  const float rstd = rsqrtf(warp_sum(sq) / static_cast<float>(d) + eps);
+  float mean, rstd;
+  ln_moments<PER>([&](int j) { return v[j]; }, d, lane, eps, mean, rstd);
   TOut* orow = out + row * out_pitch;
 #pragma unroll
   for (int j = 0; j < PER; ++j) {
@@ -68,7 +39,7 @@ layernorm_rows_kernel(const TIn* __restrict__ x, long long rows, int d, long lon
     if (c < d) {
       const float g = gamma != nullptr ? gamma[c] : 1.f;
       const float b = beta != nullptr ? beta[c] : 0.f;
-      ln_store(orow + c, (v[j] - mean) * rstd * g + b);
+      ln_store(orow + c, ln_apply(v[j], mean, rstd, g, b));
     }
   }
 }
@@ -81,17 +52,17 @@ static int launch_layernorm(const void* x, long long rows, int d, long long in_p
   const int warps = 8;
   const unsigned blocks = static_cast<unsigned>((rows + warps - 1) / warps);
   const TIn* xi = static_cast<const TIn*>(x);
-  const int per = ceil_div(d, 32);
+  const int per = ln_per_bucket(d);
 #define WSAE_LN_CASE(P)                                                                        \
   layernorm_rows_kernel<TIn, TOut, P><<<blocks, warps * 32, 0, stream>>>(xi, rows, d, in_pitch, gamma, \
                                                                    beta, eps, out, out_pitch)
-  if (per <= 4) WSAE_LN_CASE(4);
-  else if (per <= 12) WSAE_LN_CASE(12);
-  else if (per <= 16) WSAE_LN_CASE(16);
-  else if (per <= 24) WSAE_LN_CASE(24);
-  else if (per <= 32) WSAE_LN_CASE(32);
-  else if (per <= 40) WSAE_LN_CASE(40);
-  else if (per <= 64) WSAE_LN_CASE(64);
+  if (per == 4) WSAE_LN_CASE(4);
+  else if (per == 12) WSAE_LN_CASE(12);
+  else if (per == 16) WSAE_LN_CASE(16);
+  else if (per == 24) WSAE_LN_CASE(24);
+  else if (per == 32) WSAE_LN_CASE(32);
+  else if (per == 40) WSAE_LN_CASE(40);
+  else if (per == 64) WSAE_LN_CASE(64);
   else WSAE_LN_CASE(kLnMaxPerLane);
 #undef WSAE_LN_CASE
   return static_cast<int>(cudaGetLastError());

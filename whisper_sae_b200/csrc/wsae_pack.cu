@@ -11,7 +11,7 @@
 // T terms:  T=1: a0*w0        T=3: a0*w0 + a1*w0 + a0*w1
 //           T=6: a0*w0 + a0*w1 + a1*w0 + a0*w2 + a1*w1 + a2*w0   (error ~2^-24: fp32 grade)
 // The bias block is always a 3-piece split, so the bias is exact to fp32 in every mode.
-#include "wsae_common.cuh"
+#include "wsae_rownorm.cuh"
 
 namespace wsae {
 
@@ -132,15 +132,9 @@ pack_activations_bf16_kernel(const TX* __restrict__ x, const TX* const* __restri
         a.x -= ca.x; a.y -= ca.y; a.z -= ca.z; a.w -= ca.w;
         b.x -= cb.x; b.y -= cb.y; b.z -= cb.z; b.w -= cb.w;
       }
-      __nv_bfloat162 p0 = __floats2bfloat162_rn(a.x, a.y), p1 = __floats2bfloat162_rn(a.z, a.w);
-      __nv_bfloat162 p2 = __floats2bfloat162_rn(b.x, b.y), p3 = __floats2bfloat162_rn(b.z, b.w);
-      out.x = *reinterpret_cast<uint32_t*>(&p0);
-      out.y = *reinterpret_cast<uint32_t*>(&p1);
-      out.z = *reinterpret_cast<uint32_t*>(&p2);
-      out.w = *reinterpret_cast<uint32_t*>(&p3);
+      out = k0_pack8(a, b);
     } else if (c0 == d) {
-      out.x = 0x3F803F80u;   // bf16 1.0, 1.0
-      out.y = 0x00003F80u;   // bf16 1.0, 0
+      out = k0_bias_block8();
     }
   }
   *reinterpret_cast<uint4*>(dst + static_cast<size_t>(r) * Kp + c0) = out;

@@ -725,3 +725,111 @@ def layernorm_rows_(x: Tensor, gamma: Tensor | None, beta: Tensor | None, eps: f
     dst = out.data_ptr() + row0 * out.stride(0) * out.element_size()
     _run("wsae_layernorm_rows", lib.wsae_layernorm_rows_typed, _ptr(x2), _LN_DTYPES[x.dtype], n, d, x2.stride(0),
          _ptr(gamma), _ptr(beta), float(eps), dst, _LN_DTYPES[out.dtype], out.stride(0), _stream())
+
+
+# splice modes of wsae_splice_decode (include/wsae.h)
+SPLICE_MODES = {"replace": 0, "error": 1}
+SPLICE_MAX_D = 4096
+
+
+def _splice_rows(h: Tensor, d: int) -> Tensor:
+    if h.dtype not in _LN_DTYPES:
+        raise RuntimeError(f"unsupported hidden-state dtype {h.dtype} (float32, bfloat16 or float16)")
+    if d % 8 != 0 or d > SPLICE_MAX_D:
+        raise RuntimeError(f"the splice kernels need d % 8 == 0 and d <= {SPLICE_MAX_D} (got d = {d})")
+    h2 = h.reshape(-1, d)
+    if not h2.is_contiguous() or h2.data_ptr() % 16 != 0:
+        h2 = h2.contiguous()
+    return h2
+
+
+def _ln_params(gamma: Tensor | None, beta: Tensor | None) -> tuple[Tensor | None, Tensor | None]:
+    # a half-precision Whisper carries half-precision LayerNorm parameters: the kernels compute in fp32
+    gamma = None if gamma is None else gamma.detach().to(torch.float32).contiguous()
+    beta = None if beta is None else beta.detach().to(torch.float32).contiguous()
+    return gamma, beta
+
+
+def splice_pack(h: Tensor, gamma: Tensor | None, beta: Tensor | None, eps: float, b_pre: Tensor | None,
+                out: Tensor | None = None, row_stats: Tensor | None = None) -> tuple[Tensor, Tensor]:
+    """wsae_splice_pack: final LayerNorm of the hidden rows ``h [..., d]`` (float32, bfloat16 or float16)
+    and K0's single-term packing in one pass.  Returns (a_packed bf16 [Bp, Kp], row_stats float32 [N, 2] =
+    (mean, rstd)); ``a_packed`` equals ``pack_activations(layernorm_rows(h), b_pre, 1)`` bit for bit."""
+    _need_cuda(h, gamma, beta, b_pre, out, row_stats)
+    d = h.shape[-1]
+    h2 = _splice_rows(h, d)
+    gamma, beta = _ln_params(gamma, beta)
+    _f32c(b_pre, "b_pre")
+    N = h2.shape[0]
+    if N == 0:
+        raise RuntimeError("splice_pack needs at least one row")
+    ps = packed_shape(d, 1)
+    Bp = _round_up(N, 128)
+    if out is None or out.shape != (Bp, ps.kp) or out.dtype != torch.bfloat16:
+        out = torch.empty((Bp, ps.kp), dtype=torch.bfloat16, device=h.device)
+    if row_stats is None or row_stats.shape != (N, 2):
+        row_stats = torch.empty((N, 2), dtype=torch.float32, device=h.device)
+    _f32c(row_stats, "row_stats")
+    lib = _lib.load()
+    _run("wsae_splice_pack", lib.wsae_splice_pack, _ptr(h2), _LN_DTYPES[h2.dtype], N, Bp, d, _ptr(gamma), _ptr(beta),
+         float(eps), _ptr(b_pre), _ptr(out), _ptr(row_stats), _stream())
+    return out, row_stats
+
+
+def splice_decode(h: Tensor, row_stats: Tensor | None, gamma: Tensor | None, beta: Tensor | None,
+                  w_decT_bf16: Tensor, b_dec: Tensor, b_pre: Tensor | None, idx: Tensor, val: Tensor, *,
+                  mode: str, gain: Tensor | None = None, steer: Tensor | None = None, out: Tensor | None = None,
+                  stats: Tensor | None = None, x_sum: Tensor | None = None,
+                  feature_count: Tensor | None = None) -> Tensor:
+    """wsae_splice_decode: the spliced layer output h' (``h``'s shape and dtype) from K1's ``(idx, val)``
+    (include/wsae.h states the formulas).  ``row_stats`` from ``splice_pack`` (None: no LayerNorm, x = h).
+    ``mode``: "replace" or "error".  Accumulators (caller-zeroed, added to): ``stats`` int64 [3] holding
+    {float64 sse, float64 sum x^2, uint64 l0}, ``x_sum`` float64 [d], ``feature_count`` int64 [F]."""
+    if mode not in SPLICE_MODES:
+        raise RuntimeError(f"unknown splice mode {mode!r} (one of {sorted(SPLICE_MODES)})")
+    _need_cuda(h, row_stats, gamma, beta, w_decT_bf16, b_dec, b_pre, idx, val, gain, steer, out, stats, x_sum,
+               feature_count)
+    F, d = w_decT_bf16.shape
+    if h.shape[-1] != d:
+        raise RuntimeError(f"hidden width {h.shape[-1]} != decoder width {d}")
+    h2 = _splice_rows(h, d)
+    N = h2.shape[0]
+    if w_decT_bf16.dtype != torch.bfloat16 or not w_decT_bf16.is_contiguous():
+        raise RuntimeError("w_decT_bf16 must be a contiguous [F, d] bfloat16 matrix")
+    _f32c(b_dec, "decoder.bias")
+    _f32c(b_pre, "b_pre")
+    _f32c(gain, "gain")
+    _f32c(steer, "steer")
+    if gain is not None and gain.numel() != F:
+        raise RuntimeError(f"gain must have {F} elements")
+    if steer is not None and steer.numel() != d:
+        raise RuntimeError(f"steer must have {d} elements")
+    if idx.dtype != torch.int32 or val.dtype != torch.float32 or idx.shape != val.shape or idx.dim() != 2 \
+            or idx.shape[0] != N or not idx.is_contiguous() or not val.is_contiguous():
+        raise RuntimeError(f"idx / val must be contiguous int32 / float32 [{N}, k]")
+    k = idx.shape[1]
+    if row_stats is not None:
+        _f32c(row_stats, "row_stats")
+        if row_stats.shape != (N, 2):
+            raise RuntimeError(f"row_stats must be [{N}, 2]")
+        gamma, beta = _ln_params(gamma, beta)
+    else:
+        gamma = beta = None
+    if stats is not None and (stats.dtype != torch.int64 or stats.numel() != 3 or not stats.is_contiguous()):
+        raise RuntimeError("stats must be a contiguous int64 [3] tensor")
+    if x_sum is not None and (x_sum.dtype != torch.float64 or x_sum.numel() != d or not x_sum.is_contiguous()):
+        raise RuntimeError(f"x_sum must be a contiguous float64 [{d}] tensor")
+    if feature_count is not None and (feature_count.dtype != torch.int64 or feature_count.numel() != F
+                                      or not feature_count.is_contiguous()):
+        raise RuntimeError(f"feature_count must be a contiguous int64 [{F}] tensor")
+    if out is None:
+        out = torch.empty(h.shape, dtype=h.dtype, device=h.device)
+    elif out.shape != h.shape or out.dtype != h.dtype or not out.is_contiguous():
+        raise RuntimeError("out must be a contiguous tensor of h's shape and dtype")
+    if N == 0:
+        return out
+    lib = _lib.load()
+    _run("wsae_splice_decode", lib.wsae_splice_decode, _ptr(h2), _LN_DTYPES[h2.dtype], _ptr(row_stats), _ptr(gamma),
+         _ptr(beta), _ptr(w_decT_bf16), _ptr(b_dec), _ptr(b_pre), _ptr(idx), _ptr(val), _ptr(gain), _ptr(steer),
+         N, d, F, k, SPLICE_MODES[mode], _ptr(out), _ptr(stats), _ptr(x_sum), _ptr(feature_count), _stream())
+    return out
